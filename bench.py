@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the LEC hot path (BASELINE.json metric) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (``configs[3]`` of BASELINE.json, the largest single-GPU configuration): synthetic
 ERA5 0.25 deg global-shape fields, 1440 x 721 x 37 levels, fp32, fixed box = all
@@ -63,7 +63,15 @@ def parse_args():
     ap.add_argument("--no-fp64", action="store_true")
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--no-plugin", action="store_true", help="skip the lec_fixed (plugin call) end-to-end line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed passes, write what the last one returned (terms, levels, flags; all ranks) "
+                         "to DIR/<name>.npy as float64; the inputs are seeded, so two builds compare file for file")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def row_kernel_name():
@@ -388,6 +396,29 @@ def bench_plugin(args, grid, nslots, dev, rank, local_rank, world):
                    "-> per-level CSVs + results CSV on tmpfs (best of %d calls, wall clock)" % args.e2e_passes}
 
 
+def dump_outputs(d, g_res, flags, chunk, rank, world, dev):
+    """``--dump-outputs``: the gathered results of the last timed pass as a caller receives them -- terms
+    [steps, 16], levels [steps, 19, levels] and flags [steps] over the time steps of all ranks -- written by rank 0
+    as float64 ``.npy`` (~0.3 MB per rank)."""
+    import torch
+    import torch.distributed as dist
+    from lorenzcycletoolkit_b200 import engine as E
+    if world > 1:
+        gathered = torch.empty(world * chunk, dtype=flags.dtype, device=dev)
+        dist.all_gather_into_tensor(gathered, flags)
+        flags = gathered
+    if rank != 0:
+        return
+    nt = chunk * E.NTERMS
+    per_rank = g_res.view(world, -1)
+    arrays = {"terms": per_rank[:, :nt].reshape(world * chunk, E.NTERMS),
+              "levels": per_rank[:, nt:].reshape(world * chunk, E.NLEVEL_TERMS, NLEV),
+              "flags": flags}
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, f"{name}.npy"), a.cpu().numpy().astype(np.float64))
+
+
 # --------------------------------------------------------------------------------------- #
 def run_b200(args, rank, local_rank, world):
     import torch
@@ -477,6 +508,8 @@ def run_b200(args, rank, local_rank, world):
     launches = eng.launch_count - launches0
     clocks = sampler.summary(wall0, wall1) if sampler else None
     value = world * chunk * args.steps / (elapsed_ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, g_res, out[2], chunk, rank, world, dev)
 
     # ---- the same box with float64 fields (the path int16-packed ERA5 takes) ------------------
     fp64_line = None if args.no_fp64 else bench_fp64(args, grid, fields, steps, dev, local_rank, world)

@@ -223,6 +223,27 @@ int lec_timing_reset(lec_handle *h);
 /* Number of kernel launches issued by this handle so far. */
 int64_t lec_launch_count(lec_handle *h);
 
+/* Row-moment kernel that the last kernel batch of the last lec_run_* call on this handle launched (a call
+ * with more steps than max_steps runs several batches; each chooses again).  Read-only: it reports what
+ * the dispatcher chose and changes nothing.  LEC_ERR_INVALID before the first batch. */
+#define LEC_ROWS_DIRECT          0   /* direct loads, one warp per row                                 */
+#define LEC_ROWS_SUBWARP         1   /* direct loads, a group of `group` lanes per row (narrow boxes)  */
+#define LEC_ROWS_TILED           2   /* TMA ring of tile_rows-row tiles, one warp per row (wide boxes)  */
+#define LEC_ROWS_TILED_SUBWARP   3   /* TMA ring feeding 8-lane row groups (track boxes, opt-in)        */
+typedef struct lec_dispatch {
+  int32_t kernel;           /* LEC_ROWS_* */
+  int32_t vec;              /* elements per lane load: 4 (fp32) / 2 (fp64) on 16-byte aligned rows, 1 scalar */
+  int32_t group;            /* lanes per row: 4, 8 or 16 for the sub-warp kernels, else 32 */
+  int32_t lonw;             /* longitude tables: 0 uniform, 1 per-column weights, 2 weights and stencil */
+  int32_t comp;             /* 1: compensated fp32 linear sums */
+  int32_t math64;           /* 1: fp64 pointwise arithmetic (fp64 fields or LEC_MATH_F64) */
+  int32_t tile_rows;        /* box rows per tile (tiled kernels), per CTA otherwise */
+  int32_t tiles_per_band;   /* tiles per latitude band of the block order */
+  int32_t nbands;           /* latitude bands (1: step-major order) */
+  int32_t reserved;
+} lec_dispatch;
+int lec_last_dispatch(const lec_handle *h, lec_dispatch *out);
+
 /* Bytes the last lec_run_host moved over PCIe: out[0] host->device (fields: T for every slot a step
  * or its time neighbours touch, u/v/omega/Phi for the centre slots only; slots shared by two staged
  * chunks are copied device-to-device and not counted), out[1] device->host (results). */

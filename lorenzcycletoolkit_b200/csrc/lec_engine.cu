@@ -88,6 +88,8 @@ struct lec_handle {
   bool call_timed = false;
   bool accumulate_timing = false;
   long long launches = 0;
+  lec_dispatch dispatch{};                      // row kernel of the last kernel batch (lec_last_dispatch)
+  bool dispatched = false;
   std::string err;
 };
 
@@ -329,6 +331,12 @@ static thread_local std::string g_free_err;   // error text of the handle-free e
 const char* lec_last_error(lec_handle* h) { return h ? h->err.c_str() : g_free_err.c_str(); }
 
 int64_t lec_launch_count(lec_handle* h) { return h ? h->launches : 0; }
+
+int lec_last_dispatch(const lec_handle* h, lec_dispatch* out) {
+  if (!h || !out || !h->dispatched) return LEC_ERR_INVALID;
+  *out = h->dispatch;
+  return LEC_OK;
+}
 
 int lec_last_transfer(lec_handle* h, int64_t out_bytes[2]) {
   if (!h || !out_bytes) return LEC_ERR_INVALID;
@@ -675,6 +683,20 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   // TMA loads of u, v, omega, Phi with an L2 evict-first hint: fp64 fields only (46.7 -> 39.0 GB of DRAM reads per
   // 24-step launch, +3.4 %; with fp32 fields the working set of a band fits without it and the hint costs 2 %)
   rp.prefetch_mode = h->prefetch_mode | ((h->tma_hint < 0 ? h->desc.dtype == LEC_F64 : h->tma_hint != 0) ? 8 : 0);
+  {   // the template instance launched below, for lec_last_dispatch (COMP only exists for fp32 arithmetic; the
+      // sub-warp kernels have no per-column-weight variant: any table is the full one)
+    lec_dispatch& d = h->dispatch;
+    const int lonw = lon_mode(h);
+    d.kernel = want_tile ? LEC_ROWS_TILED : want_ntile ? LEC_ROWS_TILED_SUBWARP : narrow_g ? LEC_ROWS_SUBWARP : LEC_ROWS_DIRECT;
+    d.vec = vec ? vecw : 1;
+    d.group = want_tile ? 32 : want_ntile ? 8 : narrow_g ? narrow_g : 32;
+    d.lonw = (d.kernel == LEC_ROWS_SUBWARP || d.kernel == LEC_ROWS_TILED_SUBWARP) && lonw != 0 ? 2 : lonw;
+    d.comp = comp && !math64;
+    d.math64 = math64;
+    d.tile_rows = tile_rows; d.tiles_per_band = rp.tiles_per_band; d.nbands = rp.nbands;
+    d.reserved = 0;
+    h->dispatched = true;
+  }
 
   cudaEvent_t e0 = next_event(h), e1 = next_event(h), e2 = next_event(h);
   if (!e0 || !e1 || !e2) { h->err = "cudaEventCreate"; return LEC_ERR_CUDA; }

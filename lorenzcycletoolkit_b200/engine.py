@@ -62,6 +62,13 @@ class _RawDesc(C.Structure):
                 ("big_endian", C.c_int32), ("reserved", C.c_int32), ("record_stride", C.c_int64 * 5)]
 
 
+class _Dispatch(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("kernel", "vec", "group", "lonw", "comp", "math64", "tile_rows",
+                                         "tiles_per_band", "nbands", "reserved")]
+
+
+ROW_KERNELS = ("direct", "subwarp", "tiled", "tiled_subwarp")      # lec_dispatch.kernel (LEC_ROWS_*)
+
 LEC_RAW_F32, LEC_RAW_F64, LEC_RAW_I16 = 0, 1, 2
 _RAW_DTYPES = {np.dtype(np.float32): LEC_RAW_F32, np.dtype(np.float64): LEC_RAW_F64, np.dtype(np.int16): LEC_RAW_I16}
 
@@ -161,6 +168,8 @@ def load_library():
     lib.lec_unpin_host.restype = C.c_int
     lib.lec_launch_count.argtypes = [vp]
     lib.lec_launch_count.restype = C.c_int64
+    lib.lec_last_dispatch.argtypes = [vp, C.POINTER(_Dispatch)]
+    lib.lec_last_dispatch.restype = C.c_int
     lib.lec_diag850_host.argtypes = [C.POINTER(_DiagGrid), vp, vp, vp, C.c_int32, vp, C.c_int32, vp, vp]
     lib.lec_diag850_host.restype = C.c_int
     lib.lec_diag850_device.argtypes = [C.POINTER(_DiagGrid), vp, vp, vp, C.c_int32, vp, C.c_int32, vp, vp, vp]
@@ -536,6 +545,16 @@ class LecEngine:
         out = (C.c_int64 * 2)()
         self._check(self._lib.lec_last_transfer(self._h, out), "lec_last_transfer")
         return int(out[0]), int(out[1])
+
+    def last_dispatch(self) -> dict:
+        """Row kernel of the last kernel batch (``lec_last_dispatch``): ``kernel`` (one of :data:`ROW_KERNELS`),
+        ``vec``, ``group``, ``lonw``, ``comp``, ``math64``, ``tile_rows``, ``tiles_per_band``, ``nbands``."""
+        d = _Dispatch()
+        self._check(self._lib.lec_last_dispatch(self._h, C.byref(d)), "lec_last_dispatch")
+        out = {n: int(getattr(d, n)) for n, _ in _Dispatch._fields_ if n != "reserved"}
+        out["kernel"] = ROW_KERNELS[out["kernel"]]
+        out["comp"], out["math64"] = bool(out["comp"]), bool(out["math64"])
+        return out
 
     @property
     def launch_count(self) -> int:

@@ -21,12 +21,13 @@ SAM = os.path.join(H.GOLDEN, "samples")
 
 
 def _workdir(tmp_path, box=None, track=None):
+    # contents only (copyfile, not copy): the staged inputs stay writable when the checkout is read-only
     os.makedirs(tmp_path / "inputs")
-    shutil.copy(os.path.join(INP, "namelist_NCEP-R2"), tmp_path / "inputs" / "namelist")
+    shutil.copyfile(os.path.join(INP, "namelist_NCEP-R2"), tmp_path / "inputs" / "namelist")
     if box:
-        shutil.copy(os.path.join(INP, box), tmp_path / "inputs" / "box_limits")
+        shutil.copyfile(os.path.join(INP, box), tmp_path / "inputs" / "box_limits")
     if track:
-        shutil.copy(os.path.join(INP, track), tmp_path / "inputs" / "track")
+        shutil.copyfile(os.path.join(INP, track), tmp_path / "inputs" / "track")
 
 
 def test_cli_fixed_catarina_matches_bundled_results(tmp_path, monkeypatch):

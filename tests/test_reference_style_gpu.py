@@ -37,12 +37,14 @@ def _reference_flow(monkeypatch, argv, method):
 
 
 def _stage(tmp_path, monkeypatch, namelist, sample=None):
+    # contents only (copyfile, not copy): the staged inputs stay writable when the checkout is read-only, so the
+    # tests can put box_limits_Reg1 over box_limits as the reference's tests do
     os.makedirs(tmp_path / "inputs")
     os.makedirs(tmp_path / "samples")
     for f in os.listdir(INP):
-        shutil.copy(os.path.join(INP, f), tmp_path / "inputs" / f)
+        shutil.copyfile(os.path.join(INP, f), tmp_path / "inputs" / f)
     if sample:
-        shutil.copy(os.path.join(SAM, sample), tmp_path / "samples" / sample)
+        shutil.copyfile(os.path.join(SAM, sample), tmp_path / "samples" / sample)
     monkeypatch.chdir(tmp_path)
     shutil.copy(f"inputs/{namelist}", "inputs/namelist")
 

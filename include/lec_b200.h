@@ -190,6 +190,34 @@ int lec_run_host_raw(lec_handle *h, const lec_raw_desc *raw_desc, const void *co
                      const int32_t *slot_record, int32_t nslots, const lec_step *steps, int32_t nsteps,
                      double *out_terms, double *out_levels, int32_t *out_flags);
 
+/* ---- int16-packed fields resident in device memory ----------------------------------------------------
+ * lec_run_device for fields stored the way ERA5 and most reanalysis files store them: int16 with a per-field
+ * scale_factor / add_offset (2 bytes per value instead of the 4 or 8 of the decoded fields).  The row kernels decode
+ * every value they load by the rule of lec_run_host_raw:
+ *   x = double(raw);  x = x * scale (use_scale);  x = x + offset (use_offset)  (two roundings, no FMA)
+ *   x = double(float(x)) (round_f32);  raw == fill[0] (nfill >= 1) or raw == fill[1] (nfill >= 2) -> NaN
+ * and the value is x in the handle's dtype (LEC_F32 / LEC_F64); arithmetic as lec_run_device (desc.math), so the
+ * results have the bits of lec_run_device on the decoded fields.  Device data is native-endian.
+ * fields[f]: int16 [nslots][nlev][nlat][pitch], C order, 16-byte aligned; the pitch - nlon pad columns are never
+ * read into a result.  Everything else (steps, outputs, stream, batches of max_steps, lec_set_boundary_levels,
+ * timing, nsteps = 0) as lec_run_device.  LEC_ERR_INVALID for a pitch below nlon or not a multiple of 8, a
+ * misaligned field, nfill outside 0..2 or a fill value that is not an int16 value.  The row kernel is the TMA-tiled
+ * one for wide boxes and the sub-warp one for narrow boxes whatever LEC_ROW_KERNEL / LEC_NARROW_TILE say;
+ * lec_last_dispatch reports it with packed = 1. */
+typedef struct lec_packed_desc {
+  int32_t pitch;                 /* row length of the packed fields in elements: >= nlon, multiple of 8 (16 B) */
+  int32_t reserved;
+  double scale[5], offset[5];
+  int32_t use_scale[5], use_offset[5];
+  int32_t round_f32[5];
+  int32_t nfill[5];
+  double fill[5][2];
+} lec_packed_desc;
+
+int lec_run_device_packed(lec_handle *h, const lec_packed_desc *pd, const int16_t *const fields[5], int32_t nslots,
+                          const lec_step *steps, int32_t nsteps, double *out_terms, double *out_levels,
+                          int32_t *out_flags, void *stream);
+
 /* Optional extra output of every following lec_run_* on this handle: the 18 per-level boundary pieces
  *   out[step][LEC_NBOUNDARY_PIECES][nlev],  piece = 3 * term + part,
  *   term in BAz BAe BKz BKe BPhiZ BPhiE, part 0 = east-minus-west flux integrated over latitude,
@@ -240,7 +268,7 @@ typedef struct lec_dispatch {
   int32_t tile_rows;        /* box rows per tile (tiled kernels), per CTA otherwise */
   int32_t tiles_per_band;   /* tiles per latitude band of the block order */
   int32_t nbands;           /* latitude bands (1: step-major order) */
-  int32_t reserved;
+  int32_t packed;           /* 1: int16 fields decoded by the row kernel (lec_run_device_packed) */
 } lec_dispatch;
 int lec_last_dispatch(const lec_handle *h, lec_dispatch *out);
 

@@ -38,7 +38,6 @@ struct lec_handle {
   lec_grid_desc desc{};
   int device = 0;
   GridDev g{};
-  GridDev g_pad{};                               // same tables, rows padded to a whole number of 128-bit chunks
   int pitch = 0;                                 // row length of the engine's own staging (lec_run_host*)
   double* d_tables = nullptr;
   float* d_tables32 = nullptr;
@@ -161,19 +160,19 @@ void launch_rows(const lec_handle* h, const RowParams& rp, bool vec, bool comp, 
   }
 }
 
-template <typename FT, typename CT, int VEC, bool COMP>
+template <typename FT, typename CT, int VEC, bool COMP, typename ST>
 void launch_narrow_c(const RowParams& rp, bool table, int G, long long grid, cudaStream_t st) {
-#define LEC_NARROW(LW, GG) lec_row_moments_narrow_kernel<FT, CT, VEC, LW, GG, COMP><<<(unsigned)grid, kNarrowThreads, 0, st>>>(rp)
+#define LEC_NARROW(LW, GG) lec_row_moments_narrow_kernel<FT, CT, VEC, LW, GG, COMP, ST><<<(unsigned)grid, kNarrowThreads, 0, st>>>(rp)
   if (table) { if (G == 16) LEC_NARROW(2, 16); else if (G == 8) LEC_NARROW(2, 8); else LEC_NARROW(2, 4); }
   else { if (G == 16) LEC_NARROW(0, 16); else if (G == 8) LEC_NARROW(0, 8); else LEC_NARROW(0, 4); }
 #undef LEC_NARROW
 }
-template <typename FT, typename CT, int VEC>
+template <typename FT, typename CT, int VEC, typename ST = FT>
 void launch_narrow_t(const RowParams& rp, bool table, bool comp, int G, long long grid, cudaStream_t st) {
   if constexpr (sizeof(CT) == 4) {
-    if (comp) { launch_narrow_c<FT, CT, VEC, true>(rp, table, G, grid, st); return; }
+    if (comp) { launch_narrow_c<FT, CT, VEC, true, ST>(rp, table, G, grid, st); return; }
   }
-  launch_narrow_c<FT, CT, VEC, false>(rp, table, G, grid, st);
+  launch_narrow_c<FT, CT, VEC, false, ST>(rp, table, G, grid, st);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -192,39 +191,43 @@ EncodeTiledFn encode_tiled_fn() {
   return fn;
 }
 
-// 4-D tensor map over a [slot][level][lat][lon] field with a (bx x by) box in (lon, lat).
-bool make_map(CUtensorMap* m, const void* base, bool f64, int nlon, int nlat, int nlev, int nslots, int bx, int by,
+// 4-D tensor map over a [slot][level][lat][lon] field of `esize`-byte elements (fp64 / fp32 / int16) with a
+// (bx x by) box in (lon, lat).
+bool make_map(CUtensorMap* m, const void* base, int esize, int nlon, int nlat, int nlev, int nslots, int bx, int by,
               int promo = 3) {
   EncodeTiledFn enc = encode_tiled_fn();
   if (!enc) return false;
-  const cuuint64_t e = f64 ? 8 : 4;
+  const cuuint64_t e = (cuuint64_t)esize;
   const cuuint64_t dims[4] = {(cuuint64_t)nlon, (cuuint64_t)nlat, (cuuint64_t)nlev, (cuuint64_t)nslots};
   const cuuint64_t strides[3] = {nlon * e, (cuuint64_t)nlat * nlon * e, (cuuint64_t)nlev * nlat * nlon * e};
   const cuuint32_t box[4] = {(cuuint32_t)bx, (cuuint32_t)by, 1, 1};
   const cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, f64 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void*>(base),
+  // (int16 fields: the driver has no signed 16-bit type; TMA copies the bits unchanged, zero fill included)
+  const CUtensorMapDataType dt = esize == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64
+                                 : esize == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT16;
+  return enc(m, dt, 4, const_cast<void*>(base),
              dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
              promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : promo == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
              : promo == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <typename FT, typename CT, int R, int S, bool COMP, int GL = 32, int MINB = 1>
+template <typename FT, typename CT, int R, int S, bool COMP, int GL = 32, int MINB = 1, typename ST = FT>
 cudaError_t launch_tile_c(const TmaMaps& maps, const RowParams& rp, int lonw, int grid, cudaStream_t st) {
-  using G = TileGeom<FT, R, S, GL>;
+  using G = TileGeom<FT, R, S, GL, ST>;
   cudaError_t e = cudaSuccess;
 #define LEC_TILE_LAUNCH(LW, TB, SMEM)                                                                             \
   do {                                                                                                            \
-    e = cudaFuncSetAttribute(lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, GL, MINB>,              \
+    e = cudaFuncSetAttribute(lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, GL, MINB, ST>,          \
                              cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);                                  \
-    if (e == cudaSuccess) lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, GL, MINB><<<grid, G::threads, SMEM, st>>>(maps, rp); \
+    if (e == cudaSuccess) lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, GL, MINB, ST><<<grid, G::threads, SMEM, st>>>(maps, rp); \
   } while (0)
   if constexpr (GL != 32) {      // track boxes: no table / full tables, as the sub-warp kernel
     if (lonw == 0) LEC_TILE_LAUNCH(0, false, G::smem_bytes);
     else LEC_TILE_LAUNCH(2, false, G::smem_bytes);
   } else {
     // fp32 per-column weights (LONW == 1): table in shared memory when it fits behind the ring
-    const int tab_bytes = ((rp.g.nlon + 3) & ~3) * 4;
+    const int tab_bytes = (sizeof(ST) == sizeof(FT) ? (rp.g.nlon + 3) & ~3 : rp.pk.ntab) * 4;
     if (lonw == 0) LEC_TILE_LAUNCH(0, false, G::smem_bytes);
     else if (lonw == 1) {
       if (sizeof(CT) == 4 && sizeof(FT) == 4 && G::smem_bytes + tab_bytes <= 227 * 1024) LEC_TILE_LAUNCH(1, true, G::smem_bytes + tab_bytes);
@@ -256,6 +259,24 @@ cudaError_t launch_tile_t(const TmaMaps& maps, const RowParams& rp, int lonw, bo
     return launch_tile_c<FT, CT, 7, 6, false>(maps, rp, lonw, grid, st);      // fp32 fields, fp64 arithmetic (LEC_MATH_F64)
   } else {
     return launch_tile_c<FT, CT, 11, 4, false>(maps, rp, lonw, grid, st);
+  }
+}
+
+// Tile shapes over int16 fields: a stage holds about half (fp32) or a quarter (fp64) of the bytes, so the ring gets
+// more stages (at most 8: the barriers share the 128 bytes behind it).  fp32 arithmetic takes 11 rows, not 15: 15
+// consumer warps leave 128 registers and the decode's fp64 temporaries spill there (16-56 B).
+//   fp32 arithmetic, plain or compensated  11 rows x 7 stages  (196 KB)
+//   fp64 decode                            11 rows x 8 stages  (122 KB)
+//   fp32 decode, fp64 arithmetic            7 rows x 8 stages  (142 KB)
+template <typename FT, typename CT>
+cudaError_t launch_tile_packed(const TmaMaps& maps, const RowParams& rp, int lonw, bool comp, int grid, cudaStream_t st) {
+  if constexpr (sizeof(CT) == 4) {
+    if (comp) return launch_tile_c<FT, CT, 11, 7, true, 32, 1, short>(maps, rp, lonw, grid, st);
+    return launch_tile_c<FT, CT, 11, 7, false, 32, 1, short>(maps, rp, lonw, grid, st);
+  } else if constexpr (sizeof(FT) == 4) {
+    return launch_tile_c<FT, CT, 7, 8, false, 32, 1, short>(maps, rp, lonw, grid, st);
+  } else {
+    return launch_tile_c<FT, CT, 11, 8, false, 32, 1, short>(maps, rp, lonw, grid, st);
   }
 }
 
@@ -570,8 +591,6 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
   {
     const int vecw = desc->dtype == LEC_F64 ? 2 : 4;
     h->pitch = (nlon + vecw - 1) / vecw * vecw;
-    h->g_pad = g;
-    h->g_pad.nlon = h->pitch;
   }
 
   const size_t rec_bytes = (size_t)h->max_steps * L * h->max_ny * LEC_NREC * sizeof(double);
@@ -585,14 +604,17 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
   return LEC_OK;
 }
 
-// One kernel batch (<= max_steps steps) on `st`.
+// One kernel batch (<= max_steps steps) on `st`.  pitch: row length of the fields in elements (0: the grid's);
+// pk: the fields are int16, decoded by the row kernel (lec_run_device_packed).
 static int run_batch(lec_handle* h, const void* const fields[5], int nslots, const lec_step* steps, int n,
                      double* out_terms, double* out_levels, int* out_flags, double* out_bnd, cudaStream_t st,
-                     bool padded = false) {
-  // nlon below is the ROW LENGTH of the field buffers: the grid's for caller-owned device fields, the padded
-  // pitch for the engine's own staging (box indices are checked against the grid in build_step)
-  const int L = h->desc.nlev, nlon = padded ? h->pitch : h->desc.nlon;
-  const GridDev& gd = padded ? h->g_pad : h->g;
+                     int pitch = 0, const PackedDev* pk = nullptr) {
+  // nlon below is the ROW LENGTH of the field buffers: the grid's for caller-owned fp device fields, the padded
+  // pitch of the engine's own staging or of caller-owned int16 fields (box indices are checked against the grid
+  // in build_step)
+  const int L = h->desc.nlev, nlon = pitch > 0 ? pitch : h->desc.nlon;
+  GridDev gd = h->g;
+  gd.nlon = nlon;
   int max_rows = 0, max_cols = 0;
   bool same_box = true, same_rows = true;
   const int par = h->batch_parity;
@@ -625,6 +647,8 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   // latitude banding (fixed box, several steps): sweep time inside a band of box rows so T(t+-1) stays in L2
   int band_rows = h->desc.band_rows;
   if (band_rows <= 0) {
+    // (counted at the handle's element size for int16 fields too: they take the block order of lec_run_device on the
+    //  decoded fields; a budget for 2-byte values has not been measured)
     const double band_budget = 18e6;   // bytes of all five fields per band-step
     band_rows = int(band_budget / (5.0 * L * max_cols * h->elem));
   }
@@ -644,15 +668,17 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   // without it).  Tall boxes and short rows run the plain sums (7 % fewer FP instructions).
   int comp_mode = h->comp_mode;
   const bool comp = comp_mode == 1 || (comp_mode < 0 && max_chunks > 32 * 4 && max_rows <= 128);
-  // wide boxes: the TMA-tiled kernel (rows 16-byte aligned, a tensor-map encoder in the driver)
-  const bool want_tile = h->use_tile && vec && !narrow_g && encode_tiled_fn() != nullptr;
+  // wide boxes: the TMA-tiled kernel (rows 16-byte aligned, a tensor-map encoder in the driver); int16 fields have
+  // no other wide-box kernel (the caller's pitch makes every row 16-byte aligned)
+  const bool want_tile = (h->use_tile || pk) && vec && !narrow_g && encode_tiled_fn() != nullptr;
+  if (pk && !narrow_g && !want_tile) { h->err = "int16 fields need the TMA-tiled row kernel: no tensor-map encoder"; return LEC_ERR_CUDA; }
   // tile height: fp32 arithmetic fits 128 registers -> 15 consumer warps + the producer (16 warps, 3 stages);
   // fp64 arithmetic needs the 168 registers that at most 12 warps per CTA leave -> 11 rows, 4 stages
   const bool math64 = h->desc.dtype == LEC_F64 || h->desc.math == LEC_MATH_F64;
-  const int tile_R = (math64 && h->desc.dtype != LEC_F64) ? 7 : (math64 || comp) ? 11 : h->tile_rows;
+  const int tile_R = (math64 && h->desc.dtype != LEC_F64) ? 7 : (math64 || comp || pk) ? 11 : h->tile_rows;
   // track boxes (8-lane row groups), fp32 arithmetic: the same TMA ring with 13 consumer warps x 4 rows; the box is
   // cut into equal tiles of at most 52 rows
-  const bool want_ntile = h->use_tile && h->use_ntile && narrow_g == 8 && !math64 && !comp && encode_tiled_fn() != nullptr;
+  const bool want_ntile = !pk && h->use_tile && h->use_ntile && narrow_g == 8 && !math64 && !comp && encode_tiled_fn() != nullptr;
   int ntile_rows = 0;
   if (want_ntile) {
     const int nt = (max_rows + kNarrowTileRows - 1) / kNarrowTileRows;
@@ -680,6 +706,7 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   const long long grid = (long long)rp.nbands * n * L * rp.tiles_per_band;
   if (grid > 0x7fffffffLL) return LEC_ERR_INVALID;
   rp.grid = grid;
+  if (pk) rp.pk = *pk;
   // TMA loads of u, v, omega, Phi with an L2 evict-first hint: fp64 fields only (46.7 -> 39.0 GB of DRAM reads per
   // 24-step launch, +3.4 %; with fp32 fields the working set of a band fits without it and the hint costs 2 %)
   rp.prefetch_mode = h->prefetch_mode | ((h->tma_hint < 0 ? h->desc.dtype == LEC_F64 : h->tma_hint != 0) ? 8 : 0);
@@ -694,7 +721,7 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
     d.comp = comp && !math64;
     d.math64 = math64;
     d.tile_rows = tile_rows; d.tiles_per_band = rp.tiles_per_band; d.nbands = rp.nbands;
-    d.reserved = 0;
+    d.packed = pk != nullptr;
     h->dispatched = true;
   }
 
@@ -706,20 +733,26 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
     const bool f64 = h->desc.dtype == LEC_F64;
     const bool m64 = f64 || h->desc.math == LEC_MATH_F64;
     const int C = f64 ? 64 : 128, V = f64 ? 2 : 4, R = tile_R;
+    // box widths of TileGeom: int16 boxes have 8 more columns and a 16-byte halo on each side (aligned box starts)
+    const int esz = pk ? 2 : f64 ? 8 : 4, PW = pk ? C + 8 : C, HV = pk ? 8 : V;
     TmaMaps maps;
     const int nlat = h->desc.nlat;
-    bool ok = make_map(&maps.t_halo, fields[0], f64, nlon, nlat, L, nslots, C + 2 * V, R + 2) &&
-              make_map(&maps.t_plain, fields[0], f64, nlon, nlat, L, nslots, C, R) &&
-              make_map(&maps.u, fields[1], f64, nlon, nlat, L, nslots, C, R) &&
-              make_map(&maps.v, fields[2], f64, nlon, nlat, L, nslots, C, R) &&
-              make_map(&maps.w, fields[3], f64, nlon, nlat, L, nslots, C, R) &&
-              make_map(&maps.f, fields[4], f64, nlon, nlat, L, nslots, C, R);
+    bool ok = make_map(&maps.t_halo, fields[0], esz, nlon, nlat, L, nslots, PW + 2 * HV, R + 2) &&
+              make_map(&maps.t_plain, fields[0], esz, nlon, nlat, L, nslots, PW, R) &&
+              make_map(&maps.u, fields[1], esz, nlon, nlat, L, nslots, PW, R) &&
+              make_map(&maps.v, fields[2], esz, nlon, nlat, L, nslots, PW, R) &&
+              make_map(&maps.w, fields[3], esz, nlon, nlat, L, nslots, PW, R) &&
+              make_map(&maps.f, fields[4], esz, nlon, nlat, L, nslots, PW, R);
     if (!ok) { h->err = "cuTensorMapEncodeTiled failed"; return LEC_ERR_CUDA; }
     const int pgrid = (int)std::min<long long>(grid, (long long)h->num_sms);
     const int lonw = lon_mode(h);
-    cudaError_t e = f64 ? launch_tile_t<double, double>(maps, rp, lonw, comp, R, pgrid, st)
-                        : (m64 ? launch_tile_t<float, double>(maps, rp, lonw, comp, R, pgrid, st)
-                               : launch_tile_t<float, float>(maps, rp, lonw, comp, h->tile_rows, pgrid, st));
+    cudaError_t e;
+    if (pk) e = f64 ? launch_tile_packed<double, double>(maps, rp, lonw, comp, pgrid, st)
+                    : (m64 ? launch_tile_packed<float, double>(maps, rp, lonw, comp, pgrid, st)
+                           : launch_tile_packed<float, float>(maps, rp, lonw, comp, pgrid, st));
+    else e = f64 ? launch_tile_t<double, double>(maps, rp, lonw, comp, R, pgrid, st)
+                 : (m64 ? launch_tile_t<float, double>(maps, rp, lonw, comp, R, pgrid, st)
+                        : launch_tile_t<float, float>(maps, rp, lonw, comp, h->tile_rows, pgrid, st));
     if (e != cudaSuccess) { h->err = std::string("tiled row kernel launch: ") + cudaGetErrorString(e); return LEC_ERR_CUDA; }
     tma_done = true;
   }
@@ -728,12 +761,12 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
     TmaMaps maps;
     const int nlat = h->desc.nlat, R = ntile_rows;
     const int pm = 3;      // L2 promotion of the tensor maps: none / 64 B / 128 B / 256 B measured 2.09 / 2.16 / 2.10 / 2.06 ms
-    bool ok = make_map(&maps.t_halo, fields[0], false, nlon, nlat, L, nslots, C + 2 * V, R + 2, pm) &&
-              make_map(&maps.t_plain, fields[0], false, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.u, fields[1], false, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.v, fields[2], false, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.w, fields[3], false, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.f, fields[4], false, nlon, nlat, L, nslots, C, R, pm);
+    bool ok = make_map(&maps.t_halo, fields[0], 4, nlon, nlat, L, nslots, C + 2 * V, R + 2, pm) &&
+              make_map(&maps.t_plain, fields[0], 4, nlon, nlat, L, nslots, C, R, pm) &&
+              make_map(&maps.u, fields[1], 4, nlon, nlat, L, nslots, C, R, pm) &&
+              make_map(&maps.v, fields[2], 4, nlon, nlat, L, nslots, C, R, pm) &&
+              make_map(&maps.w, fields[3], 4, nlon, nlat, L, nslots, C, R, pm) &&
+              make_map(&maps.f, fields[4], 4, nlon, nlat, L, nslots, C, R, pm);
     if (!ok) { h->err = "cuTensorMapEncodeTiled failed"; return LEC_ERR_CUDA; }
     const int pgrid = (int)std::min<long long>(grid, (long long)h->num_sms * kNarrowTileCtas);
     cudaError_t e = launch_tile_c<float, float, kNarrowTileWarps, 3, false, 8, kNarrowTileCtas>(maps, rp, lon_mode(h), pgrid, st);
@@ -744,7 +777,11 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
     const bool f64 = h->desc.dtype == LEC_F64;
     const bool m64 = f64 || h->desc.math == LEC_MATH_F64;
     const bool table = lon_mode(h) != 0;
-    if (f64) launch_narrow_t<double, double, 2>(rp, table, comp, narrow_g, grid, st);
+    if (pk) {
+      if (f64) launch_narrow_t<double, double, 2, short>(rp, table, comp, narrow_g, grid, st);
+      else if (m64) launch_narrow_t<float, double, 4, short>(rp, table, comp, narrow_g, grid, st);
+      else launch_narrow_t<float, float, 4, short>(rp, table, comp, narrow_g, grid, st);
+    } else if (f64) launch_narrow_t<double, double, 2>(rp, table, comp, narrow_g, grid, st);
     else if (m64) launch_narrow_t<float, double, 4>(rp, table, comp, narrow_g, grid, st);
     else launch_narrow_t<float, float, 4>(rp, table, comp, narrow_g, grid, st);
     CK(cudaGetLastError());
@@ -769,11 +806,10 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   return LEC_OK;
 }
 
-int lec_run_device(lec_handle* h, const void* const fields[5], int32_t nslots, const lec_step* steps,
-                   int32_t nsteps, double* out_terms, double* out_levels, int32_t* out_flags, void* stream) {
-  if (h && nsteps == 0) return LEC_OK;      // an empty batch: nothing to launch, the (empty) outputs may be NULL
-  if (!h || !fields || !steps || nsteps < 0 || nslots < 1 || !out_terms) return LEC_ERR_INVALID;
-  for (int f = 0; f < 5; ++f) if (!fields[f]) return LEC_ERR_INVALID;
+// lec_run_device and lec_run_device_packed after their argument checks
+static int run_device_impl(lec_handle* h, const void* const fields[5], int32_t nslots, const lec_step* steps,
+                           int32_t nsteps, double* out_terms, double* out_levels, int32_t* out_flags, void* stream,
+                           int pitch = 0, const PackedDev* pk = nullptr) {
   CK(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int L = h->desc.nlev;
@@ -785,11 +821,52 @@ int lec_run_device(lec_handle* h, const void* const fields[5], int32_t nslots, c
     const int rc = run_batch(h, fields, nslots, steps + s0, n, out_terms + (size_t)s0 * LEC_NTERMS,
                              out_levels ? out_levels + (size_t)s0 * LEC_NLEVEL_TERMS * L : nullptr,
                              out_flags ? out_flags + s0 : nullptr,
-                             h->bnd_user ? h->bnd_user + (size_t)s0 * kNB * L : nullptr, st);
+                             h->bnd_user ? h->bnd_user + (size_t)s0 * kNB * L : nullptr, st, pitch, pk);
     if (rc != LEC_OK) return rc;
   }
   CK(cudaEventRecord(h->ev_call1, st));
   return LEC_OK;
+}
+
+int lec_run_device(lec_handle* h, const void* const fields[5], int32_t nslots, const lec_step* steps,
+                   int32_t nsteps, double* out_terms, double* out_levels, int32_t* out_flags, void* stream) {
+  if (h && nsteps == 0) return LEC_OK;      // an empty batch: nothing to launch, the (empty) outputs may be NULL
+  if (!h || !fields || !steps || nsteps < 0 || nslots < 1 || !out_terms) return LEC_ERR_INVALID;
+  for (int f = 0; f < 5; ++f) if (!fields[f]) return LEC_ERR_INVALID;
+  return run_device_impl(h, fields, nslots, steps, nsteps, out_terms, out_levels, out_flags, stream);
+}
+
+int lec_run_device_packed(lec_handle* h, const lec_packed_desc* pd, const int16_t* const fields[5], int32_t nslots,
+                          const lec_step* steps, int32_t nsteps, double* out_terms, double* out_levels,
+                          int32_t* out_flags, void* stream) {
+  if (h && nsteps == 0) return LEC_OK;
+  if (!h || !pd || !fields || !steps || nsteps < 0 || nslots < 1 || !out_terms) return LEC_ERR_INVALID;
+  if (pd->pitch < h->desc.nlon || pd->pitch % 8 != 0) {
+    h->err = "pitch must be at least nlon and a multiple of 8 elements (16-byte rows)";
+    return LEC_ERR_INVALID;
+  }
+  PackedDev pk{};
+  const void* ptrs[5];
+  for (int f = 0; f < 5; ++f) {
+    if (!fields[f] || reinterpret_cast<uintptr_t>(fields[f]) % 16 != 0) {
+      h->err = "int16 fields must be 16-byte aligned device pointers";
+      return LEC_ERR_INVALID;
+    }
+    if (pd->nfill[f] < 0 || pd->nfill[f] > 2) { h->err = "at most two fill values per field"; return LEC_ERR_INVALID; }
+    int fill[2] = {kNoFill, kNoFill};
+    for (int n = 0; n < pd->nfill[f]; ++n) {
+      const double v = pd->fill[f][n];
+      if (!(v >= -32768.0 && v <= 32767.0 && v == std::floor(v))) { h->err = "a fill value is not an int16 value"; return LEC_ERR_INVALID; }
+      fill[n] = (int)v;
+    }
+    pk.fill0[f] = fill[0]; pk.fill1[f] = fill[1];
+    pk.scale[f] = pd->use_scale[f] ? pd->scale[f] : 1.0;
+    pk.offset[f] = pd->use_offset[f] ? pd->offset[f] : -0.0;
+    pk.round32[f] = pd->round_f32[f] != 0;
+    ptrs[f] = fields[f];
+  }
+  pk.ntab = (h->desc.nlon + 3) & ~3;
+  return run_device_impl(h, ptrs, nslots, steps, nsteps, out_terms, out_levels, out_flags, stream, pd->pitch, &pk);
 }
 
 // Where lec_run_host* takes its slots from: engine-layout host arrays, or raw records + index maps.
@@ -1023,7 +1100,7 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
     const int rc = run_batch(h, h->stage[b], hi - lo + 1, local.data(), s1 - s0,
                              h->d_out_terms + (size_t)s0 * LEC_NTERMS,
                              h->d_out_levels + (size_t)s0 * LEC_NLEVEL_TERMS * L, h->d_out_flags + s0,
-                             h->bnd_user ? h->d_out_bnd + (size_t)s0 * kNB * L : nullptr, h->s_comp, true);
+                             h->bnd_user ? h->d_out_bnd + (size_t)s0 * kNB * L : nullptr, h->s_comp, h->pitch);
     if (rc != LEC_OK) return rc;
     CK(cudaEventRecord(h->ev_done[b], h->s_comp));
     s0 = s1; ++chunk;

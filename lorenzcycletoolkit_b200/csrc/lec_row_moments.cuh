@@ -52,6 +52,17 @@ struct FastDiv {
   }
 };
 
+// Decode of int16 fields resident in device memory (lec_run_device_packed), per field: the rule of lec_ingest_kernel
+// with the switches folded into the constants (no scale: 1.0; no offset: -0.0, which adds exactly nothing, signed
+// zeros included) and the fill values as raw integers (kNoFill never matches an int16).
+constexpr int kNoFill = 0x10000;
+struct PackedDev {
+  double scale[5], offset[5];
+  int fill0[5], fill1[5];
+  int round32[5];          // fp64 fields: the decoded variable is float32 (rounded once)
+  int ntab;                // longitude-table entries of the tiled kernel's shared copy (the row pitch may be longer)
+};
+
 struct RowParams {
   const void* field[5];
   GridDev g;
@@ -66,6 +77,7 @@ struct RowParams {
   long long slot_stride; // elements per slot = nlev*nlat*nlon
   int prefetch_mode;     // bit 0: L2 bulk prefetch of the DRAM-sourced rows at row start
   long long grid;        // number of CTAs
+  PackedDev pk;          // int16 instances only
 };
 
 // TMA bulk prefetch of a byte range into L2 (no destination, no completion tracking).
@@ -99,6 +111,56 @@ template <> struct VecLoad<double, 2> {
 template <typename FT> struct VecLoad<FT, 1> {
   static __device__ __forceinline__ void ld(const FT* p, FT (&v)[1]) { v[0] = __ldg(p); }
   static __device__ __forceinline__ void ld_stream(const FT* p, FT (&v)[1]) { v[0] = __ldcs(p); }
+};
+
+// One int16 element of field F decoded to FT: x = double(raw) * scale + offset (two roundings, no FMA), rounded
+// through float32 where the decoded variable is float32, NaN for a fill value -- lec_ingest_kernel's rule, so the
+// row kernels see the bits lec_run_device sees on the decoded fields.  (A float32 FT rounds once anyway.)
+// NAN_OR: how a float32 value becomes NaN -- a select, or an integer OR into x (the same bits); which of the two
+// builds without spills depends on the kernel (ptxas: the sub-warp kernel wants the select, the tiled one the OR).
+template <typename FT, int F, bool NAN_OR = false>
+__device__ __forceinline__ FT unpack_i16(short raw, const PackedDev& pk) {
+  const double x = __dadd_rn(__dmul_rn(double(raw), pk.scale[F]), pk.offset[F]);
+  const bool fill = int(raw) == pk.fill0[F] || int(raw) == pk.fill1[F];
+  if constexpr (sizeof(FT) == 8) {
+    return fill ? __longlong_as_double(0x7ff8000000000000LL) : pk.round32[F] ? double(float(x)) : x;
+  } else if constexpr (NAN_OR) {
+    // a fill sets the exponent and quiet bit of x: a NaN, whose float32 conversion is the canonical NaN
+    return float(__hiloint2double(__double2hiint(x) | (fill ? 0x7ff80000 : 0), __double2loint(x)));
+  } else {
+    return fill ? __int_as_float(0x7fffffff) : float(x);    // = float(NaN)
+  }
+}
+
+template <typename FT, int VEC, int F, bool NAN_OR = false>
+__device__ __forceinline__ void unpack_i16_vec(unsigned lo, unsigned hi, FT (&v)[VEC], const PackedDev& pk) {
+  v[0] = unpack_i16<FT, F, NAN_OR>(short(lo & 0xffffu), pk);
+  v[1] = unpack_i16<FT, F, NAN_OR>(short(lo >> 16), pk);
+  if constexpr (VEC == 4) {
+    v[2] = unpack_i16<FT, F, NAN_OR>(short(hi & 0xffffu), pk);
+    v[3] = unpack_i16<FT, F, NAN_OR>(short(hi >> 16), pk);
+  }
+}
+
+// Global loads of the row kernels by stored element type ST: the float types load as stored (VecLoad); int16 loads
+// the lane's VEC values (8 bytes for fp32, 4 for fp64) and decodes them.  F = field (LEC_FIELD_*).
+template <typename ST, typename FT, int VEC>
+struct RowLoad {
+  template <int F> static __device__ __forceinline__ void ld(const ST* p, FT (&v)[VEC], const PackedDev&) { VecLoad<FT, VEC>::ld(p, v); }
+  template <int F> static __device__ __forceinline__ FT one(const ST* p, const PackedDev&) { return __ldg(p); }
+};
+template <typename FT, int VEC>
+struct RowLoad<short, FT, VEC> {
+  static_assert(VEC == 4 || VEC == 2, "int16 rows are read in the chunks of the vector kernels");
+  template <int F> static __device__ __forceinline__ void ld(const short* p, FT (&v)[VEC], const PackedDev& pk) {
+    if constexpr (VEC == 4) {
+      const uint2 t = __ldg(reinterpret_cast<const uint2*>(p));
+      unpack_i16_vec<FT, VEC, F>(t.x, t.y, v, pk);
+    } else {
+      unpack_i16_vec<FT, VEC, F>(__ldg(reinterpret_cast<const unsigned*>(p)), 0u, v, pk);
+    }
+  }
+  template <int F> static __device__ __forceinline__ FT one(const short* p, const PackedDev& pk) { return unpack_i16<FT, F>(__ldg(p), pk); }
 };
 
 __device__ __forceinline__ double shfl_xor_f64(double v, int m) {

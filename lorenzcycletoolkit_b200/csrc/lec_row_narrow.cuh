@@ -48,8 +48,10 @@ __device__ __forceinline__ int bitrev_group(int gl) {
   return r;
 }
 
-template <typename FT, typename CT, int VEC, int LONW, int G, bool COMP>
-__global__ void __launch_bounds__(kNarrowThreads, (sizeof(CT) == 8 ? 384 : 512) / kNarrowThreads)   // fp64 arithmetic: 12 warps/SM, 168 registers
+// ST: stored element type -- FT, or int16 decoded on load (lec_run_device_packed; RowParams::pk)
+template <typename FT, typename CT, int VEC, int LONW, int G, bool COMP, typename ST = FT>
+// fp64 arithmetic: 12 warps/SM, 168 registers; fp32 values decoded from int16 in fp64 arithmetic: 8 warps/SM, 255 registers
+__global__ void __launch_bounds__(kNarrowThreads, (sizeof(CT) == 8 ? (sizeof(ST) == 2 && sizeof(FT) == 4 ? 256 : 384) : 512) / kNarrowThreads)
 lec_row_moments_narrow_kernel(const RowParams p) {
   constexpr int RPW = 32 / G;                     // rows per warp
   const int warp = threadIdx.x >> 5, lane31 = threadIdx.x & 31;
@@ -73,11 +75,11 @@ lec_row_moments_narrow_kernel(const RowParams p) {
 
   const long long plane = (long long)nlat * nlon;
   const long long row_c = ((long long)st->slot * nlev + k) * plane + (long long)j * nlon;
-  const FT* __restrict__ Tc_row = static_cast<const FT*>(p.field[0]) + row_c;
-  const FT* __restrict__ U_row = static_cast<const FT*>(p.field[1]) + row_c;
-  const FT* __restrict__ V_row = static_cast<const FT*>(p.field[2]) + row_c;
-  const FT* __restrict__ W_row = static_cast<const FT*>(p.field[3]) + row_c;
-  const FT* __restrict__ F_row = static_cast<const FT*>(p.field[4]) + row_c;
+  const ST* __restrict__ Tc_row = static_cast<const ST*>(p.field[0]) + row_c;
+  const ST* __restrict__ U_row = static_cast<const ST*>(p.field[1]) + row_c;
+  const ST* __restrict__ V_row = static_cast<const ST*>(p.field[2]) + row_c;
+  const ST* __restrict__ W_row = static_cast<const ST*>(p.field[3]) + row_c;
+  const ST* __restrict__ F_row = static_cast<const ST*>(p.field[4]) + row_c;
   const int d_m = int((long long)(st->slot_m - st->slot) * p.slot_stride);
   const int d_p = int((long long)(st->slot_p - st->slot) * p.slot_stride);
   const int d_km = (k > 0) ? -int(plane) : 0, d_kp = (k < nlev - 1) ? int(plane) : 0;
@@ -88,9 +90,10 @@ lec_row_moments_narrow_kernel(const RowParams p) {
   // prefetch.global.L2 per stream (the bulk form is serialised through the uniform datapath and was slower)
   // Straight-line on purpose (lines 1 .. G-1, clamped to the row end): the same prefetches inside a per-lane loop
   // over all lines of a longer row measured SLOWER than no prefetch (2.05 vs 1.99 ms), straight-line 1.83 ms on the
-  // C5 track; 61-column boxes 0.49 -> 0.46 ms, 301-column boxes 7.66 -> 7.50 ms.
+  // C5 track; 61-column boxes 0.49 -> 0.46 ms, 301-column boxes 7.66 -> 7.50 ms.  The stride is the bytes of one
+  // fp sweep iteration whatever the stored type (int16 rows: lines 1 .. G-1 of the row, two iterations each).
   if ((p.prefetch_mode & 16) && lane >= 1) {
-    const int pc = min(i0 + lane * (G * VEC), i1);
+    const int pc = min(i0 + lane * (G * VEC * (int)sizeof(FT) / (int)sizeof(ST)), i1);
     asm volatile("prefetch.global.L2 [%0];" ::"l"(U_row + pc));
     asm volatile("prefetch.global.L2 [%0];" ::"l"(V_row + pc));
     asm volatile("prefetch.global.L2 [%0];" ::"l"(W_row + pc));
@@ -105,8 +108,10 @@ lec_row_moments_narrow_kernel(const RowParams p) {
   [[maybe_unused]] const double fxd = rs.fxd;
   const bool box_aligned = (i0 % VEC == 0) && ((i1 + 1) % VEC == 0);
 
-  const FT shT = __ldg(Tc_row + i0), shU = __ldg(U_row + i0), shV = __ldg(V_row + i0),
-           shW = __ldg(W_row + i0), shF = __ldg(F_row + i0);
+  using LD = RowLoad<ST, FT, VEC>;
+  const FT shT = LD::template one<0>(Tc_row + i0, p.pk), shU = LD::template one<1>(U_row + i0, p.pk),
+           shV = LD::template one<2>(V_row + i0, p.pk), shW = LD::template one<3>(W_row + i0, p.pk),
+           shF = LD::template one<4>(F_row + i0, p.pk);
   const CT cshT = CT(shT), cshU = CT(shU), cshV = CT(shV), cshW = CT(shW), cshF = CT(shF);
 
   CT S[R_NSUM], Cc[R_NLIN];

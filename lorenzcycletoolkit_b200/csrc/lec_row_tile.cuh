@@ -39,21 +39,31 @@ struct alignas(64) TmaMaps {
 // carries 32/GL rows, a chunk is GL x 128 bit wide -- the lane <-> row / column mapping of the sub-warp kernel).
 // R = consumer warps; a tile has up to R * 32/GL rows (the host picks the height actually used, RowParams::tile_rows,
 // so that a box of any height is cut into equal tiles -- the TMA box height lives in the tensor map, not in the code).
-template <typename FT, int R, int NSTG, int GL = 32>
+// ST = stored element type: FT, or int16 (lec_run_device_packed), which keeps the lane <-> column map of FT (VEC) and
+// shrinks the ring's bytes.  Every TMA box starts on a 16-byte boundary of the row: the fp chunks do by construction
+// (VEC columns = 16 bytes), an int16 chunk starts at column c0 * VEC, a multiple of 4 (fp32) or 2 (fp64) only, so the
+// int16 boxes start at that column rounded down to a multiple of 8 and are 8 columns wider (PW); the consumers add the
+// row's shift (c0 * VEC) & 7.  The int16 lon halo is 8 columns (16 bytes) a side.
+template <typename FT, int R, int NSTG, int GL = 32, typename ST = FT>
 struct TileGeom {
+  static constexpr bool I16 = sizeof(ST) != sizeof(FT);
   static constexpr int VEC = 16 / sizeof(FT);
+  static constexpr int HV = I16 ? 8 : VEC;                   // lon halo columns each side (16 bytes)
   static constexpr int RPW = 32 / GL;                        // rows per consumer warp
   static constexpr int ROWS = R * RPW;                       // most rows a tile can hold
   static constexpr int C = GL * VEC;                         // columns per chunk
-  static constexpr int HP = C + 2 * VEC;                     // halo tile pitch (elements)
-  static constexpr int halo_bytes = (ROWS + 2) * HP * sizeof(FT);
+  static constexpr int PW = I16 ? C + 8 : C;                 // plain tile pitch (elements)
+  static constexpr int HP = PW + 2 * HV;                     // halo tile pitch (elements)
+  static_assert(HP * sizeof(ST) % 16 == 0 && PW * sizeof(ST) % 16 == 0, "TMA boxes are whole 16-byte units wide");
+  static constexpr int halo_bytes = (ROWS + 2) * HP * sizeof(ST);
   static constexpr int halo_bytes_pad = (halo_bytes + 127) / 128 * 128;
-  static constexpr int tile_bytes = ROWS * C * sizeof(FT);
+  // (int16: every plain tile starts on a 128-byte boundary, the alignment of a TMA destination)
+  static constexpr int tile_bytes = I16 ? (ROWS * PW * (int)sizeof(ST) + 127) / 128 * 128 : ROWS * C * sizeof(ST);
   static constexpr int stage_bytes = halo_bytes_pad + 8 * tile_bytes;
   static constexpr int smem_bytes = NSTG * stage_bytes + 128;               // + barriers
   static constexpr int threads = (R + 1) * 32;                           // R consumer warps + the producer warp
   // what the 9 loads of a chunk deliver when the tile is `rows` high
-  static __host__ __device__ constexpr int tx_bytes(int rows) { return ((rows + 2) * HP + 8 * rows * C) * (int)sizeof(FT); }
+  static __host__ __device__ constexpr int tx_bytes(int rows) { return ((rows + 2) * HP + 8 * rows * PW) * (int)sizeof(ST); }
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -118,6 +128,31 @@ __device__ __forceinline__ float lds_one(unsigned a, float) {
 __device__ __forceinline__ double lds_one(unsigned a, double) {
   double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v;
 }
+// the same by stored type: int16 vectors (8 or 4 bytes) and elements are decoded (F = field)
+template <typename ST, typename FT, int VEC, int F>
+__device__ __forceinline__ void lds_row(unsigned a, FT (&v)[VEC], const PackedDev& pk) {
+  if constexpr (sizeof(ST) == sizeof(FT)) {
+    lds_vec<FT, VEC>(a, v);
+  } else if constexpr (VEC == 4) {
+    unsigned lo, hi;
+    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(lo), "=r"(hi) : "r"(a));
+    unpack_i16_vec<FT, VEC, F, true>(lo, hi, v, pk);
+  } else {
+    unsigned lo;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(lo) : "r"(a));
+    unpack_i16_vec<FT, VEC, F, true>(lo, 0u, v, pk);
+  }
+}
+template <typename ST, typename FT, int F>
+__device__ __forceinline__ FT lds_elem(unsigned a, const PackedDev& pk) {
+  if constexpr (sizeof(ST) == sizeof(FT)) {
+    return lds_one(a, FT());
+  } else {
+    unsigned short r;
+    asm volatile("ld.shared.u16 %0, [%1];" : "=h"(r) : "r"(a));
+    return unpack_i16<FT, F, true>(short(r), pk);
+  }
+}
 
 // longitude-table load of the shared body: from shared memory (plain load, address space known) or global
 template <bool SHARED, int VEC>
@@ -151,11 +186,12 @@ __device__ __forceinline__ TileId decode_tile(unsigned id, const RowParams& p) {
 }
 
 // MINB = CTAs per SM (1; two to four smaller CTAs at different phases were tried for track boxes and were slower)
-template <typename FT, typename CT, int LONW, int R, int NSTG, bool COMP, bool TABS, int GL = 32, int MINB = 1>
+template <typename FT, typename CT, int LONW, int R, int NSTG, bool COMP, bool TABS, int GL = 32, int MINB = 1, typename ST = FT>
 __global__ void __launch_bounds__((R + 1) * 32, MINB)
 lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParams p) {
-  using G = TileGeom<FT, R, NSTG, GL>;
-  constexpr int VEC = G::VEC, C = G::C, HP = G::HP, RPW = G::RPW;
+  using G = TileGeom<FT, R, NSTG, GL, ST>;
+  constexpr int VEC = G::VEC, C = G::C, PW = G::PW, HP = G::HP, HV = G::HV, RPW = G::RPW;
+  static_assert(!G::I16 || GL == 32, "int16 fields: one warp per row");
   // rows of a tile = the TMA box height: R for a warp per row (compile-time tile offsets), chosen by the host for
   // track boxes (<= G::ROWS)
   const int trows = (GL == 32) ? R : p.tile_rows;
@@ -173,7 +209,9 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
   const float* wl_tab = p.g.wl32;
   if constexpr (TABS) {
     float* wl_s = reinterpret_cast<float*>(smem + G::smem_bytes);
-    for (int i = threadIdx.x; i < p.g.nlon; i += blockDim.x) wl_s[i] = __ldg(p.g.wl32 + i);
+    int ntab = p.g.nlon;                         // = the row length of fp fields (whole 128-bit chunks here)
+    if constexpr (sizeof(ST) != sizeof(FT)) ntab = p.pk.ntab;
+    for (int i = threadIdx.x; i < ntab; i += blockDim.x) wl_s[i] = __ldg(p.g.wl32 + i);
     wl_tab = wl_s;
   }
   __syncthreads();
@@ -196,11 +234,13 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
         const int c0 = st->i0 / VEC, c1 = st->i1 / VEC;
         const int nch = (c1 - c0 + GL) / GL;
         const unsigned tx = (unsigned)G::tx_bytes(trows);
-        const unsigned tile_b = (unsigned)(trows * C * (int)sizeof(FT));    // the plain tiles are packed at the runtime height
+        // the plain tiles are packed at the runtime height (int16: one warp per row, so trows == R)
+        const unsigned tile_b = G::I16 ? (unsigned)G::tile_bytes : (unsigned)(trows * C * (int)sizeof(ST));
         const int jt0 = st->j0 + jr;
         const int k = t.k, km = k > 0 ? k - 1 : k, kp = k < nlev - 1 ? k + 1 : k;
         const int slot = st->slot, slot_m = st->slot_m, slot_p = st->slot_p;
         int col = c0 * VEC;
+        if constexpr (G::I16) col &= ~7;             // 16-byte aligned box start
         for (int ch = 0; ch < nch; ++ch, col += C) {
           mbar_wait(empty0 + 8 * stg, phase ^ 1);
           const unsigned fb = full0 + 8 * stg;
@@ -211,7 +251,7 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
           }
           mbar_expect_tx(fb, tx);
           const unsigned base = smem_u32(smem) + (unsigned)stg * G::stage_bytes;
-          tma_load_4d(base, &maps.t_halo, fb, col - VEC, jt0 - 1, k, slot);
+          tma_load_4d(base, &maps.t_halo, fb, col - HV, jt0 - 1, k, slot);
           unsigned d = base + G::halo_bytes_pad;
           if (p.prefetch_mode & 8) {
             tma_load_4d_hint(d, &maps.u, fb, col, jt0, k, slot, pol_stream); d += tile_b;
@@ -240,9 +280,9 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
   const unsigned sbase0 = smem_u32(smem);
   const int gl = lane & (GL - 1);                      // lane within the row's group
   const int rowt = warp * RPW + lane / GL;             // row within the tile
-  const unsigned off_hc = (unsigned)(((rowt + 1) * HP + VEC + gl * VEC) * sizeof(FT));
-  const unsigned off_t = (unsigned)(G::halo_bytes_pad + (rowt * C + gl * VEC) * sizeof(FT));
-  const unsigned kTile = (unsigned)(trows * C * (int)sizeof(FT));
+  const unsigned off_hc = (unsigned)(((rowt + 1) * HP + HV + gl * VEC) * sizeof(ST));
+  const unsigned off_t = (unsigned)(G::halo_bytes_pad + (rowt * PW + gl * VEC) * sizeof(ST));
+  const unsigned kTile = G::I16 ? (unsigned)G::tile_bytes : (unsigned)(trows * C * (int)sizeof(ST));
   // current stage: base address, its full barrier (the empty one sits 8 NSTG bytes behind it), index, phase; the
   // advance wraps by subtraction, so the ring needs no second copy of the base addresses in registers
   unsigned sb = sbase0, fb = full0;
@@ -266,6 +306,8 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
     const int k = t.k;
     const int c0 = i0 / VEC, c1 = i1 / VEC;
     const int niter = (c1 - c0 + GL) / GL;
+    // int16: the row's first chunk sits this many bytes into the (16-byte aligned) boxes; 0 for fp fields
+    const unsigned adj = G::I16 ? (unsigned)(((c0 * VEC) & 7) * (int)sizeof(ST)) : 0u;
 
     // (No L2 prefetch here: bulk prefetches of the next tile's rows -- issued by the producer thread or by the
     //  consumer warps -- were measured at 3.1-3.7 TB/s against 5.3-5.5 without; the ring alone covers DRAM latency.)
@@ -277,8 +319,8 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
     const bool box_aligned = (i0 % VEC == 0) && ((i1 + 1) % VEC == 0);
     // at the box edges the j-1 / j+1 row falls back to the own row (its stencil coefficient is zero;
     // values outside the box are never touched)
-    const unsigned off_hm = (j > j0) ? off_hc - (unsigned)(HP * sizeof(FT)) : off_hc;
-    const unsigned off_hp = (j < j1) ? off_hc + (unsigned)(HP * sizeof(FT)) : off_hc;
+    const unsigned off_hm = (j > j0) ? off_hc - (unsigned)(HP * sizeof(ST)) : off_hc;
+    const unsigned off_hp = (j < j1) ? off_hc + (unsigned)(HP * sizeof(ST)) : off_hc;
 
     FT shT = FT(0), shU = FT(0), shV = FT(0), shW = FT(0), shF = FT(0);
     CT cshT = CT(0), cshU = CT(0), cshV = CT(0), cshW = CT(0), cshF = CT(0);

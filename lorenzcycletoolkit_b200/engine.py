@@ -62,9 +62,16 @@ class _RawDesc(C.Structure):
                 ("big_endian", C.c_int32), ("reserved", C.c_int32), ("record_stride", C.c_int64 * 5)]
 
 
+class _PackedDesc(C.Structure):
+    _fields_ = [("pitch", C.c_int32), ("reserved", C.c_int32),
+                ("scale", C.c_double * 5), ("offset", C.c_double * 5),
+                ("use_scale", C.c_int32 * 5), ("use_offset", C.c_int32 * 5), ("round_f32", C.c_int32 * 5),
+                ("nfill", C.c_int32 * 5), ("fill", (C.c_double * 2) * 5)]
+
+
 class _Dispatch(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("kernel", "vec", "group", "lonw", "comp", "math64", "tile_rows",
-                                         "tiles_per_band", "nbands", "reserved")]
+                                         "tiles_per_band", "nbands", "packed")]
 
 
 ROW_KERNELS = ("direct", "subwarp", "tiled", "tiled_subwarp")      # lec_dispatch.kernel (LEC_ROWS_*)
@@ -145,6 +152,9 @@ def load_library():
     lib.lec_destroy.restype = C.c_int
     lib.lec_run_device.argtypes = [vp, C.POINTER(vp), C.c_int32, vp, C.c_int32, vp, vp, vp, vp]
     lib.lec_run_device.restype = C.c_int
+    lib.lec_run_device_packed.argtypes = [vp, C.POINTER(_PackedDesc), C.POINTER(vp), C.c_int32, vp, C.c_int32, vp, vp, vp,
+                                          vp]
+    lib.lec_run_device_packed.restype = C.c_int
     lib.lec_run_host.argtypes = [vp, C.POINTER(vp), C.c_int32, vp, C.c_int32, vp, vp, vp]
     lib.lec_run_host.restype = C.c_int
     lib.lec_run_host_raw.argtypes = [vp, C.POINTER(_RawDesc), C.POINTER(vp), C.c_int32, vp, C.c_int32, vp, C.c_int32,
@@ -292,6 +302,27 @@ def pin_arrays(arrays, limit_bytes=None):
         ref = None
     _PINNED[lo] = (hi - lo, ref)
     return True
+
+
+def _set_decode(d, decode, strict=False):
+    """Fill the decode fields (scale, offset, use_*, round_f32, nfill, fill) that ``lec_raw_desc`` and
+    ``lec_packed_desc`` share from per-field dicts ``scale``, ``offset``, ``fills``, ``float32``.  ``strict``: more than
+    two fill values, or one that is not an int16 value, is an error (otherwise the first two are used)."""
+    for f, dec in enumerate(decode or [{}] * 5):
+        d.scale[f] = float(dec.get("scale", 1.0) if dec.get("scale") is not None else 1.0)
+        d.offset[f] = float(dec.get("offset", 0.0) if dec.get("offset") is not None else 0.0)
+        d.use_scale[f] = int(dec.get("scale") is not None)
+        d.use_offset[f] = int(dec.get("offset") is not None)
+        d.round_f32[f] = int(bool(dec.get("float32", False)))
+        fills = list(dec.get("fills", ()))
+        if strict and (len(fills) > 2 or any(not (float(v) == int(v) and -32768 <= int(v) <= 32767)
+                                             for v in fills if np.isfinite(float(v)))
+                       or not all(np.isfinite(float(v)) for v in fills)):
+            raise ValueError(f"field {f}: int16 decoding takes at most two fill values, each an int16 value (got {fills})")
+        fills = fills[:2]
+        d.nfill[f] = len(fills)
+        for n, fv in enumerate(fills):
+            d.fill[f][n] = float(fv)
 
 
 def make_steps(nsteps: int) -> np.ndarray:
@@ -455,16 +486,7 @@ class LecEngine:
             d.record_stride[f] = int(a.strides[0])
         ip = C.POINTER(C.c_int32)
         d.lon_map, d.lat_map, d.lev_map = (m.ctypes.data_as(ip) for m in maps)
-        for f, dec in enumerate(decode or [{}] * 5):
-            d.scale[f] = float(dec.get("scale", 1.0) if dec.get("scale") is not None else 1.0)
-            d.offset[f] = float(dec.get("offset", 0.0) if dec.get("offset") is not None else 0.0)
-            d.use_scale[f] = int(dec.get("scale") is not None)
-            d.use_offset[f] = int(dec.get("offset") is not None)
-            d.round_f32[f] = int(bool(dec.get("float32", False)))
-            fills = list(dec.get("fills", ()))[:2]
-            d.nfill[f] = len(fills)
-            for n, fv in enumerate(fills):
-                d.fill[f][n] = float(fv)
+        _set_decode(d, decode)
         steps, sp = self._steps_arg(steps)
         n = steps.size
         terms = np.empty((n, NTERMS), dtype=np.float64)
@@ -530,6 +552,67 @@ class LecEngine:
                         levels.data_ptr() if levels is not None else None, flags.data_ptr(), stream)
         return terms, levels, flags
 
+    def run_device_packed(self, field_ptrs, nslots, pitch, decode, steps, out_terms_ptr, out_levels_ptr=None,
+                          out_flags_ptr=None, stream=None):
+        """``lec_run_device_packed`` on raw device pointers (ints) to int16 fields ``[slot][level][lat][pitch]``;
+        ``decode`` = per field a dict as in :meth:`run_host_raw`; asynchronous on ``stream``."""
+        d = _PackedDesc()
+        d.pitch = int(pitch)
+        _set_decode(d, decode, strict=True)
+        steps, sp = self._steps_arg(steps)
+        ptrs = (C.c_void_p * 5)(*[int(p) for p in field_ptrs])
+        rc = self._lib.lec_run_device_packed(self._h, C.byref(d), ptrs, int(nslots), sp, steps.size,
+                                             C.c_void_p(int(out_terms_ptr)),
+                                             C.c_void_p(int(out_levels_ptr)) if out_levels_ptr else None,
+                                             C.c_void_p(int(out_flags_ptr)) if out_flags_ptr else None,
+                                             C.c_void_p(int(stream)) if stream else None)
+        self._check(rc, "lec_run_device_packed")
+
+    def run_torch_packed(self, fields, decode, steps, want_levels=True, out=None):
+        """:meth:`run_torch` for five int16 CUDA tensors that stay packed in device memory (2 bytes per value):
+        ``[slot][level][lat][n]`` with contiguous rows ``pitch = stride(2)`` elements apart, a multiple of 8, and
+        ``nlon <= n <= pitch`` (the padded rows :func:`~lorenzcycletoolkit_b200.utils.preprocessing.packed_device_fields`
+        returns, or a ``[..., :nlon]`` view of them).  ``decode``: per field a dict ``scale``, ``offset``, ``fills``
+        (at most two int16 values), ``float32`` as in :meth:`run_host_raw`; the kernels decode every value they load
+        by the rule of the raw-record ingest, so the results have the bits of :meth:`run_torch` on the decoded fields.
+        Runs on torch's current stream; no synchronisation."""
+        import torch
+        if len(fields) != 5:
+            raise ValueError("need five fields: T, u, v, omega, Phi")
+        f0 = fields[0]
+        for t in fields:
+            if not t.is_cuda or t.dtype != torch.int16:
+                raise ValueError("packed fields must be int16 CUDA tensors")
+            if t.device.index != self.device:
+                raise ValueError("fields live on another device than the engine")
+            if t.dim() != 4 or tuple(t.shape[1:3]) != (self.nlev, self.nlat) or not self.nlon <= t.shape[3] <= t.stride(2):
+                raise ValueError(f"field shape {tuple(t.shape)} does not match the grid")
+            if (t.stride(3) != 1 or t.stride(2) % 8 or t.stride(1) != t.shape[2] * t.stride(2)
+                    or t.stride(0) != t.shape[1] * t.stride(1) or t.shape != f0.shape or t.stride() != f0.stride()):
+                raise ValueError("packed fields need contiguous rows with a pitch (row stride) that is a multiple of 8, "
+                                 "one shape and layout for all five")
+        n = len(steps)
+        dev = f0.device
+        if out is not None:
+            terms, levels, flags = out
+        else:
+            terms = torch.empty((n, NTERMS), dtype=torch.float64, device=dev)
+            levels = torch.empty((n, NLEVEL_TERMS, self.nlev), dtype=torch.float64, device=dev) if want_levels else None
+            flags = torch.zeros(n, dtype=torch.int32, device=dev)
+        if load_torch_extension():
+            d = _PackedDesc()
+            _set_decode(d, decode, strict=True)
+            st, _ = self._steps_arg(steps)
+            raw = np.frombuffer(bytes(d), dtype=np.uint8).copy()
+            rc = torch.ops.lec_b200.run_device_packed(int(self._h.value), list(fields), torch.from_numpy(raw),
+                                                      torch.from_numpy(st.view(np.uint8)), terms, levels, flags)
+            self._check(int(rc), "lec_run_device_packed")
+            return terms, levels, flags
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        self.run_device_packed([t.data_ptr() for t in fields], f0.shape[0], f0.stride(2), decode, steps, terms.data_ptr(),
+                               levels.data_ptr() if levels is not None else None, flags.data_ptr(), stream)
+        return terms, levels, flags
+
     def last_timing(self):
         """Device milliseconds of the last run: (row-moment kernels, finalize kernels, whole call)."""
         out = (C.c_float * 3)()
@@ -548,12 +631,13 @@ class LecEngine:
 
     def last_dispatch(self) -> dict:
         """Row kernel of the last kernel batch (``lec_last_dispatch``): ``kernel`` (one of :data:`ROW_KERNELS`),
-        ``vec``, ``group``, ``lonw``, ``comp``, ``math64``, ``tile_rows``, ``tiles_per_band``, ``nbands``."""
+        ``vec``, ``group``, ``lonw``, ``comp``, ``math64``, ``tile_rows``, ``tiles_per_band``, ``nbands``, ``packed``
+        (int16 fields: :meth:`run_torch_packed`)."""
         d = _Dispatch()
         self._check(self._lib.lec_last_dispatch(self._h, C.byref(d)), "lec_last_dispatch")
-        out = {n: int(getattr(d, n)) for n, _ in _Dispatch._fields_ if n != "reserved"}
+        out = {n: int(getattr(d, n)) for n, _ in _Dispatch._fields_}
         out["kernel"] = ROW_KERNELS[out["kernel"]]
-        out["comp"], out["math64"] = bool(out["comp"]), bool(out["math64"])
+        out["comp"], out["math64"], out["packed"] = bool(out["comp"]), bool(out["math64"]), bool(out["packed"])
         return out
 
     @property

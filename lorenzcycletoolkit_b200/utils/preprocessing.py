@@ -68,6 +68,42 @@ class RawStore:
         return out if level is None else out[:, 0]
 
 
+def packed_device_fields(store: RawStore, names, device="cuda"):
+    """Five int16 fields of a raw-backed dataset made resident on the GPU, still packed (2 bytes per value), for
+    ``LecEngine.run_torch_packed``: ``[time][level][lat][pitch]`` in the dataset's order (the store's record, level,
+    row and column maps applied), native byte order, rows padded with zeros to a pitch of a multiple of 8 elements.
+    A one-time load: one host gather and byte swap per time slot and field, then one copy to the device.  Returns
+    ``(tensors, decode)``; ``decode`` is the per-field rule of ``store.decode``.  Fields that are not int16, or whose
+    packing the decode rule cannot express (more than two fill values, a fill value that is not an int16 value, a
+    scale or offset that is not finite), raise ``ValueError``."""
+    import torch
+    nlon = len(store.lon)
+    pitch = (nlon + 7) // 8 * 8
+    decode = []
+    for v in names:
+        raw, dec = store.fields[v], store.decode[v]
+        if raw.dtype.kind != "i" or raw.dtype.itemsize != 2:
+            raise ValueError(f"{v} is stored as {raw.dtype}, not int16: packed device fields need int16 records")
+        fills = list(dec.get("fills", ()))
+        if len(fills) > 2 or not all(np.isfinite(float(x)) and float(x) == int(x) and -32768 <= int(x) <= 32767
+                                     for x in fills):
+            raise ValueError(f"{v}: fill values {fills} cannot be matched against int16 records")
+        for k in ("scale", "offset"):
+            if dec.get(k) is not None and not np.isfinite(float(dec[k])):
+                raise ValueError(f"{v}: {k} {dec[k]} is not finite")
+        decode.append(dict(dec))
+    out = []
+    for v in names:
+        raw = store.fields[v]
+        t = torch.zeros((len(store.rec), len(store.lev), len(store.lat), pitch), dtype=torch.int16, device=device)
+        host = np.zeros((len(store.lev), len(store.lat), pitch), dtype=np.int16)
+        for s, r in enumerate(store.rec):
+            host[:, :, :nlon] = raw[r][np.ix_(store.lev, store.lat, store.lon)]     # gather + byte swap to native
+            t[s].copy_(torch.from_numpy(host))
+        out.append(t)
+    return out, decode
+
+
 class _LazyVariables(dict):
     """``LecDataset.variables`` of a raw-backed dataset: decoded and re-ordered on first access."""
 

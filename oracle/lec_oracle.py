@@ -552,13 +552,18 @@ def conversion_terms(b, lv):
     return out
 
 
-def boundary_terms(b, legacy_0d=False):
+def boundary_terms(b, legacy_0d=False, pieces=None):
     """boundary_terms.py:122-418.
 
     ``legacy_0d``: evaluate ``c1, c2`` in float64 from the coordinate-dtype
     ``xlength, ylength`` (numpy 1.x value-based casting of Python-float x 0-d
     float32 array -- how the bundled goldens were produced, SURVEY.md C.1);
     default is the pinned numpy 2.0 NEP-50 behaviour (float32 on fp32 files).
+
+    ``pieces``: a dict that receives, per term, the three per-level arrays the engine returns through
+    ``lec_set_boundary_levels`` (lec_b200.h), stacked as ``[3][level]`` (``[time][3][level]`` for a fixed box):
+    part 0 the E-W flux after ``Yphi``, part 1 the N-S difference, part 2 the vertical-flux integrand, all taken
+    before ``_handle_nans``, so that ``term = c1 * trapz_p(part 0) + c2 * trapz_p(part 1) - (part 2[-1] - part 2[0])``.
     """
     s = b.sigma_AA
     p = b.p
@@ -586,63 +591,66 @@ def boundary_terms(b, legacy_0d=False):
         f, _ = handle_nans(f, p, -1)
         return f[..., -1] - f[..., 0]
 
+    def term(name, ew, ns, vert):     # ew, ns, vert: the per-level E-W, N-S and vertical pieces
+        if pieces is not None:
+            pieces[name] = np.stack([ew, ns, vert], axis=-2)
+        return vint(ew) * c1 + vint(ns) * c2 - BT(vert)
+
     out = {}
     # calc_baz :125-181
     t1 = ((2 * T_AE3 * T_ZE * b.u) + (T_AE3 ** 2 * b.u)) / (2 * sk2)
-    t1 = t1[..., E] - t1[..., W]
-    t1 = vint(Yphi(t1)) * c1
+    t1 = Yphi(t1[..., E] - t1[..., W])
     t2 = b.ZA(b.v_ZE * T_ZE) * 2 * T_AE
     t2 = (t2 + ((T_AE ** 2) * b.v_ZA)) * cos
     t2 = (t2[..., N] - t2[..., S]) / (2 * s)
-    t2 = vint(t2) * c2
     t3a = b.ZA(2 * b.omega_ZE * T_ZE) * T_AE
     t3b = b.omega_ZA * T_AE ** 2
     t3 = b.AAz(t3a + t3b) / (2 * s)
-    out["BAz"] = t1 + t2 - BT(t3)
+    out["BAz"] = term("BAz", t1, t2, t3)
     # calc_bae :183-230
     t1 = b.u * (T_ZE ** 2)
     t1 = t1[..., E] - t1[..., W]
-    t1 = vint(Yphi(t1 / (2 * sk))) * c1
+    t1 = Yphi(t1 / (2 * sk))
     t2 = b.ZA(b.v * T_ZE ** 2) * cos
     t2 = t2 / (2 * sk)
-    t2 = vint(t2[..., N] - t2[..., S]) * c2
+    t2 = t2[..., N] - t2[..., S]
     t3 = b.AA((b.omega * T_ZE ** 2) / (2 * sk2))
-    out["BAe"] = t1 + t2 - BT(t3)
+    out["BAe"] = term("BAe", t1, t2, t3)
     # calc_bkz :232-280
     Kstar = b.u ** 2 + b.v ** 2 - b.u_ZE ** 2 - b.v_ZE ** 2
     t1 = b.u * Kstar
     t1 = t1[..., E] - t1[..., W]
-    t1 = vint(Yphi(t1 / (2 * g))) * c1
+    t1 = Yphi(t1 / (2 * g))
     t2 = b.ZA(Kstar * b.v * cos[:, None])
     t2 = t2[..., N] - t2[..., S]
-    t2 = vint(t2 / (2 * g)) * c2
+    t2 = t2 / (2 * g)
     t3 = b.AA(Kstar * b.omega) / (2 * g)
-    out["BKz"] = t1 + t2 - BT(t3)
+    out["BKz"] = term("BKz", t1, t2, t3)
     # calc_bke :282-326
     Kp = b.u_ZE ** 2 + b.v_ZE ** 2
     t1 = b.u * Kp
     t1 = t1[..., E] - t1[..., W]
-    t1 = vint(Yphi(t1 / (2 * g))) * c1
+    t1 = Yphi(t1 / (2 * g))
     t2 = b.ZA(Kp * b.v * cos[:, None])
     t2 = t2[..., N] - t2[..., S]
-    t2 = vint(t2 / (2 * g)) * c2
+    t2 = t2 / (2 * g)
     t3 = b.AA(Kp * b.omega) / (2 * g)
-    out["BKe"] = t1 + t2 - BT(t3)
+    out["BKe"] = term("BKe", t1, t2, t3)
     # calc_boz :328-370 (no E-W difference, sic)
     t1 = (b.v_ZA * b.geopt_AE) / g
-    t1 = vint(Yphi(t1)) * c1
+    t1 = Yphi(t1)
     t2 = (b.v_ZA * b.geopt_AE) * cos / g
-    t2 = vint(t2[..., N] - t2[..., S]) * c2
+    t2 = t2[..., N] - t2[..., S]
     t3 = b.AAz(b.omega_AE * b.geopt_AE) / g
-    out["BΦZ"] = t1 + t2 - BT(t3)
+    out["BΦZ"] = term("BΦZ", t1, t2, t3)
     # calc_boe :372-418 (v_ZE*geopt_AE and BPhiZ's N-S term, sic)
     t1 = (b.v_ZE * b.geopt_AE[..., None]) / g
     t1 = t1[..., E] - t1[..., W]
-    t1 = vint(Yphi(t1)) * c1
+    t1 = Yphi(t1)
     t2 = (b.v_ZA * b.geopt_AE) * cos / g
-    t2 = vint(t2[..., N] - t2[..., S]) * c2
+    t2 = t2[..., N] - t2[..., S]
     t3 = b.AA(b.omega_ZE * b.geopt_ZE) / g
-    out["BΦE"] = t1 + t2 - BT(t3)
+    out["BΦE"] = term("BΦE", t1, t2, t3)
     return out
 
 

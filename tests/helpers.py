@@ -189,3 +189,95 @@ def write_netcdf3_copy(src, dst, edit=None, extra=None):
             for k, v in attrs.items():
                 setattr(var, k, v)
             var[:] = arr
+
+
+# --------------------------------------------------------------------------------------- #
+# one step of the oracle on any box, and the per-level boundary pieces
+BOUNDARY_TERMS = ["BAz", "BAe", "BKz", "BKe", "BΦZ", "BΦE"]
+
+
+def boundary_pieces(pieces):
+    """The dict ``O.boundary_terms(..., pieces=)`` fills, as the engine's ``[..][6][3][nlev]`` array."""
+    return np.stack([np.asarray(pieces[n], dtype=np.float64) for n in BOUNDARY_TERMS], axis=-3)
+
+
+def oracle_step(P, box, it, dTdt):
+    """One step evaluated as ``O.lec_moving`` does (a ``BoxState`` of time ``it`` on the box of grid indices
+    ``box = (i0, i1, j0, j1)``, ``dTdt`` the global ``np.gradient`` dT/dt), for a ``P`` already in the arithmetic
+    of the comparison (``O.to_mode(P, "fp64")``).  Returns (16 terms by name, per-level families by name,
+    boundary pieces ``[6][3][nlev]``)."""
+    i0, i1, j0, j1 = box
+    b = O.BoxState(P, P.lon[i0], P.lon[i1], P.lat[j0], P.lat[j1], fixed=False, dTdt=dTdt[it], tsel=it)
+    assert b.idx == tuple(box), (b.idx, box)
+    lv, terms, pieces = {}, {}, {}
+    terms.update(O.energy_contents(b, lv))
+    terms.update(O.conversion_terms(b, lv))
+    terms.update(O.boundary_terms(b, pieces=pieces))
+    terms.update(O.generation_terms(b, lv))
+    return ({k: float(v) for k, v in terms.items()}, {k: np.asarray(v, dtype=np.float64) for k, v in lv.items()},
+            boundary_pieces(pieces))
+
+
+# --------------------------------------------------------------------------------------- #
+# int16-packed fields (lec_run_device_packed) and device-side boundary pieces
+FILL = -32767
+
+
+def encode(fields, spec):
+    """int16 records of float fields + the decode dicts of LecEngine.run_torch_packed."""
+    raws, decode = [], []
+    for a, sp in zip(fields, spec):
+        a = np.asarray(a, dtype=np.float64)
+        lo, hi = float(a.min()), float(a.max())
+        if sp["offset"]:
+            scale, offset = (hi - lo) / 65000.0, 0.5 * (hi + lo)
+        else:
+            scale, offset = max(abs(lo), abs(hi)) / 32000.0, None
+        raw = np.round((a - (offset or 0.0)) / scale).astype(np.int16)
+        fills = [FILL, -32768][:sp["nfill"]]
+        raws.append(raw)
+        decode.append(dict(scale=np.float64(scale), offset=None if offset is None else np.float64(offset),
+                           fills=fills, float32=sp["float32"]))
+    return raws, decode
+
+
+def decode(raw, dec, dtype):
+    """The decode rule in numpy: multiply, then add, as separate float64 operations."""
+    x = raw.astype(np.float64)
+    if dec["scale"] is not None:
+        x = x * np.float64(dec["scale"])
+    if dec["offset"] is not None:
+        x = x + np.float64(dec["offset"])
+    if dec["float32"]:
+        x = x.astype(np.float32).astype(np.float64)
+    for fv in dec["fills"]:
+        x[raw == fv] = np.nan
+    return x.astype(dtype)
+
+
+def padded(raw, pitch):
+    """Device int16 [slot][level][lat][pitch]; the pad columns hold fill values."""
+    import torch
+    buf = np.full(raw.shape[:3] + (pitch,), FILL, dtype=np.int16)
+    buf[..., :raw.shape[3]] = raw
+    return torch.from_numpy(buf).cuda()
+
+
+def with_boundary(eng, n, fn):
+    """Run ``fn()`` (a LecEngine.run_torch* call) with the per-level boundary pieces armed on a device buffer;
+    returns (fn's results as numpy arrays..., pieces ``[n][18][nlev]``)."""
+    import ctypes as C
+    import torch
+    bnd = torch.empty((n, E.NBOUNDARY_PIECES, eng.nlev), dtype=torch.float64, device="cuda")
+    eng._check(eng._lib.lec_set_boundary_levels(eng._h, C.c_void_p(bnd.data_ptr())), "lec_set_boundary_levels")
+    try:
+        out = fn()
+    finally:
+        eng._lib.lec_set_boundary_levels(eng._h, None)
+    torch.cuda.synchronize()
+    return tuple(x.cpu().numpy() for x in out) + (bnd.cpu().numpy(),)
+
+
+def same_bits(a, b):
+    for x, y in zip(a, b):
+        assert x.shape == y.shape and np.array_equal(x.view(np.uint8), y.view(np.uint8))

@@ -150,3 +150,25 @@ def test_stationary_track_reproduces_the_pinned_fixed_run(catarina):
     for name in ("Az", "Ae", "Kz", "Ke", "Ge", "Gz", "Ck", "Ca", "Ce", "Cz"):
         f, m = np.asarray(flv[name]), np.asarray(mlv[name])
         assert f.shape == m.shape and np.max(np.abs(f - m)) <= 1e-12 * np.max(np.abs(f)), name
+
+
+def test_boundary_pieces_reassemble_the_boundary_terms(catarina):
+    """The per-level pieces ``boundary_terms(pieces=)`` exposes (the engine's ``lec_set_boundary_levels`` output)
+    rebuild the six boundary terms: c1 * trapz_p(E-W) + c2 * trapz_p(N-S) - (vertical at the last level - at the
+    first).  Fixed box: one [time][3][level] array per term."""
+    P, box = catarina
+    b = O.BoxState(O.to_mode(P, "fp64"), *box, fixed=True)
+    pieces = {}
+    out = O.boundary_terms(b, pieces=pieces)
+    assert set(pieces) == set(H.BOUNDARY_TERMS)
+    nt, nlev = len(P.time), len(P.level)
+    c1 = -1 / (O.Re * b.xlength * b.ylength)
+    c2 = -1 / (O.Re * b.ylength)
+    arr = H.boundary_pieces(pieces)
+    assert arr.shape == (nt, 6, 3, nlev) and np.isfinite(arr).all()
+    np.testing.assert_array_equal(arr[:, 5, 1], arr[:, 4, 1])              # BΦE takes BΦZ's N-S piece (sic)
+    for n, name in enumerate(H.BOUNDARY_TERMS):
+        ew, ns, vert = arr[:, n, 0], arr[:, n, 1], arr[:, n, 2]
+        want = c1 * O.trapz(ew, b.p, -1) + c2 * O.trapz(ns, b.p, -1) - (vert[:, -1] - vert[:, 0])
+        assert H.series_err(want, out[name]) <= 1e-12, name
+        assert np.abs(ew).max() > 0 and np.abs(ns).max() > 0 and np.abs(vert).max() > 0, name

@@ -23,7 +23,7 @@ torch = pytest.importorskip("torch")
 ARITH = {"f32": (np.float32, E.LEC_MATH_AUTO, 4), "m64": (np.float32, E.LEC_MATH_F64, 4),
          "f64": (np.float64, E.LEC_MATH_AUTO, 2)}
 LONW = {"exact": 0, "f32": 1, "irregular": 2}
-FILL = -32767
+FILL = H.FILL
 T0 = np.datetime64("2020-01-01T00")
 NT, NLEV = 4, 4
 WIDE = (816, 131)
@@ -43,38 +43,6 @@ def _decode_spec(arith):
         spec[3] = dict(offset=False, float32=True, nfill=1)
         spec[4] = dict(offset=False, float32=True, nfill=2)
     return spec
-
-
-def _encode(fields, spec):
-    """int16 records of float fields + the decode dicts of LecEngine.run_torch_packed."""
-    raws, decode = [], []
-    for a, sp in zip(fields, spec):
-        a = np.asarray(a, dtype=np.float64)
-        lo, hi = float(a.min()), float(a.max())
-        if sp["offset"]:
-            scale, offset = (hi - lo) / 65000.0, 0.5 * (hi + lo)
-        else:
-            scale, offset = max(abs(lo), abs(hi)) / 32000.0, None
-        raw = np.round((a - (offset or 0.0)) / scale).astype(np.int16)
-        fills = [FILL, -32768][:sp["nfill"]]
-        raws.append(raw)
-        decode.append(dict(scale=np.float64(scale), offset=None if offset is None else np.float64(offset),
-                           fills=fills, float32=sp["float32"]))
-    return raws, decode
-
-
-def _decode(raw, dec, dtype):
-    """The decode rule in numpy: multiply, then add, as separate float64 operations."""
-    x = raw.astype(np.float64)
-    if dec["scale"] is not None:
-        x = x * np.float64(dec["scale"])
-    if dec["offset"] is not None:
-        x = x + np.float64(dec["offset"])
-    if dec["float32"]:
-        x = x.astype(np.float32).astype(np.float64)
-    for fv in dec["fills"]:
-        x[raw == fv] = np.nan
-    return x.astype(dtype)
 
 
 _DATA = {}
@@ -120,35 +88,11 @@ def _plant_fills(raws, box, vecw, inside=None):
     return out
 
 
-def _padded(raw, pitch):
-    """Device int16 [slot][level][lat][pitch]; the pad columns hold fill values."""
-    buf = np.full(raw.shape[:3] + (pitch,), FILL, dtype=np.int16)
-    buf[..., :raw.shape[3]] = raw
-    return torch.from_numpy(buf).cuda()
-
-
 def _steps(P, boxes):
     steps = E.time_stencil(H.tsec_of(P), E.make_steps(len(P.time)))
     for it, b in enumerate(boxes):
         steps["i0"][it], steps["i1"][it], steps["j0"][it], steps["j1"][it] = b
     return steps
-
-
-def _with_boundary(eng, n, fn):
-    """Run ``fn()`` with the per-level boundary pieces armed on a device buffer; returns (fn's results, pieces)."""
-    bnd = torch.empty((n, E.NBOUNDARY_PIECES, eng.nlev), dtype=torch.float64, device="cuda")
-    eng._check(eng._lib.lec_set_boundary_levels(eng._h, C.c_void_p(bnd.data_ptr())), "lec_set_boundary_levels")
-    try:
-        out = fn()
-    finally:
-        eng._lib.lec_set_boundary_levels(eng._h, None)
-    torch.cuda.synchronize()
-    return tuple(x.cpu().numpy() for x in out) + (bnd.cpu().numpy(),)
-
-
-def _same_bits(a, b):
-    for x, y in zip(a, b):
-        assert x.shape == y.shape and np.array_equal(x.view(np.uint8), y.view(np.uint8))
 
 
 def _pair(P, raws, decode, boxes, arith, band_rows=0, pitch_extra=0):
@@ -157,12 +101,12 @@ def _pair(P, raws, decode, boxes, arith, band_rows=0, pitch_extra=0):
     steps = _steps(P, boxes)
     nlon = raws[0].shape[3]
     pitch = (nlon + 7) // 8 * 8 + pitch_extra
-    dec_t = [torch.from_numpy(np.ascontiguousarray(_decode(r, d, dtype))).cuda() for r, d in zip(raws, decode)]
-    pk_t = [_padded(r, pitch) for r in raws]
+    dec_t = [torch.from_numpy(np.ascontiguousarray(H.decode(r, d, dtype))).cuda() for r, d in zip(raws, decode)]
+    pk_t = [H.padded(r, pitch) for r in raws]
     with H.make_engine(P, dtype, [1.0] * 5, math=math, band_rows=band_rows) as eng:
-        a = _with_boundary(eng, len(steps), lambda: eng.run_torch_packed(pk_t, decode, steps))
+        a = H.with_boundary(eng, len(steps), lambda: eng.run_torch_packed(pk_t, decode, steps))
         da = eng.last_dispatch()
-        b = _with_boundary(eng, len(steps), lambda: eng.run_torch(dec_t, steps))
+        b = H.with_boundary(eng, len(steps), lambda: eng.run_torch(dec_t, steps))
         db = eng.last_dispatch()
     return (a, da), (b, db)
 
@@ -174,7 +118,7 @@ def _packed_tile_rows(arith):
 def _cell(key, boxes, arith, inside=None, **kw):
     P, fields = _dataset(*key)
     vecw = ARITH[arith][2]
-    raws, decode = _encode(fields, _decode_spec(arith))
+    raws, decode = H.encode(fields, _decode_spec(arith))
     if len(set(boxes)) == 1:
         raws = _plant_fills(raws, boxes[0], vecw, inside)
     (a, da), (b, db) = _pair(P, raws, decode, boxes, arith, **kw)
@@ -188,7 +132,7 @@ def _cell(key, boxes, arith, inside=None, **kw):
         assert da["tile_rows"] == db["tile_rows"], (da, db)
     if inside is None:
         assert not a[2].any() and np.isfinite(a[0]).all() and np.isfinite(a[1]).all(), a[2]
-        _same_bits(a, b)
+        H.same_bits(a, b)
     else:
         for x, y in zip(a, b):
             assert np.array_equal(x, y, equal_nan=True)
@@ -276,20 +220,20 @@ def test_direct_and_tiled_sub_warp_switches_do_not_apply(monkeypatch):
     monkeypatch.setenv("LEC_ROW_KERNEL", "direct")
     monkeypatch.setenv("LEC_NARROW_TILE", "1")
     P, fields = _dataset("f32", *WIDE)
-    raws, decode = _encode(fields, _decode_spec("f32"))
+    raws, decode = H.encode(fields, _decode_spec("f32"))
     for chunks, kernel in ((60, "subwarp"), (201, "tiled")):
         box = _box(chunks, 4, 5, 1, 40)
         steps = _steps(P, [box] * NT)
         with H.make_engine(P, np.float32, [1.0] * 5) as eng:
-            eng.run_torch_packed([_padded(r, 816) for r in raws], decode, steps)
+            eng.run_torch_packed([H.padded(r, 816) for r in raws], decode, steps)
             d = eng.last_dispatch()
         assert d["kernel"] == kernel and d["packed"], d
 
 
 def test_the_torch_operator_and_the_ctypes_route_agree(monkeypatch):
     P, fields = _dataset("f32", *WIDE)
-    raws, decode = _encode(fields, _decode_spec("f32"))
-    tens = [_padded(r, 824) for r in raws]
+    raws, decode = H.encode(fields, _decode_spec("f32"))
+    tens = [H.padded(r, 824) for r in raws]
     outs = []
     for ext in (True, False):
         if E.load_torch_extension() != ext:
@@ -299,27 +243,27 @@ def test_the_torch_operator_and_the_ctypes_route_agree(monkeypatch):
             for box in (_box(60, 4, 5, 1, 40), _box(201, 4, 5, 1, 40)):
                 outs.append(tuple(x.cpu().numpy() for x in eng.run_torch_packed(tens, decode, _steps(P, [box] * NT))))
     assert len(outs) == 4
-    _same_bits(outs[0], outs[2])
-    _same_bits(outs[1], outs[3])
+    H.same_bits(outs[0], outs[2])
+    H.same_bits(outs[1], outs[3])
 
 
 def test_a_view_of_the_first_nlon_columns_is_accepted():
     P, fields = _dataset("f32", 810, 40)
-    raws, decode = _encode(fields, _decode_spec("f32"))
+    raws, decode = H.encode(fields, _decode_spec("f32"))
     box = _box(202, 4, 1, 1, 38)
     steps = _steps(P, [box] * NT)
-    full = [_padded(r, 816) for r in raws]
+    full = [H.padded(r, 816) for r in raws]
     with H.make_engine(P, np.float32, [1.0] * 5) as eng:
         a = tuple(x.cpu().numpy() for x in eng.run_torch_packed(full, decode, steps))
         b = tuple(x.cpu().numpy() for x in eng.run_torch_packed([t[..., :810] for t in full], decode, steps))
-    _same_bits(a, b)
+    H.same_bits(a, b)
 
 
 def test_invalid_arguments_are_rejected():
     P, fields = _dataset("f32", 810, 40)
-    raws, decode = _encode(fields, _decode_spec("f32"))
+    raws, decode = H.encode(fields, _decode_spec("f32"))
     steps = _steps(P, [_box(202, 4, 1, 1, 38)] * NT)
-    good = [_padded(r, 816) for r in raws]
+    good = [H.padded(r, 816) for r in raws]
     terms = torch.empty((NT, E.NTERMS), dtype=torch.float64, device="cuda")
     with H.make_engine(P, np.float32, [1.0] * 5) as eng:
         ptrs = [t.data_ptr() for t in good]
@@ -373,7 +317,7 @@ def test_era5_records_have_the_bits_of_the_raw_record_path(tmp_path):
             a = tuple(x.cpu().numpy() for x in eng.run_torch_packed(tens, decode, steps))
             b = eng.run_host_raw([store.fields[v] for v in names], store.lon, store.lat, store.lev, store.rec, steps,
                                  decode=[store.decode[v] for v in names])
-        _same_bits(a, b)
+        H.same_bits(a, b)
 
 
 def test_non_int16_records_are_refused(tmp_path):
@@ -388,12 +332,12 @@ def test_non_int16_records_are_refused(tmp_path):
 def _packed_prepared(P, names, fp32):
     """int16 encodings of the prepared fields ``names`` and P with those fields replaced by their decoded values."""
     spec = [dict(offset=not fp32, float32=fp32, nfill=1)] * len(names)
-    raws, decode = _encode([P.fields[n] for n in names], spec)
+    raws, decode = H.encode([P.fields[n] for n in names], spec)
     Q = O.Prepared()
     Q.__dict__.update(P.__dict__)
     Q.fields = dict(P.fields)
     for n, r, d in zip(names, raws, decode):
-        Q.fields[n] = _decode(r, d, np.float64)
+        Q.fields[n] = H.decode(r, d, np.float64)
     return raws, decode, Q
 
 
@@ -408,7 +352,7 @@ def test_catarina_fixed_box_matches_the_oracle(dtype, tol):
     _, scale = H.engine_inputs(Q, dtype)
     pitch = (raws[0].shape[3] + 7) // 8 * 8
     with H.make_engine(Q, dtype, scale) as eng:
-        terms, _, flags = eng.run_torch_packed([_padded(r, pitch) for r in raws], decode, H.fixed_steps(Q, *box))
+        terms, _, flags = eng.run_torch_packed([H.padded(r, pitch) for r in raws], decode, H.fixed_steps(Q, *box))
         assert eng.last_dispatch()["packed"]
     errs = H.compare_terms(terms.cpu().numpy(), df, extra=extra)
     assert max(errs.values()) <= tol, errs
@@ -425,6 +369,6 @@ def test_testdata_track_matches_the_oracle(dtype, tol):
     pitch = (raws[0].shape[3] + 7) // 8 * 8
     steps = H.moving_steps(Q, track)
     with H.make_engine(Q, dtype, scale, max_box_rows=int((steps["j1"] - steps["j0"]).max()) + 1) as eng:
-        terms, _, flags = eng.run_torch_packed([_padded(r, pitch) for r in raws], decode, steps)
+        terms, _, flags = eng.run_torch_packed([H.padded(r, pitch) for r in raws], decode, steps)
     errs = H.compare_terms(terms.cpu().numpy(), df)
     assert len(errs) >= 14 and max(errs.values()) <= tol, errs

@@ -202,7 +202,7 @@ int lec_run_host_raw(lec_handle *h, const lec_raw_desc *raw_desc, const void *co
  * read into a result.  Everything else (steps, outputs, stream, batches of max_steps, lec_set_boundary_levels,
  * timing, nsteps = 0) as lec_run_device.  LEC_ERR_INVALID for a pitch below nlon or not a multiple of 8, a
  * misaligned field, nfill outside 0..2 or a fill value that is not an int16 value.  The row kernel is the TMA-tiled
- * one for wide boxes and the sub-warp one for narrow boxes whatever LEC_ROW_KERNEL / LEC_NARROW_TILE say;
+ * one for wide boxes and the sub-warp one for narrow boxes whatever LEC_ROW_KERNEL says;
  * lec_last_dispatch reports it with packed = 1. */
 typedef struct lec_packed_desc {
   int32_t pitch;                 /* row length of the packed fields in elements: >= nlon, multiple of 8 (16 B) */
@@ -257,15 +257,14 @@ int64_t lec_launch_count(lec_handle *h);
 #define LEC_ROWS_DIRECT          0   /* direct loads, one warp per row                                 */
 #define LEC_ROWS_SUBWARP         1   /* direct loads, a group of `group` lanes per row (narrow boxes)  */
 #define LEC_ROWS_TILED           2   /* TMA ring of tile_rows-row tiles, one warp per row (wide boxes)  */
-#define LEC_ROWS_TILED_SUBWARP   3   /* TMA ring feeding 8-lane row groups (track boxes, opt-in)        */
 typedef struct lec_dispatch {
   int32_t kernel;           /* LEC_ROWS_* */
   int32_t vec;              /* elements per lane load: 4 (fp32) / 2 (fp64) on 16-byte aligned rows, 1 scalar */
-  int32_t group;            /* lanes per row: 4, 8 or 16 for the sub-warp kernels, else 32 */
+  int32_t group;            /* lanes per row: 4, 8 or 16 for the sub-warp kernel, else 32 */
   int32_t lonw;             /* longitude tables: 0 uniform, 1 per-column weights, 2 weights and stencil */
   int32_t comp;             /* 1: compensated fp32 linear sums */
   int32_t math64;           /* 1: fp64 pointwise arithmetic (fp64 fields or LEC_MATH_F64) */
-  int32_t tile_rows;        /* box rows per tile (tiled kernels), per CTA otherwise */
+  int32_t tile_rows;        /* box rows per tile (tiled kernel), per CTA otherwise */
   int32_t tiles_per_band;   /* tiles per latitude band of the block order */
   int32_t nbands;           /* latitude bands (1: step-major order) */
   int32_t packed;           /* 1: int16 fields decoded by the row kernel (lec_run_device_packed) */

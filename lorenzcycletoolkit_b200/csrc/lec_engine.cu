@@ -19,20 +19,9 @@
 
 using namespace lec;
 
-#ifndef LEC_TILE_DEFAULT
-#define LEC_TILE_DEFAULT 1          // 1: wide boxes take the TMA-tiled row kernel unless LEC_ROW_KERNEL=direct
-#endif
 #ifndef LEC_TILE_ROWS_DEFAULT
 #define LEC_TILE_ROWS_DEFAULT 15
 #endif
-
-#ifndef LEC_NTILE_WARPS      // measured on the C5 track: 13 x 1 -> 1.98 ms, 6 x 2 -> 2.24 ms, 4 x 3 -> 2.19 ms, 3 x 4 -> 2.21 ms
-#define LEC_NTILE_WARPS 13
-#define LEC_NTILE_CTAS 1
-#endif
-constexpr int kNarrowTileWarps = LEC_NTILE_WARPS;      // consumer warps per CTA of the TMA-tiled kernel for track boxes
-constexpr int kNarrowTileCtas = LEC_NTILE_CTAS;        // CTAs per SM (independent rings at different phases)
-constexpr int kNarrowTileRows = kNarrowTileWarps * 4;  // 8-lane groups: 4 rows per warp
 
 struct lec_handle {
   lec_grid_desc desc{};
@@ -43,14 +32,13 @@ struct lec_handle {
   float* d_tables32 = nullptr;
   int prefetch_mode = 1 | 16;                   // bit 0: own-row L2 bulk prefetch of the direct wide kernel (+9 % measured), bit 4: per-lane
                                                 // L2 prefetch of a track-box row's later sweep iterations (+8 %); LEC_PREFETCH=0 disables both
-  int use_tile = LEC_TILE_DEFAULT;              // LEC_ROW_KERNEL=tile|direct: TMA-tiled row kernel for wide boxes
+  int use_tile = 1;                             // LEC_ROW_KERNEL=tile|direct: TMA-tiled row kernel for wide boxes
   int tile_rows = LEC_TILE_ROWS_DEFAULT;        // rows per tile (experiment builds: LEC_TILE_ROWS=8|11|12|15)
   int num_sms = 148;
   long long h2d_bytes = 0, d2h_bytes = 0;      // PCIe traffic of the last lec_run_host
   int comp_mode = -1;                           // LEC_COMP=0|1: force the compensated fp32 linear sums off / on (-1: by box shape)
   int use_narrow = 1;                           // LEC_NARROW=0: never use the sub-warp kernel for narrow boxes
   int tma_hint = -1;                            // LEC_TMA_HINT=0|1: evict-first hint on the once-read fields (-1: fp64 fields only)
-  int use_ntile = 0;                            // LEC_NARROW_TILE=1: track boxes (8-lane row groups) through the TMA ring instead of direct loads (same bits; measured 2 % slower)
   int force_narrow_g = 0;                       // LEC_NARROW_G=4|8|16: force the group width (measurements)
   double* d_rec = nullptr;
   double* d_fin = nullptr;             // finalize scratch [max_steps][nlev][kLevStride]
@@ -94,11 +82,7 @@ struct lec_handle {
 
 namespace {
 
-#if LEC_TILE_DEFAULT
 const char* kVersion = "lec_b200 0.2 (sm_100a; rows=tile)";
-#else
-const char* kVersion = "lec_b200 0.2 (sm_100a; rows=direct)";
-#endif
 
 #define CK(call)                                                                   \
   do {                                                                             \
@@ -129,35 +113,11 @@ int lon_mode(const lec_handle* h) {
   return h->g.stencil_uniform >= need ? 1 : 2;
 }
 
-// COMP (compensated linear sums) only exists for fp32 arithmetic.
 template <typename FT, typename CT, int VEC, bool COMP>
-void launch_rows_c(const RowParams& rp, int lonw, long long grid, cudaStream_t st) {
+void launch_direct_c(const RowParams& rp, int lonw, long long grid, cudaStream_t st) {
   if (lonw == 0) lec_row_moments_kernel<FT, CT, VEC, 0, COMP><<<(unsigned)grid, kRowThreads, 0, st>>>(rp);
   else if (lonw == 1) lec_row_moments_kernel<FT, CT, VEC, 1, COMP><<<(unsigned)grid, kRowThreads, 0, st>>>(rp);
   else lec_row_moments_kernel<FT, CT, VEC, 2, COMP><<<(unsigned)grid, kRowThreads, 0, st>>>(rp);
-}
-template <typename FT, typename CT, int VEC>
-void launch_rows_t(const RowParams& rp, int lonw, bool comp, long long grid, cudaStream_t st) {
-  if constexpr (sizeof(CT) == 4) {
-    if (comp) { launch_rows_c<FT, CT, VEC, true>(rp, lonw, grid, st); return; }
-  }
-  launch_rows_c<FT, CT, VEC, false>(rp, lonw, grid, st);
-}
-
-void launch_rows(const lec_handle* h, const RowParams& rp, bool vec, bool comp, long long grid, cudaStream_t st) {
-  const bool f64 = h->desc.dtype == LEC_F64;
-  const bool m64 = f64 || h->desc.math == LEC_MATH_F64;
-  const int lonw = lon_mode(h);
-  if (f64) {
-    if (vec) launch_rows_t<double, double, 2>(rp, lonw, comp, grid, st);
-    else launch_rows_t<double, double, 1>(rp, lonw, comp, grid, st);
-  } else if (m64) {
-    if (vec) launch_rows_t<float, double, 4>(rp, lonw, comp, grid, st);
-    else launch_rows_t<float, double, 1>(rp, lonw, comp, grid, st);
-  } else {
-    if (vec) launch_rows_t<float, float, 4>(rp, lonw, comp, grid, st);
-    else launch_rows_t<float, float, 1>(rp, lonw, comp, grid, st);
-  }
 }
 
 template <typename FT, typename CT, int VEC, bool COMP, typename ST>
@@ -166,13 +126,6 @@ void launch_narrow_c(const RowParams& rp, bool table, int G, long long grid, cud
   if (table) { if (G == 16) LEC_NARROW(2, 16); else if (G == 8) LEC_NARROW(2, 8); else LEC_NARROW(2, 4); }
   else { if (G == 16) LEC_NARROW(0, 16); else if (G == 8) LEC_NARROW(0, 8); else LEC_NARROW(0, 4); }
 #undef LEC_NARROW
-}
-template <typename FT, typename CT, int VEC, typename ST = FT>
-void launch_narrow_t(const RowParams& rp, bool table, bool comp, int G, long long grid, cudaStream_t st) {
-  if constexpr (sizeof(CT) == 4) {
-    if (comp) { launch_narrow_c<FT, CT, VEC, true, ST>(rp, table, G, grid, st); return; }
-  }
-  launch_narrow_c<FT, CT, VEC, false, ST>(rp, table, G, grid, st);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -193,8 +146,7 @@ EncodeTiledFn encode_tiled_fn() {
 
 // 4-D tensor map over a [slot][level][lat][lon] field of `esize`-byte elements (fp64 / fp32 / int16) with a
 // (bx x by) box in (lon, lat).
-bool make_map(CUtensorMap* m, const void* base, int esize, int nlon, int nlat, int nlev, int nslots, int bx, int by,
-              int promo = 3) {
+bool make_map(CUtensorMap* m, const void* base, int esize, int nlon, int nlat, int nlev, int nslots, int bx, int by) {
   EncodeTiledFn enc = encode_tiled_fn();
   if (!enc) return false;
   const cuuint64_t e = (cuuint64_t)esize;
@@ -207,77 +159,106 @@ bool make_map(CUtensorMap* m, const void* base, int esize, int nlon, int nlat, i
                                  : esize == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT16;
   return enc(m, dt, 4, const_cast<void*>(base),
              dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-             promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : promo == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-             : promo == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+             CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <typename FT, typename CT, int R, int S, bool COMP, int GL = 32, int MINB = 1, typename ST = FT>
-cudaError_t launch_tile_c(const TmaMaps& maps, const RowParams& rp, int lonw, int grid, cudaStream_t st) {
-  using G = TileGeom<FT, R, S, GL, ST>;
-  cudaError_t e = cudaSuccess;
-#define LEC_TILE_LAUNCH(LW, TB, SMEM)                                                                             \
-  do {                                                                                                            \
-    e = cudaFuncSetAttribute(lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, GL, MINB, ST>,          \
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);                                  \
-    if (e == cudaSuccess) lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, GL, MINB, ST><<<grid, G::threads, SMEM, st>>>(maps, rp); \
-  } while (0)
-  if constexpr (GL != 32) {      // track boxes: no table / full tables, as the sub-warp kernel
-    if (lonw == 0) LEC_TILE_LAUNCH(0, false, G::smem_bytes);
-    else LEC_TILE_LAUNCH(2, false, G::smem_bytes);
-  } else {
-    // fp32 per-column weights (LONW == 1): table in shared memory when it fits behind the ring
-    const int tab_bytes = (sizeof(ST) == sizeof(FT) ? (rp.g.nlon + 3) & ~3 : rp.pk.ntab) * 4;
-    if (lonw == 0) LEC_TILE_LAUNCH(0, false, G::smem_bytes);
-    else if (lonw == 1) {
-      if (sizeof(CT) == 4 && sizeof(FT) == 4 && G::smem_bytes + tab_bytes <= 227 * 1024) LEC_TILE_LAUNCH(1, true, G::smem_bytes + tab_bytes);
-      else LEC_TILE_LAUNCH(1, false, G::smem_bytes);
-    } else LEC_TILE_LAUNCH(2, false, G::smem_bytes);
-  }
-#undef LEC_TILE_LAUNCH
-  return e != cudaSuccess ? e : cudaGetLastError();
-}
-
-// Tile shapes: R consumer warps + 1 producer warp; the per-SMSP register file allows 168 registers per thread
-// up to 12 warps per CTA and 128 up to 16.  Stages sized to fill the 227 KB of shared memory.
+// Ring shapes of the tiled kernel, rows (= consumer warps) x stages: the one place the tile height is chosen
+// (run_batch records it in lec_dispatch::tile_rows, launch_rows instantiates it).  R consumer warps + 1 producer warp;
+// the per-SMSP register file allows 168 registers per thread up to 12 warps per CTA and 128 up to 16.  Stages sized
+// to fill the 227 KB of shared memory.
 //   fp32 arithmetic                 15 rows x 3 stages  (128 registers, no spills)
 //   fp32 with compensated sums      11 rows x 4 stages  (six more live registers)
 //   fp64 fields                     11 rows x 4 stages  (158-168 registers)
 //   fp32 fields, fp64 arithmetic     7 rows x 6 stages  (four values per lane in fp64: > 168 registers)
-template <typename FT, typename CT>
-cudaError_t launch_tile_t(const TmaMaps& maps, const RowParams& rp, int lonw, bool comp, int rows, int grid,
-                          cudaStream_t st) {
-  if constexpr (sizeof(CT) == 4) {
-    if (comp) return launch_tile_c<FT, CT, 11, 4, true>(maps, rp, lonw, grid, st);
-#ifdef LEC_TILE_ALL_SHAPES
-    if (rows == 8) return launch_tile_c<FT, CT, 8, 5, false>(maps, rp, lonw, grid, st);
-    if (rows == 11) return launch_tile_c<FT, CT, 11, 4, false>(maps, rp, lonw, grid, st);
-    if (rows == 12) return launch_tile_c<FT, CT, 12, 4, false>(maps, rp, lonw, grid, st);
-#endif
-    return launch_tile_c<FT, CT, 15, 3, false>(maps, rp, lonw, grid, st);
-  } else if constexpr (sizeof(FT) == 4) {
-    return launch_tile_c<FT, CT, 7, 6, false>(maps, rp, lonw, grid, st);      // fp32 fields, fp64 arithmetic (LEC_MATH_F64)
-  } else {
-    return launch_tile_c<FT, CT, 11, 4, false>(maps, rp, lonw, grid, st);
-  }
-}
-
-// Tile shapes over int16 fields: a stage holds about half (fp32) or a quarter (fp64) of the bytes, so the ring gets
-// more stages (at most 8: the barriers share the 128 bytes behind it).  fp32 arithmetic takes 11 rows, not 15: 15
-// consumer warps leave 128 registers and the decode's fp64 temporaries spill there (16-56 B).
+// Over int16 fields a stage holds about half (fp32) or a quarter (fp64) of the bytes, so the ring gets more stages (at
+// most 8: the barriers share the 128 bytes behind it).  fp32 arithmetic takes 11 rows, not 15: 15 consumer warps
+// leave 128 registers and the decode's fp64 temporaries spill there (16-56 B).
 //   fp32 arithmetic, plain or compensated  11 rows x 7 stages  (196 KB)
 //   fp64 decode                            11 rows x 8 stages  (122 KB)
 //   fp32 decode, fp64 arithmetic            7 rows x 8 stages  (142 KB)
-template <typename FT, typename CT>
-cudaError_t launch_tile_packed(const TmaMaps& maps, const RowParams& rp, int lonw, bool comp, int grid, cudaStream_t st) {
-  if constexpr (sizeof(CT) == 4) {
-    if (comp) return launch_tile_c<FT, CT, 11, 7, true, 32, 1, short>(maps, rp, lonw, grid, st);
-    return launch_tile_c<FT, CT, 11, 7, false, 32, 1, short>(maps, rp, lonw, grid, st);
-  } else if constexpr (sizeof(FT) == 4) {
-    return launch_tile_c<FT, CT, 7, 8, false, 32, 1, short>(maps, rp, lonw, grid, st);
-  } else {
-    return launch_tile_c<FT, CT, 11, 8, false, 32, 1, short>(maps, rp, lonw, grid, st);
+// `rows` (LEC_TILE_ROWS in LEC_TILE_ALL_SHAPES experiment builds) picks among the plain fp32 shapes 8, 11, 12 and 15.
+struct RingShape { int rows, stages; };
+constexpr RingShape ring_shape(bool f64, bool m64, bool comp, bool i16, int rows) {
+  if (i16) return f64 ? RingShape{11, 8} : m64 ? RingShape{7, 8} : RingShape{11, 7};
+  if (f64) return {11, 4};
+  if (m64) return {7, 6};
+  if (comp) return {11, 4};
+  return rows == 8 ? RingShape{8, 5} : rows == 11 || rows == 12 ? RingShape{rows, 4} : RingShape{15, 3};
+}
+
+template <typename FT, typename CT, int R, bool COMP, typename ST>
+cudaError_t launch_tile_c(const TmaMaps& maps, const RowParams& rp, int lonw, int grid, cudaStream_t st) {
+  constexpr RingShape shape = ring_shape(sizeof(FT) == 8, sizeof(CT) == 8, COMP, sizeof(ST) != sizeof(FT), R);
+  static_assert(shape.rows == R, "a ring shape of the table");
+  constexpr int S = shape.stages;
+  using G = TileGeom<FT, R, S, ST>;
+  cudaError_t e = cudaSuccess;
+#define LEC_TILE_LAUNCH(LW, TB, SMEM)                                                                             \
+  do {                                                                                                            \
+    e = cudaFuncSetAttribute(lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, ST>,                          \
+                             cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);                                  \
+    if (e == cudaSuccess) lec_row_moments_tile_kernel<FT, CT, LW, R, S, COMP, TB, ST><<<grid, G::threads, SMEM, st>>>(maps, rp); \
+  } while (0)
+  // fp32 per-column weights (LONW == 1): table in shared memory when it fits behind the ring
+  const int tab_bytes = (sizeof(ST) == sizeof(FT) ? (rp.g.nlon + 3) & ~3 : rp.pk.ntab) * 4;
+  if (lonw == 0) LEC_TILE_LAUNCH(0, false, G::smem_bytes);
+  else if (lonw == 1) {
+    if (sizeof(CT) == 4 && sizeof(FT) == 4 && G::smem_bytes + tab_bytes <= 227 * 1024) LEC_TILE_LAUNCH(1, true, G::smem_bytes + tab_bytes);
+    else LEC_TILE_LAUNCH(1, false, G::smem_bytes);
+  } else LEC_TILE_LAUNCH(2, false, G::smem_bytes);
+#undef LEC_TILE_LAUNCH
+  return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+// The row-kernel instance that `d` names, over fields of FT stored as ST (int16 when d.packed).
+template <typename FT, typename CT, bool COMP, typename ST>
+cudaError_t launch_rows_c(const lec_dispatch& d, const RowParams& rp, const TmaMaps& maps, long long grid, int num_sms,
+                          cudaStream_t st) {
+  constexpr int VEC = 16 / sizeof(FT);
+  if (d.kernel == LEC_ROWS_TILED) {
+    const int pgrid = (int)std::min<long long>(grid, (long long)num_sms);      // persistent: one CTA per SM
+#ifdef LEC_TILE_ALL_SHAPES
+    if constexpr (sizeof(CT) == 4 && !COMP && sizeof(ST) == sizeof(FT)) {
+      if (d.tile_rows == 8) return launch_tile_c<FT, CT, 8, COMP, ST>(maps, rp, d.lonw, pgrid, st);
+      if (d.tile_rows == 11) return launch_tile_c<FT, CT, 11, COMP, ST>(maps, rp, d.lonw, pgrid, st);
+      if (d.tile_rows == 12) return launch_tile_c<FT, CT, 12, COMP, ST>(maps, rp, d.lonw, pgrid, st);
+    }
+#endif
+    constexpr int R = ring_shape(sizeof(FT) == 8, sizeof(CT) == 8, COMP, sizeof(ST) != sizeof(FT), LEC_TILE_ROWS_DEFAULT).rows;
+    return launch_tile_c<FT, CT, R, COMP, ST>(maps, rp, d.lonw, pgrid, st);
   }
+  if (d.kernel == LEC_ROWS_SUBWARP) launch_narrow_c<FT, CT, VEC, COMP, ST>(rp, d.lonw != 0, d.group, grid, st);
+  else if constexpr (sizeof(ST) != sizeof(FT)) return cudaErrorInvalidValue;     // no direct kernel reads int16 fields
+  else if (d.vec == 1) launch_direct_c<FT, CT, 1, COMP>(rp, d.lonw, grid, st);
+  else launch_direct_c<FT, CT, VEC, COMP>(rp, d.lonw, grid, st);
+  return cudaGetLastError();
+}
+
+// COMP (compensated linear sums) only exists for fp32 arithmetic.
+template <typename FT, typename CT, typename ST>
+cudaError_t launch_rows_t(const lec_dispatch& d, const RowParams& rp, const TmaMaps& maps, long long grid, int num_sms,
+                          cudaStream_t st) {
+  if constexpr (sizeof(CT) == 4) {
+    if (d.comp) return launch_rows_c<FT, CT, true, ST>(d, rp, maps, grid, num_sms, st);
+  }
+  return launch_rows_c<FT, CT, false, ST>(d, rp, maps, grid, num_sms, st);
+}
+
+// Launches the row kernel of one batch: the instance `d` (filled by run_batch) names, over the handle's field dtype.
+cudaError_t launch_rows(const lec_handle* h, const lec_dispatch& d, const RowParams& rp, const TmaMaps& maps,
+                        long long grid, cudaStream_t st) {
+  const int sms = h->num_sms;
+  if (h->desc.dtype == LEC_F64) {
+    return d.packed ? launch_rows_t<double, double, short>(d, rp, maps, grid, sms, st)
+                    : launch_rows_t<double, double, double>(d, rp, maps, grid, sms, st);
+  }
+  if (d.math64) {
+    return d.packed ? launch_rows_t<float, double, short>(d, rp, maps, grid, sms, st)
+                    : launch_rows_t<float, double, float>(d, rp, maps, grid, sms, st);
+  }
+  return d.packed ? launch_rows_t<float, float, short>(d, rp, maps, grid, sms, st)
+                  : launch_rows_t<float, float, float>(d, rp, maps, grid, sms, st);
 }
 
 cudaEvent_t next_event(lec_handle* h) {
@@ -449,7 +430,6 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
   if (const char* e = std::getenv("LEC_PREFETCH")) h->prefetch_mode = std::atoi(e);
   if (const char* e = std::getenv("LEC_NARROW")) h->use_narrow = std::atoi(e) != 0;
   if (const char* e = std::getenv("LEC_COMP")) h->comp_mode = std::atoi(e) != 0;
-  if (const char* e = std::getenv("LEC_NARROW_TILE")) h->use_ntile = std::atoi(e) != 0;
   if (const char* e = std::getenv("LEC_TMA_HINT")) h->tma_hint = std::atoi(e) != 0;
   if (const char* e = std::getenv("LEC_NARROW_G")) {
     const int gq = std::atoi(e);
@@ -672,19 +652,22 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   // no other wide-box kernel (the caller's pitch makes every row 16-byte aligned)
   const bool want_tile = (h->use_tile || pk) && vec && !narrow_g && encode_tiled_fn() != nullptr;
   if (pk && !narrow_g && !want_tile) { h->err = "int16 fields need the TMA-tiled row kernel: no tensor-map encoder"; return LEC_ERR_CUDA; }
-  // tile height: fp32 arithmetic fits 128 registers -> 15 consumer warps + the producer (16 warps, 3 stages);
-  // fp64 arithmetic needs the 168 registers that at most 12 warps per CTA leave -> 11 rows, 4 stages
+  // The row-kernel instance of this batch, decided here once: launch_rows instantiates it and lec_last_dispatch
+  // reports it.  COMP only exists for fp32 arithmetic; the sub-warp kernel has no per-column-weight variant (any
+  // table is the full one).
   const bool math64 = h->desc.dtype == LEC_F64 || h->desc.math == LEC_MATH_F64;
-  const int tile_R = (math64 && h->desc.dtype != LEC_F64) ? 7 : (math64 || comp || pk) ? 11 : h->tile_rows;
-  // track boxes (8-lane row groups), fp32 arithmetic: the same TMA ring with 13 consumer warps x 4 rows; the box is
-  // cut into equal tiles of at most 52 rows
-  const bool want_ntile = !pk && h->use_tile && h->use_ntile && narrow_g == 8 && !math64 && !comp && encode_tiled_fn() != nullptr;
-  int ntile_rows = 0;
-  if (want_ntile) {
-    const int nt = (max_rows + kNarrowTileRows - 1) / kNarrowTileRows;
-    ntile_rows = (max_rows + nt - 1) / nt;
-  }
-  const int tile_rows = want_tile ? tile_R : want_ntile ? ntile_rows : narrow_g ? kNarrowWarps * (32 / narrow_g) : kRowsPerCta;
+  const int lonw = lon_mode(h);
+  lec_dispatch d{};
+  d.kernel = want_tile ? LEC_ROWS_TILED : narrow_g ? LEC_ROWS_SUBWARP : LEC_ROWS_DIRECT;
+  d.vec = vec ? vecw : 1;
+  d.group = d.kernel == LEC_ROWS_SUBWARP ? narrow_g : 32;
+  d.lonw = d.kernel == LEC_ROWS_SUBWARP && lonw != 0 ? 2 : lonw;
+  d.comp = comp && !math64;
+  d.math64 = math64;
+  d.tile_rows = d.kernel == LEC_ROWS_TILED ? ring_shape(h->desc.dtype == LEC_F64, math64, d.comp, pk, h->tile_rows).rows
+                : d.kernel == LEC_ROWS_SUBWARP ? kNarrowWarps * (32 / narrow_g) : kRowsPerCta;
+  d.packed = pk != nullptr;
+  const int tile_rows = d.tile_rows;
   band_rows = std::max(tile_rows, band_rows / tile_rows * tile_rows);
   // (moving boxes of one height were tried with the banded order too: 3.06 TB/s against 3.28 unbanded on the C5
   //  track -- a whole 151 x 151 x 55 step is 35 MB, so step-major order already keeps T(t+-1) in L2)
@@ -695,7 +678,6 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   RowParams rp{};
   for (int f = 0; f < 5; ++f) rp.field[f] = fields[f];
   rp.g = gd; rp.steps = ds; rp.rec = h->d_rec; rp.nsteps = n; rp.max_ny = h->max_ny;
-  rp.tile_rows = tile_rows;
   rp.tiles_per_band = band_rows / tile_rows;
   rp.dv_tiles = FastDiv::make((unsigned)rp.tiles_per_band);
   rp.dv_lev = FastDiv::make((unsigned)L);
@@ -710,32 +692,19 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   // TMA loads of u, v, omega, Phi with an L2 evict-first hint: fp64 fields only (46.7 -> 39.0 GB of DRAM reads per
   // 24-step launch, +3.4 %; with fp32 fields the working set of a band fits without it and the hint costs 2 %)
   rp.prefetch_mode = h->prefetch_mode | ((h->tma_hint < 0 ? h->desc.dtype == LEC_F64 : h->tma_hint != 0) ? 8 : 0);
-  {   // the template instance launched below, for lec_last_dispatch (COMP only exists for fp32 arithmetic; the
-      // sub-warp kernels have no per-column-weight variant: any table is the full one)
-    lec_dispatch& d = h->dispatch;
-    const int lonw = lon_mode(h);
-    d.kernel = want_tile ? LEC_ROWS_TILED : want_ntile ? LEC_ROWS_TILED_SUBWARP : narrow_g ? LEC_ROWS_SUBWARP : LEC_ROWS_DIRECT;
-    d.vec = vec ? vecw : 1;
-    d.group = want_tile ? 32 : want_ntile ? 8 : narrow_g ? narrow_g : 32;
-    d.lonw = (d.kernel == LEC_ROWS_SUBWARP || d.kernel == LEC_ROWS_TILED_SUBWARP) && lonw != 0 ? 2 : lonw;
-    d.comp = comp && !math64;
-    d.math64 = math64;
-    d.tile_rows = tile_rows; d.tiles_per_band = rp.tiles_per_band; d.nbands = rp.nbands;
-    d.packed = pk != nullptr;
-    h->dispatched = true;
-  }
+  d.tiles_per_band = rp.tiles_per_band; d.nbands = rp.nbands;
+  h->dispatch = d;
+  h->dispatched = true;
 
   cudaEvent_t e0 = next_event(h), e1 = next_event(h), e2 = next_event(h);
   if (!e0 || !e1 || !e2) { h->err = "cudaEventCreate"; return LEC_ERR_CUDA; }
   CK(cudaEventRecord(e0, st));
-  bool tma_done = false;
-  if (want_tile) {
+  TmaMaps maps;
+  if (d.kernel == LEC_ROWS_TILED) {
     const bool f64 = h->desc.dtype == LEC_F64;
-    const bool m64 = f64 || h->desc.math == LEC_MATH_F64;
-    const int C = f64 ? 64 : 128, V = f64 ? 2 : 4, R = tile_R;
+    const int C = f64 ? 64 : 128, V = f64 ? 2 : 4, R = d.tile_rows;
     // box widths of TileGeom: int16 boxes have 8 more columns and a 16-byte halo on each side (aligned box starts)
     const int esz = pk ? 2 : f64 ? 8 : 4, PW = pk ? C + 8 : C, HV = pk ? 8 : V;
-    TmaMaps maps;
     const int nlat = h->desc.nlat;
     bool ok = make_map(&maps.t_halo, fields[0], esz, nlon, nlat, L, nslots, PW + 2 * HV, R + 2) &&
               make_map(&maps.t_plain, fields[0], esz, nlon, nlat, L, nslots, PW, R) &&
@@ -744,52 +713,11 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
               make_map(&maps.w, fields[3], esz, nlon, nlat, L, nslots, PW, R) &&
               make_map(&maps.f, fields[4], esz, nlon, nlat, L, nslots, PW, R);
     if (!ok) { h->err = "cuTensorMapEncodeTiled failed"; return LEC_ERR_CUDA; }
-    const int pgrid = (int)std::min<long long>(grid, (long long)h->num_sms);
-    const int lonw = lon_mode(h);
-    cudaError_t e;
-    if (pk) e = f64 ? launch_tile_packed<double, double>(maps, rp, lonw, comp, pgrid, st)
-                    : (m64 ? launch_tile_packed<float, double>(maps, rp, lonw, comp, pgrid, st)
-                           : launch_tile_packed<float, float>(maps, rp, lonw, comp, pgrid, st));
-    else e = f64 ? launch_tile_t<double, double>(maps, rp, lonw, comp, R, pgrid, st)
-                 : (m64 ? launch_tile_t<float, double>(maps, rp, lonw, comp, R, pgrid, st)
-                        : launch_tile_t<float, float>(maps, rp, lonw, comp, h->tile_rows, pgrid, st));
-    if (e != cudaSuccess) { h->err = std::string("tiled row kernel launch: ") + cudaGetErrorString(e); return LEC_ERR_CUDA; }
-    tma_done = true;
   }
-  if (!tma_done && want_ntile) {
-    constexpr int C = 8 * 4, V = 4;
-    TmaMaps maps;
-    const int nlat = h->desc.nlat, R = ntile_rows;
-    const int pm = 3;      // L2 promotion of the tensor maps: none / 64 B / 128 B / 256 B measured 2.09 / 2.16 / 2.10 / 2.06 ms
-    bool ok = make_map(&maps.t_halo, fields[0], 4, nlon, nlat, L, nslots, C + 2 * V, R + 2, pm) &&
-              make_map(&maps.t_plain, fields[0], 4, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.u, fields[1], 4, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.v, fields[2], 4, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.w, fields[3], 4, nlon, nlat, L, nslots, C, R, pm) &&
-              make_map(&maps.f, fields[4], 4, nlon, nlat, L, nslots, C, R, pm);
-    if (!ok) { h->err = "cuTensorMapEncodeTiled failed"; return LEC_ERR_CUDA; }
-    const int pgrid = (int)std::min<long long>(grid, (long long)h->num_sms * kNarrowTileCtas);
-    cudaError_t e = launch_tile_c<float, float, kNarrowTileWarps, 3, false, 8, kNarrowTileCtas>(maps, rp, lon_mode(h), pgrid, st);
-    if (e != cudaSuccess) { h->err = std::string("tiled sub-warp row kernel launch: ") + cudaGetErrorString(e); return LEC_ERR_CUDA; }
-    tma_done = true;
-  }
-  if (!tma_done && narrow_g) {
-    const bool f64 = h->desc.dtype == LEC_F64;
-    const bool m64 = f64 || h->desc.math == LEC_MATH_F64;
-    const bool table = lon_mode(h) != 0;
-    if (pk) {
-      if (f64) launch_narrow_t<double, double, 2, short>(rp, table, comp, narrow_g, grid, st);
-      else if (m64) launch_narrow_t<float, double, 4, short>(rp, table, comp, narrow_g, grid, st);
-      else launch_narrow_t<float, float, 4, short>(rp, table, comp, narrow_g, grid, st);
-    } else if (f64) launch_narrow_t<double, double, 2>(rp, table, comp, narrow_g, grid, st);
-    else if (m64) launch_narrow_t<float, double, 4>(rp, table, comp, narrow_g, grid, st);
-    else launch_narrow_t<float, float, 4>(rp, table, comp, narrow_g, grid, st);
-    CK(cudaGetLastError());
-    tma_done = true;
-  }
-  if (!tma_done) {
-    launch_rows(h, rp, vec, comp, grid, st);
-    CK(cudaGetLastError());
+  const cudaError_t le = launch_rows(h, d, rp, maps, grid, st);
+  if (le != cudaSuccess) {
+    h->err = std::string(d.kernel == LEC_ROWS_TILED ? "tiled row kernel launch: " : "cudaGetLastError(): ") + cudaGetErrorString(le);
+    return LEC_ERR_CUDA;
   }
   CK(cudaEventRecord(e1, st));
   FinParams fp{};

@@ -18,14 +18,11 @@
 // is fixed, so results are bit-reproducible across launches, shards and GPUs.
 #pragma once
 #include "lec_common.cuh"
-#include "lec_packed.cuh"
+#include "lec_pair.cuh"
 
 namespace lec {
 
-#ifndef LEC_ROWS_PER_CTA
-#define LEC_ROWS_PER_CTA 2
-#endif
-constexpr int kRowsPerCta = LEC_ROWS_PER_CTA; // warps per CTA, one row each (adjacent rows share L1 lines)
+constexpr int kRowsPerCta = 2;                // warps per CTA, one row each (adjacent rows share L1 lines)
 constexpr int kRowThreads = kRowsPerCta * 32;
 
 // Division of a 31-bit numerator by a run-time constant as one wide multiply and a shift (the block / tile index is
@@ -70,10 +67,9 @@ struct RowParams {
   double* rec;
   int nsteps;
   int max_ny;            // record rows reserved per (step, level)
-  int tile_rows;         // TMA-tiled kernel: rows of a tile (the box height of the tensor maps)
+  int nbands;            // (read by the host only)
   int tiles_per_band;    // CTA row-tiles per latitude band
   FastDiv dv_tiles, dv_lev, dv_steps;   // block / tile index -> (band, step, level, row tile)
-  int nbands;
   long long slot_stride; // elements per slot = nlev*nlat*nlon
   int prefetch_mode;     // bit 0: L2 bulk prefetch of the DRAM-sourced rows at row start
   long long grid;        // number of CTAs
@@ -92,9 +88,6 @@ __device__ __forceinline__ void prefetch_l2_range(const void* p, long long lo_by
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(lo), "r"(n) : "memory");
 }
 
-#ifdef LEC_NO_STREAM     // experiment: u, v, omega, Phi through the normal-priority read-only path as well
-#define __ldcs __ldg
-#endif
 template <typename FT, int VEC> struct VecLoad;
 template <> struct VecLoad<float, 4> {
   static __device__ __forceinline__ void ld(const float* p, float (&v)[4]) {
@@ -212,8 +205,6 @@ struct RowCoefS {
 constexpr int R_NLIN = 6;   // the linear sums S_a .. S_q carry a compensation term in fp32 arithmetic
 
 // s += x with the rounding error of the addition collected in c (FastTwoSum: exact when |s| >= |x|, i.e.
-// whenever the error matters).  fp64 arithmetic needs none.
-// s += x with the rounding error of the addition collected in c (FastTwoSum: exact when |s| >= |x|, i.e.
 // whenever the error matters).  COMP is chosen per launch: the compensation matters when a lane adds many
 // chunks (long rows) while the terms are built from small differences of zonal means (a box of few rows);
 // fp64 arithmetic needs none.
@@ -292,11 +283,9 @@ struct RowSetup {
 
 // LONW: 0 = uniform longitudes (weight applied once after the reduction), 1 = per-column trapezoid
 // weights with a uniform lon stencil, 2 = per-column weights and stencil (irregular longitudes).
-#ifndef LEC_ROW_MIN_CTAS
-#define LEC_ROW_MIN_CTAS (512 / kRowThreads)
-#endif
+// CTAs per SM: 8 (16 warps), 6 (12 warps) for fp64 arithmetic and compensated fp32 sums
 template <typename FT, typename CT, int VEC, int LONW, bool COMP>
-__global__ void __launch_bounds__(kRowThreads, sizeof(CT) == 8 ? (LEC_ROW_MIN_CTAS * 3) / 4 : COMP ? (LEC_ROW_MIN_CTAS * 3) / 4 : LEC_ROW_MIN_CTAS)   // fp64 arithmetic and compensated fp32 sums: 12 warps/SM
+__global__ void __launch_bounds__(kRowThreads, sizeof(CT) == 8 || COMP ? 6 : 8)
 lec_row_moments_kernel(const RowParams p) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // CTA order: band-major, then step, level, row-tile.  Sweeping time inside a latitude

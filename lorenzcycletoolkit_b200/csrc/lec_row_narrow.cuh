@@ -8,7 +8,7 @@
 // the row records are those of the wide kernel.
 #pragma once
 #include "lec_common.cuh"
-#include "lec_packed.cuh"
+#include "lec_pair.cuh"
 #include "lec_row_moments.cuh"
 
 namespace lec {

@@ -16,16 +16,12 @@
 //    shuffle (lanes 0 / 31: one LDS.32 of the halo column) -> the shared iteration body (lec_row_body.inc)
 //    -> arrive(empty).  No global addressing, no long-scoreboard stalls in the arithmetic warps; rows
 //    outside the box or the grid are zero-filled by TMA and masked as before.
-//  * GL < 32 (track boxes, opt-in): a row is swept by a group of GL lanes, a consumer warp carries 32/GL rows,
-//    a chunk is GL x 128 bit wide and the tile height is chosen by the host -- the lane <-> row / column
-//    mapping and the group butterfly of lec_row_moments_narrow_kernel, so again the same bits.
 #pragma once
 #include <cuda.h>
 
 #include "lec_common.cuh"
-#include "lec_packed.cuh"
+#include "lec_pair.cuh"
 #include "lec_row_moments.cuh"
-#include "lec_row_narrow.cuh"
 
 namespace lec {
 
@@ -35,35 +31,29 @@ struct alignas(64) TmaMaps {
   CUtensorMap u, v, w, f;
 };
 
-// GL = lanes that sweep one row: 32 (a warp per row, wide boxes) or 16 / 8 (Semi-Lagrangian track boxes: a warp
-// carries 32/GL rows, a chunk is GL x 128 bit wide -- the lane <-> row / column mapping of the sub-warp kernel).
-// R = consumer warps; a tile has up to R * 32/GL rows (the host picks the height actually used, RowParams::tile_rows,
-// so that a box of any height is cut into equal tiles -- the TMA box height lives in the tensor map, not in the code).
+// R = consumer warps = rows of a tile (the box height of the tensor maps); a chunk is 32 x 128 bit of a row.
 // ST = stored element type: FT, or int16 (lec_run_device_packed), which keeps the lane <-> column map of FT (VEC) and
 // shrinks the ring's bytes.  Every TMA box starts on a 16-byte boundary of the row: the fp chunks do by construction
 // (VEC columns = 16 bytes), an int16 chunk starts at column c0 * VEC, a multiple of 4 (fp32) or 2 (fp64) only, so the
 // int16 boxes start at that column rounded down to a multiple of 8 and are 8 columns wider (PW); the consumers add the
 // row's shift (c0 * VEC) & 7.  The int16 lon halo is 8 columns (16 bytes) a side.
-template <typename FT, int R, int NSTG, int GL = 32, typename ST = FT>
+template <typename FT, int R, int NSTG, typename ST = FT>
 struct TileGeom {
   static constexpr bool I16 = sizeof(ST) != sizeof(FT);
   static constexpr int VEC = 16 / sizeof(FT);
   static constexpr int HV = I16 ? 8 : VEC;                   // lon halo columns each side (16 bytes)
-  static constexpr int RPW = 32 / GL;                        // rows per consumer warp
-  static constexpr int ROWS = R * RPW;                       // most rows a tile can hold
-  static constexpr int C = GL * VEC;                         // columns per chunk
+  static constexpr int C = 32 * VEC;                         // columns per chunk
   static constexpr int PW = I16 ? C + 8 : C;                 // plain tile pitch (elements)
   static constexpr int HP = PW + 2 * HV;                     // halo tile pitch (elements)
   static_assert(HP * sizeof(ST) % 16 == 0 && PW * sizeof(ST) % 16 == 0, "TMA boxes are whole 16-byte units wide");
-  static constexpr int halo_bytes = (ROWS + 2) * HP * sizeof(ST);
+  static constexpr int halo_bytes = (R + 2) * HP * sizeof(ST);
   static constexpr int halo_bytes_pad = (halo_bytes + 127) / 128 * 128;
   // (int16: every plain tile starts on a 128-byte boundary, the alignment of a TMA destination)
-  static constexpr int tile_bytes = I16 ? (ROWS * PW * (int)sizeof(ST) + 127) / 128 * 128 : ROWS * C * sizeof(ST);
+  static constexpr int tile_bytes = I16 ? (R * PW * (int)sizeof(ST) + 127) / 128 * 128 : R * C * sizeof(ST);
   static constexpr int stage_bytes = halo_bytes_pad + 8 * tile_bytes;
   static constexpr int smem_bytes = NSTG * stage_bytes + 128;               // + barriers
   static constexpr int threads = (R + 1) * 32;                           // R consumer warps + the producer warp
-  // what the 9 loads of a chunk deliver when the tile is `rows` high
-  static __host__ __device__ constexpr int tx_bytes(int rows) { return ((rows + 2) * HP + 8 * rows * PW) * (int)sizeof(ST); }
+  static constexpr int tx_bytes = ((R + 2) * HP + 8 * R * PW) * (int)sizeof(ST);   // what the 9 loads of a chunk deliver
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -154,16 +144,6 @@ __device__ __forceinline__ FT lds_elem(unsigned a, const PackedDev& pk) {
   }
 }
 
-// longitude-table load of the shared body: from shared memory (plain load, address space known) or global
-template <bool SHARED, int VEC>
-__device__ __forceinline__ void tab_load(const float* ptr, float (&v)[VEC]) {
-  if constexpr (SHARED && VEC == 4) {
-    const float4 t = *reinterpret_cast<const float4*>(ptr); v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-  } else {
-    VecLoad<float, VEC>::ld(ptr, v);
-  }
-}
-
 // the tiled kernel's weight load: by 32-bit shared address when the table was copied behind the ring
 template <bool SHARED, int VEC>
 __device__ __forceinline__ void tab_load_tile(const float* ptr, unsigned saddr, float (&v)[VEC]) {
@@ -185,16 +165,11 @@ __device__ __forceinline__ TileId decode_tile(unsigned id, const RowParams& p) {
   return t;
 }
 
-// MINB = CTAs per SM (1; two to four smaller CTAs at different phases were tried for track boxes and were slower)
-template <typename FT, typename CT, int LONW, int R, int NSTG, bool COMP, bool TABS, int GL = 32, int MINB = 1, typename ST = FT>
-__global__ void __launch_bounds__((R + 1) * 32, MINB)
+template <typename FT, typename CT, int LONW, int R, int NSTG, bool COMP, bool TABS, typename ST = FT>
+__global__ void __launch_bounds__((R + 1) * 32, 1)
 lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParams p) {
-  using G = TileGeom<FT, R, NSTG, GL, ST>;
-  constexpr int VEC = G::VEC, C = G::C, PW = G::PW, HP = G::HP, HV = G::HV, RPW = G::RPW;
-  static_assert(!G::I16 || GL == 32, "int16 fields: one warp per row");
-  // rows of a tile = the TMA box height: R for a warp per row (compile-time tile offsets), chosen by the host for
-  // track boxes (<= G::ROWS)
-  const int trows = (GL == 32) ? R : p.tile_rows;
+  using G = TileGeom<FT, R, NSTG, ST>;
+  constexpr int VEC = G::VEC, C = G::C, PW = G::PW, HP = G::HP, HV = G::HV;
   extern __shared__ __align__(1024) unsigned char smem[];   // plain shared pointer: keeps LDS (not generic LD)
   unsigned long long* bars = reinterpret_cast<unsigned long long*>(smem + NSTG * G::stage_bytes);
   const unsigned full0 = smem_u32(bars), empty0 = smem_u32(bars + NSTG);
@@ -229,13 +204,10 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
       for (unsigned id = blockIdx.x; id < (unsigned)p.grid; id += gridDim.x) {
         const TileId t = decode_tile(id, p);
         const StepDev* __restrict__ st = p.steps + t.s;
-        const int jr = (t.band * p.tiles_per_band + t.jt) * trows;
+        const int jr = (t.band * p.tiles_per_band + t.jt) * R;
         if (jr > st->j1 - st->j0) continue;
         const int c0 = st->i0 / VEC, c1 = st->i1 / VEC;
-        const int nch = (c1 - c0 + GL) / GL;
-        const unsigned tx = (unsigned)G::tx_bytes(trows);
-        // the plain tiles are packed at the runtime height (int16: one warp per row, so trows == R)
-        const unsigned tile_b = G::I16 ? (unsigned)G::tile_bytes : (unsigned)(trows * C * (int)sizeof(ST));
+        const int nch = (c1 - c0 + 32) / 32;
         const int jt0 = st->j0 + jr;
         const int k = t.k, km = k > 0 ? k - 1 : k, kp = k < nlev - 1 ? k + 1 : k;
         const int slot = st->slot, slot_m = st->slot_m, slot_p = st->slot_p;
@@ -249,24 +221,24 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
             if (++stg == NSTG) { stg = 0; phase ^= 1; }
             continue;
           }
-          mbar_expect_tx(fb, tx);
+          mbar_expect_tx(fb, (unsigned)G::tx_bytes);
           const unsigned base = smem_u32(smem) + (unsigned)stg * G::stage_bytes;
           tma_load_4d(base, &maps.t_halo, fb, col - HV, jt0 - 1, k, slot);
           unsigned d = base + G::halo_bytes_pad;
           if (p.prefetch_mode & 8) {
-            tma_load_4d_hint(d, &maps.u, fb, col, jt0, k, slot, pol_stream); d += tile_b;
-            tma_load_4d_hint(d, &maps.v, fb, col, jt0, k, slot, pol_stream); d += tile_b;
-            tma_load_4d_hint(d, &maps.w, fb, col, jt0, k, slot, pol_stream); d += tile_b;
-            tma_load_4d_hint(d, &maps.f, fb, col, jt0, k, slot, pol_stream); d += tile_b;
+            tma_load_4d_hint(d, &maps.u, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.v, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.w, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.f, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
           } else {
-            tma_load_4d(d, &maps.u, fb, col, jt0, k, slot); d += tile_b;
-            tma_load_4d(d, &maps.v, fb, col, jt0, k, slot); d += tile_b;
-            tma_load_4d(d, &maps.w, fb, col, jt0, k, slot); d += tile_b;
-            tma_load_4d(d, &maps.f, fb, col, jt0, k, slot); d += tile_b;
+            tma_load_4d(d, &maps.u, fb, col, jt0, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.v, fb, col, jt0, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.w, fb, col, jt0, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.f, fb, col, jt0, k, slot); d += G::tile_bytes;
           }
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, k, slot_p); d += tile_b;
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, k, slot_m); d += tile_b;
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, km, slot); d += tile_b;
+          tma_load_4d(d, &maps.t_plain, fb, col, jt0, k, slot_p); d += G::tile_bytes;
+          tma_load_4d(d, &maps.t_plain, fb, col, jt0, k, slot_m); d += G::tile_bytes;
+          tma_load_4d(d, &maps.t_plain, fb, col, jt0, km, slot); d += G::tile_bytes;
           tma_load_4d(d, &maps.t_plain, fb, col, jt0, kp, slot);
           if (++stg == NSTG) { stg = 0; phase ^= 1; }
         }
@@ -278,11 +250,9 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
   // ======================================= consumers ===========================================
   // per-lane tile offsets (bytes): own row of the halo tile (warp + 1) and of the eight plain tiles
   const unsigned sbase0 = smem_u32(smem);
-  const int gl = lane & (GL - 1);                      // lane within the row's group
-  const int rowt = warp * RPW + lane / GL;             // row within the tile
-  const unsigned off_hc = (unsigned)(((rowt + 1) * HP + HV + gl * VEC) * sizeof(ST));
-  const unsigned off_t = (unsigned)(G::halo_bytes_pad + (rowt * PW + gl * VEC) * sizeof(ST));
-  const unsigned kTile = G::I16 ? (unsigned)G::tile_bytes : (unsigned)(trows * C * (int)sizeof(ST));
+  const unsigned off_hc = (unsigned)(((warp + 1) * HP + HV + lane * VEC) * sizeof(ST));
+  const unsigned off_t = (unsigned)(G::halo_bytes_pad + (warp * PW + lane * VEC) * sizeof(ST));
+  constexpr unsigned kTile = G::tile_bytes;
   // current stage: base address, its full barrier (the empty one sits 8 NSTG bytes behind it), index, phase; the
   // advance wraps by subtraction, so the ring needs no second copy of the base addresses in registers
   unsigned sb = sbase0, fb = full0;
@@ -295,17 +265,16 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
     const TileId t = decode_tile(id, p);
     const StepDev* __restrict__ st = p.steps + t.s;
     const int i0 = st->i0, i1 = st->i1, j0 = st->j0, j1 = st->j1;
-    const int jrel0 = (t.band * p.tiles_per_band + t.jt) * trows;
+    const int jrel0 = (t.band * p.tiles_per_band + t.jt) * R;
     if (jrel0 > j1 - j0) continue;                 // same test as the producer: no chunk was issued
-    // warp_on: the warp has work in this tile (warp-uniform: shuffles below); row_on: so has this lane's row --
-    // rows of a live warp that lie past the tile or the box sweep the clamped last row and write nothing
-    const bool warp_on = (warp * RPW < trows) && (jrel0 + warp * RPW <= j1 - j0) && !(p.prefetch_mode & 4);   // (bit 2: timing experiment, no arithmetic)
-    const bool row_on = warp_on && (rowt < trows) && (jrel0 + rowt <= j1 - j0);
-    const int jrel = row_on ? jrel0 + rowt : j1 - j0;
+    // warp_on: the warp's row lies in the tile and the box (warp-uniform: shuffles below); warps past the box sweep
+    // the clamped last row and write nothing
+    const bool warp_on = (warp < R) && (jrel0 + warp <= j1 - j0) && !(p.prefetch_mode & 4);   // (bit 2: timing experiment, no arithmetic)
+    const int jrel = warp_on ? jrel0 + warp : j1 - j0;
     const int j = j0 + jrel;
     const int k = t.k;
     const int c0 = i0 / VEC, c1 = i1 / VEC;
-    const int niter = (c1 - c0 + GL) / GL;
+    const int niter = (c1 - c0 + 32) / 32;
     // int16: the row's first chunk sits this many bytes into the (16-byte aligned) boxes; 0 for fp fields
     const unsigned adj = G::I16 ? (unsigned)(((c0 * VEC) & 7) * (int)sizeof(ST)) : 0u;
 
@@ -366,25 +335,11 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
 #pragma unroll
         for (int n = 0; n < R_NLIN; ++n) Sd[n] += double(Cc[n]);
       }
-      if constexpr (GL == 32) {
-        double tot = butterfly_reduce<R_NSUM>(Sd, lane);
-        if (LONW == 0) tot *= p.g.wl_u;
-        const int idx = bitrev5(lane);
-        if (idx < R_NSUM) rec[idx] = tot;
-      } else {
-        constexpr int NOUT = (R_NSUM + GL - 1) / GL;
-        double tot[NOUT];
-        butterfly_reduce_seg<R_NSUM, GL>(Sd, gl, tot);
-        if (row_on) {
-          const int r = bitrev_group<GL>(gl);
-#pragma unroll
-          for (int m = 0; m < NOUT; ++m) {
-            const int idx = r + m * GL;
-            if (idx < R_NSUM) rec[idx] = (LONW == 0) ? tot[m] * p.g.wl_u : tot[m];
-          }
-        }
-      }
-      if (row_on && gl == 1) {   // raw (unscaled) shifts; the finalize kernel applies the unit scales
+      double tot = butterfly_reduce<R_NSUM>(Sd, lane);
+      if (LONW == 0) tot *= p.g.wl_u;
+      const int idx = bitrev5(lane);
+      if (idx < R_NSUM) rec[idx] = tot;
+      if (lane == 1) {   // raw (unscaled) shifts; the finalize kernel applies the unit scales
         rec[R_SH_T] = double(shT); rec[R_SH_U] = double(shU); rec[R_SH_V] = double(shV);
         rec[R_SH_W] = double(shW); rec[R_SH_F] = double(shF);
       }

@@ -74,7 +74,7 @@ class _Dispatch(C.Structure):
                                          "tiles_per_band", "nbands", "packed")]
 
 
-ROW_KERNELS = ("direct", "subwarp", "tiled", "tiled_subwarp")      # lec_dispatch.kernel (LEC_ROWS_*)
+ROW_KERNELS = ("direct", "subwarp", "tiled")      # lec_dispatch.kernel (LEC_ROWS_*)
 
 LEC_RAW_F32, LEC_RAW_F64, LEC_RAW_I16 = 0, 1, 2
 _RAW_DTYPES = {np.dtype(np.float32): LEC_RAW_F32, np.dtype(np.float64): LEC_RAW_F64, np.dtype(np.int16): LEC_RAW_I16}

@@ -12,7 +12,6 @@ or 2 fp64 columns; a box row covers ``i1 // vecw - i0 // vecw + 1`` chunks):
   longitude tables LONW = 0 / 1 / 2                 exactly uniform / per-column weights / irregular stencil
   scalar direct kernel (VEC = 1)                    caller-owned device rows that are not 16-byte aligned
   vector direct kernel                              LEC_ROW_KERNEL=direct (opt-in)
-  tiled sub-warp kernel                             LEC_NARROW_TILE=1 (opt-in)
   latitude-banded block order                       lec_grid_desc.band_rows > 0, fixed and moving boxes
 
 Cells of 16-byte aligned rows run through ``lec_run_host`` (rows padded to whole chunks) and through
@@ -44,7 +43,7 @@ RECORDS = []                                            # (dispatch record + cas
 
 @pytest.fixture(autouse=True)
 def _default_dispatcher(monkeypatch):
-    for k in ("LEC_ROW_KERNEL", "LEC_NARROW", "LEC_NARROW_TILE", "LEC_NARROW_G", "LEC_COMP"):
+    for k in ("LEC_ROW_KERNEL", "LEC_NARROW", "LEC_NARROW_G", "LEC_COMP"):
         monkeypatch.delenv(k, raising=False)
 
 
@@ -247,15 +246,6 @@ def test_vector_direct_kernel(arith, coords, monkeypatch):
                                                     comp=False, math64=arith != "f32", tile_rows=2))
 
 
-@pytest.mark.parametrize("coords", ["exact", "f32"])
-def test_tiled_sub_warp_kernel(coords, monkeypatch):
-    """``LEC_NARROW_TILE=1``: 8-lane row groups fed by the TMA ring, 129 rows cut into three tiles of 43."""
-    monkeypatch.setenv("LEC_NARROW_TILE", "1")
-    box = _box(112, 4, 5, 1, 129)
-    _cell((coords,) + WIDE, [box] * NT, "f32", dict(kernel="tiled_subwarp", vec=4, group=8,
-                                                     lonw=0 if coords == "exact" else 2, comp=False, tile_rows=43))
-
-
 @pytest.mark.parametrize("arith", ["f32", "m64", "f64"])
 @pytest.mark.parametrize("chunks", [5, 201])
 def test_direct_kernel_on_a_misaligned_base(chunks, arith):
@@ -291,8 +281,6 @@ BAND_GRID = ("exact", 406, 70)        # 406 % 4 == 2: fp32 device rows are not 1
 BAND_FAMILIES = {
     "subwarp": ("f32", "host", {}, (3, 150, 3, 63), [(3, 150, 3, 63), (6, 153, 5, 65), (1, 148, 4, 64), (8, 155, 6, 66)]),
     "tiled": ("f64", "host", {}, (1, 401, 3, 63), [(1, 401, 3, 63), (0, 400, 5, 65), (4, 404, 4, 64), (2, 402, 6, 66)]),
-    "tiled_subwarp": ("f32", "host", {"LEC_NARROW_TILE": "1"}, (3, 150, 3, 63),
-                      [(3, 150, 3, 63), (6, 153, 5, 65), (1, 148, 4, 64), (8, 155, 6, 66)]),
     "direct": ("f32", "torch", {}, (3, 150, 3, 63), [(3, 150, 3, 63), (6, 153, 5, 65), (1, 148, 4, 64), (8, 155, 6, 66)]),
 }
 BAND_CASES = [(f, m) for f in BAND_FAMILIES for m in ("fixed", "moving")]
@@ -334,13 +322,13 @@ def _cells_required():
             for k, c, r, comp in (("subwarp", 128, 128, False), ("subwarp", 129, 128, True), ("subwarp", 200, 128, True),
                                   ("subwarp", 200, 129, False), ("tiled", 201, 128, True), ("tiled", 201, 129, False))]
     req += [dict(kernel="tiled", arith="f32", comp=True, tile_rows=11)]
-    for kernel, lonws in (("direct", (0, 1, 2)), ("subwarp", (0, 2)), ("tiled", (0, 1, 2)), ("tiled_subwarp", (0, 2))):
+    for kernel, lonws in (("direct", (0, 1, 2)), ("subwarp", (0, 2)), ("tiled", (0, 1, 2))):
         req += [dict(kernel=kernel, lonw=w) for w in lonws]
         req += [dict(kernel=kernel, banded=True, moving=m) for m in (False, True)]
     return req
 
 
-N_CASES = (len(WIDTHS) * 9 + 6 + len(COMP_CASES) + len(VECTOR_DIRECT) + 2 + 6 + len(SCALAR_GRIDS) * 3
+N_CASES = (len(WIDTHS) * 9 + 6 + len(COMP_CASES) + len(VECTOR_DIRECT) + 6 + len(SCALAR_GRIDS) * 3
            + len(BAND_CASES))
 
 

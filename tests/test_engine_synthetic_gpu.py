@@ -362,12 +362,10 @@ def test_tiled_kernel_has_the_bits_of_the_direct_kernel(dtype, coords, monkeypat
     assert np.isnan(out["tile"][0]).any() and np.isfinite(out["tile"][0][3]).all()
 
 
-def test_tiled_sub_warp_kernel_has_the_bits_of_the_direct_sub_warp_kernel(monkeypatch):
-    """``LEC_NARROW_TILE=1`` feeds the 8-lane row groups of the track-box kernel from the TMA ring (tiles of equal
-    height cut from the box, four rows per consumer warp).  Lane <-> column mapping, accumulation order and the
-    group butterfly are those of the direct-load sub-warp kernel, so terms and per-level integrands must be
-    IDENTICAL: moving boxes of different sizes (odd start columns, heights that are no multiple of a warp's four
-    rows or of the tile, boxes on the grid edges) and NaNs outside / inside the boxes."""
+def test_sub_warp_kernel_reports_nans_only_for_the_boxes_that_hold_them():
+    """Track boxes take the sub-warp kernel with 8-lane row groups: moving boxes of different sizes (odd start
+    columns, heights that are no multiple of a warp's four rows, boxes on the grid edges), a NaN inside one box and a
+    NaN row outside every box but the last.  Only the steps whose box holds a NaN may report one."""
     nlon, nlat, nlev, nt = 260, 232, 5, 6
     lon = (-70.0 + 0.1 * np.arange(nlon)).astype(np.float32)
     lat = (-42.0 + 0.1 * np.arange(nlat)).astype(np.float32)
@@ -378,12 +376,8 @@ def test_tiled_sub_warp_kernel_has_the_bits_of_the_direct_sub_warp_kernel(monkey
     boxes = [(5, 155, 1, 151), (1, 151, 3, 153), (30, 180, 33, 97), (109, 259, 81, 231), (7, 67, 100, 160), (0, 150, 0, 150)]
     for it, (i0, i1, j0, j1) in enumerate(boxes):
         steps["i0"][it], steps["i1"][it], steps["j0"][it], steps["j1"][it] = i0, i1, j0, j1
-    out = {}
-    for tiled in ("0", "1"):
-        monkeypatch.setenv("LEC_NARROW_TILE", tiled)
-        with H.make_engine(P, np.float32, [1.0] * 5, max_box_rows=151) as eng:
-            out[tiled] = eng.run_host(fields, steps)
-    for x, y in zip(out["0"], out["1"]):
-        assert np.array_equal(x, y, equal_nan=True)
-    terms = out["1"][0]
+    with H.make_engine(P, np.float32, [1.0] * 5, max_box_rows=151) as eng:
+        terms = eng.run_host(fields, steps)[0]
+        d = eng.last_dispatch()
+    assert d["kernel"] == "subwarp" and d["group"] == 8, d
     assert np.isnan(terms[2]).any() and np.isnan(terms[5]).any() and np.isfinite(terms[[0, 1, 3, 4]]).all()

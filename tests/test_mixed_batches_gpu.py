@@ -37,7 +37,7 @@ WIDE = (816, 131)            # fp32: 204 chunks per row, fp64: 408
 
 @pytest.fixture(autouse=True)
 def _default_dispatcher(monkeypatch):
-    for k in ("LEC_ROW_KERNEL", "LEC_NARROW", "LEC_NARROW_TILE", "LEC_NARROW_G", "LEC_COMP"):
+    for k in ("LEC_ROW_KERNEL", "LEC_NARROW", "LEC_NARROW_G", "LEC_COMP"):
         monkeypatch.delenv(k, raising=False)
 
 

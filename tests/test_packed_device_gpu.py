@@ -31,7 +31,7 @@ WIDE = (816, 131)
 
 @pytest.fixture(autouse=True)
 def _default_dispatcher(monkeypatch):
-    for k in ("LEC_ROW_KERNEL", "LEC_NARROW", "LEC_NARROW_TILE", "LEC_NARROW_G", "LEC_COMP"):
+    for k in ("LEC_ROW_KERNEL", "LEC_NARROW", "LEC_NARROW_G", "LEC_COMP"):
         monkeypatch.delenv(k, raising=False)
 
 
@@ -216,9 +216,8 @@ def test_a_fill_inside_the_box_raises_the_nonfinite_flag(kernel, arith, field):
         assert not (np.delete(a[2], 1) & E.FLAG_NONFINITE).any()
 
 
-def test_direct_and_tiled_sub_warp_switches_do_not_apply(monkeypatch):
+def test_the_direct_kernel_switch_does_not_apply(monkeypatch):
     monkeypatch.setenv("LEC_ROW_KERNEL", "direct")
-    monkeypatch.setenv("LEC_NARROW_TILE", "1")
     P, fields = _dataset("f32", *WIDE)
     raws, decode = H.encode(fields, _decode_spec("f32"))
     for chunks, kernel in ((60, "subwarp"), (201, "tiled")):

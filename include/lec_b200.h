@@ -116,6 +116,12 @@ typedef struct lec_grid_desc {
  * over (lec_gradient_coefs gives them); this is what lets a time shard carry a
  * one-slot halo.  The box is inclusive index bounds on the prepared grid
  * (box_data.py:115-135 nearest snap; lec_nearest_index reproduces it).
+ * slot_m and slot_p may be any slots of the buffer, with one limit: in a kernel
+ * batch that runs the direct or the sub-warp row kernel (LEC_ROWS_DIRECT /
+ * LEC_ROWS_SUBWARP), |slot_m - slot| and |slot_p - slot| times the elements of
+ * one slot (nlev * nlat * row length) must stay below 2^31; such a batch fails
+ * with LEC_ERR_INVALID and a lec_last_error text.  The tiled kernel
+ * (LEC_ROWS_TILED, wide boxes) has no such limit.
  */
 typedef struct lec_step {
   int32_t slot, slot_m, slot_p;

@@ -605,15 +605,6 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   for (int s = 0; s < n; ++s) {
     const int rc = build_step(h, steps[s], nslots, hs[s]);
     if (rc != LEC_OK) return rc;
-    {   // the kernels address T(t-1), T(t+1) as 32-bit element offsets from T(t)
-      const long long stride = (long long)L * h->desc.nlat * nlon;
-      const long long dm = (long long)(steps[s].slot_m - steps[s].slot) * stride;
-      const long long dp = (long long)(steps[s].slot_p - steps[s].slot) * stride;
-      if (dm <= -(1LL << 31) || dm >= (1LL << 31) || dp <= -(1LL << 31) || dp >= (1LL << 31)) {
-        h->err = "slot_m / slot_p are too far from slot (offset exceeds 2^31 elements)";
-        return LEC_ERR_INVALID;
-      }
-    }
     max_rows = std::max(max_rows, steps[s].j1 - steps[s].j0 + 1);
     max_cols = std::max(max_cols, steps[s].i1 - steps[s].i0 + 1);
     same_box = same_box && steps[s].i0 == steps[0].i0 && steps[s].i1 == steps[0].i1 &&
@@ -667,6 +658,21 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   d.tile_rows = d.kernel == LEC_ROWS_TILED ? ring_shape(h->desc.dtype == LEC_F64, math64, d.comp, pk, h->tile_rows).rows
                 : d.kernel == LEC_ROWS_SUBWARP ? kNarrowWarps * (32 / narrow_g) : kRowsPerCta;
   d.packed = pk != nullptr;
+  if (d.kernel != LEC_ROWS_TILED) {
+    // The direct and sub-warp kernels address T(slot_m) and T(slot_p) as 32-bit element offsets from T(slot) (64-bit
+    // bases instead spill in the sub-warp kernel's fp64-arithmetic instances); the tiled kernel takes slots as TMA
+    // coordinates and has no such limit.
+    const long long stride = (long long)L * h->desc.nlat * nlon;
+    for (int s = 0; s < n; ++s) {
+      const long long dm = (long long)(steps[s].slot_m - steps[s].slot) * stride;
+      const long long dp = (long long)(steps[s].slot_p - steps[s].slot) * stride;
+      if (dm <= -(1LL << 31) || dm >= (1LL << 31) || dp <= -(1LL << 31) || dp >= (1LL << 31)) {
+        h->err = "slot_m / slot_p lie 2^31 or more elements from slot, which the direct and sub-warp row kernels "
+                 "cannot address (the tiled kernel can)";
+        return LEC_ERR_INVALID;
+      }
+    }
+  }
   const int tile_rows = d.tile_rows;
   band_rows = std::max(tile_rows, band_rows / tile_rows * tile_rows);
   // (moving boxes of one height were tried with the banded order too: 3.06 TB/s against 3.28 unbanded on the C5

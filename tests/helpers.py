@@ -223,17 +223,25 @@ def oracle_step(P, box, it, dTdt):
 FILL = -32767
 
 
-def encode(fields, spec):
-    """int16 records of float fields + the decode dicts of LecEngine.run_torch_packed."""
+def _is_torch(a):
+    return not isinstance(a, np.ndarray) and hasattr(a, "is_cuda")
+
+
+def encode(fields, spec, bounds=None):
+    """int16 records of float fields + the decode dicts of LecEngine.run_torch_packed.  ``fields``: numpy arrays, or
+    torch tensors, encoded where they live by the same float64 operations (fields too large for the host).
+    ``bounds``: per field the (min, max) of the whole series when ``fields`` hold one slice of it at a time."""
     raws, decode = [], []
-    for a, sp in zip(fields, spec):
-        a = np.asarray(a, dtype=np.float64)
-        lo, hi = float(a.min()), float(a.max())
+    for n, (a, sp) in enumerate(zip(fields, spec)):
+        dev = _is_torch(a)
+        a = a.double() if dev else np.asarray(a, dtype=np.float64)
+        lo, hi = (float(a.min()), float(a.max())) if bounds is None else (float(bounds[n][0]), float(bounds[n][1]))
         if sp["offset"]:
             scale, offset = (hi - lo) / 65000.0, 0.5 * (hi + lo)
         else:
             scale, offset = max(abs(lo), abs(hi)) / 32000.0, None
-        raw = np.round((a - (offset or 0.0)) / scale).astype(np.int16)
+        q = (a - (offset or 0.0)) / scale
+        raw = q.round().short() if dev else np.round(q).astype(np.int16)      # both round half to even
         fills = [FILL, -32768][:sp["nfill"]]
         raws.append(raw)
         decode.append(dict(scale=np.float64(scale), offset=None if offset is None else np.float64(offset),
@@ -242,16 +250,20 @@ def encode(fields, spec):
 
 
 def decode(raw, dec, dtype):
-    """The decode rule in numpy: multiply, then add, as separate float64 operations."""
-    x = raw.astype(np.float64)
+    """The decode rule in numpy (or in torch for a device tensor): multiply, then add, as separate float64
+    operations."""
+    dev = _is_torch(raw)
+    x = raw.double() if dev else raw.astype(np.float64)
     if dec["scale"] is not None:
         x = x * np.float64(dec["scale"])
     if dec["offset"] is not None:
         x = x + np.float64(dec["offset"])
     if dec["float32"]:
-        x = x.astype(np.float32).astype(np.float64)
+        x = x.float().double() if dev else x.astype(np.float32).astype(np.float64)
     for fv in dec["fills"]:
         x[raw == fv] = np.nan
+    if dev:
+        return x if np.dtype(dtype) == np.float64 else x.float()
     return x.astype(dtype)
 
 
@@ -276,6 +288,25 @@ def with_boundary(eng, n, fn):
         eng._lib.lec_set_boundary_levels(eng._h, None)
     torch.cuda.synchronize()
     return tuple(x.cpu().numpy() for x in out) + (bnd.cpu().numpy(),)
+
+
+def check_refs(out, refs, tol):
+    """Steps of one box against their oracle results (``oracle_step``): all 16 terms, 19 per-level families and 18
+    boundary pieces, series-scaled over the steps.  ``out`` = (terms, levels, flags, pieces [n][6][3][nlev]).
+    Returns the worst error."""
+    terms, levels, flags, bnd = out
+    assert not flags.any(), flags
+    assert np.isfinite(terms).all() and np.isfinite(levels).all() and np.isfinite(bnd).all()
+    errs = {name: series_err(terms[:, i], [r[0][name] for r in refs]) for i, name in enumerate(E.TERM_NAMES)}
+    errs.update({"lv:" + name: series_err(levels[:, i], np.stack([np.broadcast_to(r[1][name], levels.shape[2:])
+                                                                   for r in refs]))
+                 for i, name in enumerate(E.LEVEL_TERM_NAMES)})
+    errs.update({f"bnd:{name}.{part}": series_err(bnd[:, n, part], np.stack([r[2][n, part] for r in refs]))
+                 for n, name in enumerate(BOUNDARY_TERMS) for part in range(3)})
+    assert len(errs) == 16 + 19 + 18
+    bad = {k: v for k, v in errs.items() if not v <= tol}
+    assert not bad, bad
+    return max(errs.values())
 
 
 def same_bits(a, b):

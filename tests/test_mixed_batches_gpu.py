@@ -145,24 +145,6 @@ def _run_host(eng, coords, arith, steps):
     return t, lv, f, eng.last_boundary
 
 
-def _check_refs(out, refs, tol):
-    """Steps of one box against their oracle results: all 16 terms, 19 per-level families and 18 pieces,
-    series-scaled over the steps.  Returns the worst error."""
-    terms, levels, flags, bnd = out
-    assert not flags.any(), flags
-    assert np.isfinite(terms).all() and np.isfinite(levels).all() and np.isfinite(bnd).all()
-    errs = {name: H.series_err(terms[:, i], [r[0][name] for r in refs]) for i, name in enumerate(E.TERM_NAMES)}
-    errs.update({"lv:" + name: H.series_err(levels[:, i], np.stack([np.broadcast_to(r[1][name], levels.shape[2:])
-                                                                     for r in refs]))
-                 for i, name in enumerate(E.LEVEL_TERM_NAMES)})
-    errs.update({f"bnd:{name}.{part}": H.series_err(bnd[:, n, part], np.stack([r[2][n, part] for r in refs]))
-                 for n, name in enumerate(H.BOUNDARY_TERMS) for part in range(3)})
-    assert len(errs) == 16 + 19 + 18
-    bad = {k: v for k, v in errs.items() if not v <= tol}
-    assert not bad, bad
-    return max(errs.values())
-
-
 def _fp32_out_of_reach(box):
     """A 2-row box wider than 32 chunks: its area eddies [X]_j - [[X]] are tiny against the zonal eddies, so fp32
     arithmetic cannot reach 1e-5 of them (DESIGN.md section 5).  Measured alone on a B200: 2 rows x 801 columns
@@ -179,7 +161,7 @@ def _check_oracle(out, items, coords, arith):
             continue
         idx = [n for n, (b, _) in enumerate(items) if b == box]
         try:
-            _check_refs(tuple(x[idx] for x in out), [_oracle(coords, *items[n]) for n in idx], tol)
+            H.check_refs(tuple(x[idx] for x in out), [_oracle(coords, *items[n]) for n in idx], tol)
         except AssertionError as e:
             raise AssertionError(f"box {box}: {e}") from None
 
@@ -404,7 +386,7 @@ def test_a_band_batched_with_a_tall_box_meets_the_gate_without_compensated_sums(
         idx = [n for n, (bx, _) in enumerate(items) if bx == box]
         sub = tuple(x[idx] for x in out)
         refs = [ref[items[n]] for n in idx]
-        worst[box] = _check_refs(sub, refs, 1e-5)
+        worst[box] = H.check_refs(sub, refs, 1e-5)
     print(f"C4 band in a mixed batch: worst error {worst[C4_BAND]:.2e} (COMP {d['comp']}); "
           f"8 x 200 box {worst[C4_NARROW]:.2e}")
 

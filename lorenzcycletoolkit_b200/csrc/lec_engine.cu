@@ -19,10 +19,6 @@
 
 using namespace lec;
 
-#ifndef LEC_TILE_ROWS_DEFAULT
-#define LEC_TILE_ROWS_DEFAULT 15
-#endif
-
 struct lec_handle {
   lec_grid_desc desc{};
   int device = 0;
@@ -30,15 +26,11 @@ struct lec_handle {
   int pitch = 0;                                 // row length of the engine's own staging (lec_run_host*)
   double* d_tables = nullptr;
   float* d_tables32 = nullptr;
-  int prefetch_mode = 1 | 16;                   // bit 0: own-row L2 bulk prefetch of the direct wide kernel (+9 % measured), bit 4: per-lane
-                                                // L2 prefetch of a track-box row's later sweep iterations (+8 %); LEC_PREFETCH=0 disables both
   int use_tile = 1;                             // LEC_ROW_KERNEL=tile|direct: TMA-tiled row kernel for wide boxes
-  int tile_rows = LEC_TILE_ROWS_DEFAULT;        // rows per tile (experiment builds: LEC_TILE_ROWS=8|11|12|15)
   int num_sms = 148;
   long long h2d_bytes = 0, d2h_bytes = 0;      // PCIe traffic of the last lec_run_host
   int comp_mode = -1;                           // LEC_COMP=0|1: force the compensated fp32 linear sums off / on (-1: by box shape)
   int use_narrow = 1;                           // LEC_NARROW=0: never use the sub-warp kernel for narrow boxes
-  int tma_hint = -1;                            // LEC_TMA_HINT=0|1: evict-first hint on the once-read fields (-1: fp64 fields only)
   int force_narrow_g = 0;                       // LEC_NARROW_G=4|8|16: force the group width (measurements)
   double* d_rec = nullptr;
   double* d_fin = nullptr;             // finalize scratch [max_steps][nlev][kLevStride]
@@ -177,21 +169,19 @@ bool make_map(CUtensorMap* m, const void* base, int esize, int nlon, int nlat, i
 //   fp32 arithmetic, plain or compensated  11 rows x 7 stages  (196 KB)
 //   fp64 decode                            11 rows x 8 stages  (122 KB)
 //   fp32 decode, fp64 arithmetic            7 rows x 8 stages  (142 KB)
-// `rows` (LEC_TILE_ROWS in LEC_TILE_ALL_SHAPES experiment builds) picks among the plain fp32 shapes 8, 11, 12 and 15.
 struct RingShape { int rows, stages; };
-constexpr RingShape ring_shape(bool f64, bool m64, bool comp, bool i16, int rows) {
+constexpr RingShape ring_shape(bool f64, bool m64, bool comp, bool i16) {
   if (i16) return f64 ? RingShape{11, 8} : m64 ? RingShape{7, 8} : RingShape{11, 7};
   if (f64) return {11, 4};
   if (m64) return {7, 6};
   if (comp) return {11, 4};
-  return rows == 8 ? RingShape{8, 5} : rows == 11 || rows == 12 ? RingShape{rows, 4} : RingShape{15, 3};
+  return {15, 3};
 }
 
-template <typename FT, typename CT, int R, bool COMP, typename ST>
+template <typename FT, typename CT, bool COMP, typename ST>
 cudaError_t launch_tile_c(const TmaMaps& maps, const RowParams& rp, int lonw, int grid, cudaStream_t st) {
-  constexpr RingShape shape = ring_shape(sizeof(FT) == 8, sizeof(CT) == 8, COMP, sizeof(ST) != sizeof(FT), R);
-  static_assert(shape.rows == R, "a ring shape of the table");
-  constexpr int S = shape.stages;
+  constexpr RingShape shape = ring_shape(sizeof(FT) == 8, sizeof(CT) == 8, COMP, sizeof(ST) != sizeof(FT));
+  constexpr int R = shape.rows, S = shape.stages;
   using G = TileGeom<FT, R, S, ST>;
   cudaError_t e = cudaSuccess;
 #define LEC_TILE_LAUNCH(LW, TB, SMEM)                                                                             \
@@ -218,15 +208,7 @@ cudaError_t launch_rows_c(const lec_dispatch& d, const RowParams& rp, const TmaM
   constexpr int VEC = 16 / sizeof(FT);
   if (d.kernel == LEC_ROWS_TILED) {
     const int pgrid = (int)std::min<long long>(grid, (long long)num_sms);      // persistent: one CTA per SM
-#ifdef LEC_TILE_ALL_SHAPES
-    if constexpr (sizeof(CT) == 4 && !COMP && sizeof(ST) == sizeof(FT)) {
-      if (d.tile_rows == 8) return launch_tile_c<FT, CT, 8, COMP, ST>(maps, rp, d.lonw, pgrid, st);
-      if (d.tile_rows == 11) return launch_tile_c<FT, CT, 11, COMP, ST>(maps, rp, d.lonw, pgrid, st);
-      if (d.tile_rows == 12) return launch_tile_c<FT, CT, 12, COMP, ST>(maps, rp, d.lonw, pgrid, st);
-    }
-#endif
-    constexpr int R = ring_shape(sizeof(FT) == 8, sizeof(CT) == 8, COMP, sizeof(ST) != sizeof(FT), LEC_TILE_ROWS_DEFAULT).rows;
-    return launch_tile_c<FT, CT, R, COMP, ST>(maps, rp, d.lonw, pgrid, st);
+    return launch_tile_c<FT, CT, COMP, ST>(maps, rp, d.lonw, pgrid, st);
   }
   if (d.kernel == LEC_ROWS_SUBWARP) launch_narrow_c<FT, CT, VEC, COMP, ST>(rp, d.lonw != 0, d.group, grid, st);
   else if constexpr (sizeof(ST) != sizeof(FT)) return cudaErrorInvalidValue;     // no direct kernel reads int16 fields
@@ -427,10 +409,8 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
   h->device = desc->device;
   h->elem = desc->dtype == LEC_F64 ? 8 : 4;
   h->max_steps = desc->max_steps;
-  if (const char* e = std::getenv("LEC_PREFETCH")) h->prefetch_mode = std::atoi(e);
   if (const char* e = std::getenv("LEC_NARROW")) h->use_narrow = std::atoi(e) != 0;
   if (const char* e = std::getenv("LEC_COMP")) h->comp_mode = std::atoi(e) != 0;
-  if (const char* e = std::getenv("LEC_TMA_HINT")) h->tma_hint = std::atoi(e) != 0;
   if (const char* e = std::getenv("LEC_NARROW_G")) {
     const int gq = std::atoi(e);
     if (gq == 16 || gq == 8 || gq == 4) h->force_narrow_g = gq;
@@ -439,12 +419,6 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
     if (std::strcmp(e, "tile") == 0) h->use_tile = 1;
     else if (std::strcmp(e, "direct") == 0) h->use_tile = 0;
   }
-#ifdef LEC_TILE_ALL_SHAPES
-  if (const char* e = std::getenv("LEC_TILE_ROWS")) {      // experiment builds: other tile shapes for fp32 arithmetic
-    const int r = std::atoi(e);
-    if (r == 8 || r == 11 || r == 12 || r == 15) h->tile_rows = r;
-  }
-#endif
   h->max_ny = desc->max_box_rows ? desc->max_box_rows : nlat;
   h->lon_deg.assign(desc->lon_deg, desc->lon_deg + nlon);
   h->rlon.assign(desc->rlon, desc->rlon + nlon);
@@ -655,7 +629,7 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   d.lonw = d.kernel == LEC_ROWS_SUBWARP && lonw != 0 ? 2 : lonw;
   d.comp = comp && !math64;
   d.math64 = math64;
-  d.tile_rows = d.kernel == LEC_ROWS_TILED ? ring_shape(h->desc.dtype == LEC_F64, math64, d.comp, pk, h->tile_rows).rows
+  d.tile_rows = d.kernel == LEC_ROWS_TILED ? ring_shape(h->desc.dtype == LEC_F64, math64, d.comp, pk).rows
                 : d.kernel == LEC_ROWS_SUBWARP ? kNarrowWarps * (32 / narrow_g) : kRowsPerCta;
   d.packed = pk != nullptr;
   if (d.kernel != LEC_ROWS_TILED) {
@@ -695,9 +669,6 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   if (grid > 0x7fffffffLL) return LEC_ERR_INVALID;
   rp.grid = grid;
   if (pk) rp.pk = *pk;
-  // TMA loads of u, v, omega, Phi with an L2 evict-first hint: fp64 fields only (46.7 -> 39.0 GB of DRAM reads per
-  // 24-step launch, +3.4 %; with fp32 fields the working set of a band fits without it and the hint costs 2 %)
-  rp.prefetch_mode = h->prefetch_mode | ((h->tma_hint < 0 ? h->desc.dtype == LEC_F64 : h->tma_hint != 0) ? 8 : 0);
   d.tiles_per_band = rp.tiles_per_band; d.nbands = rp.nbands;
   h->dispatch = d;
   h->dispatched = true;

@@ -71,7 +71,6 @@ struct RowParams {
   int tiles_per_band;    // CTA row-tiles per latitude band
   FastDiv dv_tiles, dv_lev, dv_steps;   // block / tile index -> (band, step, level, row tile)
   long long slot_stride; // elements per slot = nlev*nlat*nlon
-  int prefetch_mode;     // bit 0: L2 bulk prefetch of the DRAM-sourced rows at row start
   long long grid;        // number of CTAs
   PackedDev pk;          // int16 instances only
 };
@@ -320,8 +319,8 @@ lec_row_moments_kernel(const RowParams p) {
   const int d_jm = (j > j0) ? -nlon : 0, d_jp = (j < j1) ? nlon : 0;
 
   // L2 prefetch of the rows that come from DRAM (u, v, omega, Phi of this step and T of the
-  // next time slot; T of this slot was fetched as the time neighbour one step earlier)
-  if ((p.prefetch_mode & 1) && lane < 5) {
+  // next time slot; T of this slot was fetched as the time neighbour one step earlier; +9 % measured)
+  if (lane < 5) {
     const FT* base = (lane == 0) ? Tc_row + d_p : static_cast<const FT*>(p.field[lane]) + row_c;
     prefetch_l2_range(base, (long long)i0 * sizeof(FT), (long long)(i1 + 1) * sizeof(FT));
   }

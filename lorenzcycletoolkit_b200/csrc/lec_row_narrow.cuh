@@ -92,7 +92,7 @@ lec_row_moments_narrow_kernel(const RowParams p) {
   // over all lines of a longer row measured SLOWER than no prefetch (2.05 vs 1.99 ms), straight-line 1.83 ms on the
   // C5 track; 61-column boxes 0.49 -> 0.46 ms, 301-column boxes 7.66 -> 7.50 ms.  The stride is the bytes of one
   // fp sweep iteration whatever the stored type (int16 rows: lines 1 .. G-1 of the row, two iterations each).
-  if ((p.prefetch_mode & 16) && lane >= 1) {
+  if (lane >= 1) {
     const int pc = min(i0 + lane * (G * VEC * (int)sizeof(FT) / (int)sizeof(ST)), i1);
     asm volatile("prefetch.global.L2 [%0];" ::"l"(U_row + pc));
     asm volatile("prefetch.global.L2 [%0];" ::"l"(V_row + pc));

@@ -1,6 +1,6 @@
 """Row-kernel A/B on C4-shaped data: every variant named on the command line is run on the same resident
 fields, timed with the engine's own CUDA events (isolated launches) and compared bit for bit with the first one.
-  python scripts/kernel_probe.py [nsteps] [dtype f32|f64] variant ...     variant = direct | tile:R[:band[:mode[:comp]]] (direct::::1 = direct kernel with compensation)"""
+  python scripts/kernel_probe.py [nsteps] [dtype f32|f64] variant ...     variant = direct | tile[:band[:comp]] (direct::1 = direct kernel with compensation)"""
 import os
 import sys
 
@@ -12,7 +12,7 @@ from lorenzcycletoolkit_b200 import engine as E, synthetic as S
 
 nsteps = int(sys.argv[1]) if len(sys.argv) > 1 else 24
 dt = np.float64 if (len(sys.argv) > 2 and sys.argv[2] == "f64") else np.float32
-variants = sys.argv[3:] or ["direct", "tile:11", "tile:8", "tile:12", "tile:15"]
+variants = sys.argv[3:] or ["direct", "tile"]
 g = S.era5_grid()
 f64 = lambda a: np.asarray(a, dtype=np.float64)
 fields = S.synth_fields(g, nsteps + 2, dt, "cuda:0")
@@ -24,11 +24,8 @@ ref = None
 for v in variants:
     parts = v.split(":")
     os.environ["LEC_ROW_KERNEL"] = parts[0]
-    if len(parts) > 1:
-        os.environ["LEC_TILE_ROWS"] = parts[1]
-    band = int(parts[2]) if len(parts) > 2 and parts[2] else 0
-    os.environ["LEC_PREFETCH"] = parts[3] if len(parts) > 3 and parts[3] else "17"     # tile: +2 no loads, +4 no arithmetic (timing only)
-    os.environ["LEC_COMP"] = parts[4] if len(parts) > 4 else "0"                      # compensated fp32 linear sums on / off
+    band = int(parts[1]) if len(parts) > 1 and parts[1] else 0
+    os.environ["LEC_COMP"] = parts[2] if len(parts) > 2 else "0"                      # compensated fp32 linear sums on / off
     eng = E.LecEngine(f64(g["lon"]), f64(g["lat"]), f64(g["rlons"]), f64(g["rlats"]), f64(g["coslats"]), g["level"],
                       dt, max_steps=nsteps, max_box_rows=719, band_rows=band)
     best = 1e9

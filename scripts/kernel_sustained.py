@@ -1,7 +1,7 @@
 """Sustained A/B of row-kernel variants under the power cap: every variant runs 48-step launches back to back
 for `seconds`, the variants are cycled `rounds` times in ONE process (same board, same thermal state), and the mean
 kernel time per launch is reported per visit.  bench.py's device line is this measurement for the default variant.
-  python scripts/kernel_sustained.py [seconds] [rounds] variant ...      variant = direct | tile:R"""
+  python scripts/kernel_sustained.py [seconds] [rounds] variant ...      variant = direct | tile"""
 import os
 import sys
 import time
@@ -14,7 +14,7 @@ from lorenzcycletoolkit_b200 import engine as E, synthetic as S
 
 seconds = float(sys.argv[1]) if len(sys.argv) > 1 else 3.0
 rounds = int(sys.argv[2]) if len(sys.argv) > 2 else 2
-variants = sys.argv[3:] or ["direct", "tile:15", "tile:12", "tile:111"]
+variants = sys.argv[3:] or ["direct", "tile"]
 nsteps = 48
 g = S.era5_grid()
 f64 = lambda a: np.asarray(a, dtype=np.float64)
@@ -25,10 +25,7 @@ steps["i0"], steps["i1"], steps["j0"], steps["j1"] = 0, 1439, 1, 719
 B = 5 * 37 * 719 * 1440 * 4
 engines = {}
 for v in variants:
-    parts = v.split(":")
-    os.environ["LEC_ROW_KERNEL"] = parts[0]
-    if len(parts) > 1:
-        os.environ["LEC_TILE_ROWS"] = parts[1]
+    os.environ["LEC_ROW_KERNEL"] = v
     engines[v] = E.LecEngine(f64(g["lon"]), f64(g["lat"]), f64(g["rlons"]), f64(g["rlats"]), f64(g["coslats"]), g["level"],
                              np.float32, max_steps=nsteps, max_box_rows=719)
 for r in range(rounds):

@@ -309,6 +309,33 @@ def check_refs(out, refs, tol):
     return max(errs.values())
 
 
+def staged_slots(steps, window, max_steps):
+    """The greedy chunks of ``lec_run_host*`` over a staging window of ``window`` slots, replayed: returns (T slots that
+    cross PCIe, slots of u / v / omega / Phi that cross PCIe per field, whether a chunk took T slots device to device
+    from a previous window that starts at an earlier slot).  A chunk stages T over its whole slot range, minus the
+    slots the previous chunk's window holds, and the other fields over the range of its centre slots."""
+    n, s0, chunk, prev_lo, prev_hi = len(steps), 0, 0, 0, -1
+    t_slots = c_slots = 0
+    shifted = False
+    while s0 < n:
+        lo, hi, s1 = 1 << 30, -1, s0
+        while s1 < n and s1 - s0 < max_steps:
+            sl = [int(steps[k][s1]) for k in ("slot", "slot_m", "slot_p")]
+            if max(hi, *sl) - min(lo, *sl) + 1 > window:
+                break
+            lo, hi, s1 = min(lo, *sl), max(hi, *sl), s1 + 1
+        assert s1 > s0, "a step needs more slots than the window holds"
+        t_lo = lo
+        if chunk >= 1 and prev_lo <= lo <= prev_hi:
+            t_lo = min(prev_hi, hi) + 1
+            shifted |= lo > prev_lo
+        t_slots += max(0, hi - t_lo + 1)
+        centre = steps["slot"][s0:s1]
+        c_slots += int(centre.max() - centre.min() + 1)
+        prev_lo, prev_hi, s0, chunk = lo, hi, s1, chunk + 1
+    return t_slots, c_slots, shifted
+
+
 def same_bits(a, b):
     for x, y in zip(a, b):
         assert x.shape == y.shape and np.array_equal(x.view(np.uint8), y.view(np.uint8))

@@ -141,7 +141,9 @@ def test_big_endian_interleaved_records(dtype):
 
 def test_raw_records_in_staged_chunks():
     """Several staged chunks (small windows): the two raw staging buffers and the ingest stream are reused
-    across chunks and calls; T halo slots come device-to-device from the previous chunk."""
+    across chunks and calls; T halo slots come device-to-device from the previous chunk.  Every result has the bits of
+    the one-window call, for any step order, records in any order (one serving two slots), windows that split the
+    pass mid-way, and a reused handle whose maps change; the H2D bytes are those of the slots the chunks stage."""
     rng = np.random.default_rng(15)
     P, fields = _dataset(40, 17, 6, 13, np.float32)
     steps = H.fixed_steps(P, P.lon[1], P.lon[37], P.lat[1], P.lat[15])
@@ -160,6 +162,60 @@ def test_raw_records_in_staged_chunks():
     with H.make_engine(P, np.float32, [1.0] * 5, host_stage_bytes=2 * 5 * 4 * slot_bytes) as eng:
         d = eng.run_host_raw(raws, lon_map, lat_map, lev_map, np.arange(13), steps[::-1].copy())   # steps in reverse order
         assert np.array_equal(d[0], a[0][::-1]) and np.array_equal(d[1], a[1][::-1])
+
+    def same(b, ref, idx, what):
+        for x, y in zip(ref, b):
+            assert np.array_equal(x[idx], y), what
+
+    def h2d(st, window, nk, nj):           # T at every slot that crosses PCIe, the other four at the centre slots
+        t_slots, c_slots, _ = H.staged_slots(st, window, 64)
+        return (t_slots + 4 * c_slots) * nk * nj * 40 * 4
+
+    # Step lists shuffled, reversed and with repeats, through 3-slot windows and 8-slot ones (in order, the pass splits
+    # after 7 steps and the second window starts inside the first, at a later slot: its first T slots come device to
+    # device from the other buffer)
+    lists = {"in order": np.arange(13), "shuffled": rng.permutation(13), "reversed": np.arange(13)[::-1],
+             "repeats": np.r_[np.arange(13), [5, 5, 0, 12, 6]]}
+    for w in (3, 8):
+        assert H.staged_slots(steps, w, 64)[2]
+        with H.make_engine(P, np.float32, [1.0] * 5, host_stage_bytes=2 * 5 * w * slot_bytes) as eng:
+            for name, idx in lists.items():
+                st = steps[idx].copy()
+                same(eng.run_host_raw(raws, lon_map, lat_map, lev_map, np.arange(13), st), a, idx, (w, name))
+                assert eng.last_transfer()[0] == h2d(st, w, 6, 17), (w, name)
+
+    # Records in another order, one of them serving slots 4 and 9
+    fields2 = [f.copy() for f in fields]
+    for f in fields2:
+        f[9] = f[4]
+    with H.make_engine(P, np.float32, [1.0] * 5) as eng:
+        a2 = eng.run_host(fields2, steps)
+    slot_record = np.empty(13, dtype=np.int32)
+    slot_record[np.arange(13) != 9] = rng.permutation(12)
+    slot_record[9] = slot_record[4]
+    raws2 = [np.empty((12,) + r.shape[1:], dtype=r.dtype) for r in raws]
+    keep = np.arange(13) != 9
+    for r2, r in zip(raws2, raws):
+        r2[slot_record[keep]] = r[keep]
+    with H.make_engine(P, np.float32, [1.0] * 5, host_stage_bytes=2 * 5 * 3 * slot_bytes) as eng:
+        same(eng.run_host_raw(raws2, lon_map, lat_map, lev_map, slot_record, steps), a2, slice(None), "slot_record")
+
+    # One handle, three layouts of the same fields: a wider raw level range and a row sub-range (the raw staging
+    # buffers grow; 3-D copies), then other longitude maps (the device copy of the maps is replaced)
+    def place(lon_m, lat_m, lev_m, nlev_r, nlat_r):
+        out = []
+        for f in fields:
+            r = (rng.normal(size=(13, nlev_r, nlat_r, 40)) * 1e3).astype(np.float32)
+            r[np.ix_(np.arange(13), lev_m, lat_m, lon_m)] = f
+            out.append(r)
+        return out
+    lev_b, lat_b, lon_c = np.array([7, 0, 5, 2, 3, 6]), 1 + lat_map, (np.arange(40) + 18) % 40
+    layouts = [(raws, (lon_map, lat_map, lev_map), 6), (place(lon_map, lat_b, lev_b, 9, 19), (lon_map, lat_b, lev_b), 8),
+               (place(lon_c, lat_b, lev_b, 9, 19), (lon_c, lat_b, lev_b), 8)]
+    with H.make_engine(P, np.float32, [1.0] * 5, host_stage_bytes=2 * 5 * 3 * slot_bytes) as eng:
+        for n, (raws_, maps, nk) in enumerate(layouts):
+            same(eng.run_host_raw(raws_, *maps, np.arange(13), steps), a, slice(None), f"layout {n}")
+            assert eng.last_transfer()[0] == h2d(steps, 3, nk, 17), n
 
 
 def test_raw_errors():

@@ -82,6 +82,7 @@ struct GridDev {
   const double* plev;
   const double* pa;        // np.gradient coefficients w.r.t. p incl. the one-sided ends
   const double* pc;
+  double p_2h;             // 2 h when the whole level axis is exactly uniform (np.gradient's uniform branch), else 0
   const double* sm;        // -cp sT sW S,  S = sm (T[k-1]-T) + sp (T[k+1]-T) + ss T  (stability term of Q)
   const double* sp;
   const double* ss;

@@ -85,7 +85,12 @@ const char* kVersion = "lec_b200 0.2 (sm_100a; rows=tile)";
     }                                                                              \
   } while (0)
 
-// np.gradient interior coefficients at point i of a (possibly non-uniform) axis.
+// np.gradient interior coefficients at point i of a (possibly non-uniform) axis.  The kernels apply them in
+// difference form, a (f[i-1] - f[i]) + c (f[i+1] - f[i]), which reads f[i]; numpy's branch for a wholly uniform
+// axis, (f[i+1] - f[i-1]) / 2h, never does, so a missing f[i] makes the kernels' derivative NaN where numpy's is
+// finite.  In the row kernels (d/dt, d/dlon, d/dlat, and d/dp in the stability term of Q) the derivative's
+// co-factor holds the same missing value, so the NaN cannot reach an output.  F2's d[u]/dp is the exception
+// (Ck_5 multiplies it by [w'v']): there the finalize kernel takes numpy's form on a uniform level axis (p_2h).
 inline void grad_interior(const double* x, int i, double& a, double& b, double& c) {
   const double hs = x[i] - x[i - 1], hd = x[i + 1] - x[i];
   if (hs == hd) {
@@ -494,10 +499,14 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
       tab[o_fya + j] = a; tab[o_fyc + j] = c;
     }
   }
+  double p_2h = 2.0 * (h->plev[1] - h->plev[0]);
+  for (int k = 1; k + 1 < L; ++k)
+    if (h->plev[k + 1] - h->plev[k] != h->plev[1] - h->plev[0]) p_2h = 0.0;
   {
     std::vector<double> a(L), b(L), c(L), E(L);
     lec_gradient_coefs(h->plev.data(), L, a.data(), b.data(), c.data());
-    // per-point non-uniform rule in the interior (identical to numpy's uniform branch where hs == hd)
+    // per-point non-uniform rule in the interior (identical to numpy's uniform branch where hs == hd, but for
+    // the centre read: see grad_interior)
     for (int k = 1; k + 1 < L; ++k) grad_interior(h->plev.data(), k, a[k], b[k], c[k]);
     for (int k = 0; k < L; ++k) E[k] = std::pow(h->plev[k] / kP0, kKappa);   // T / theta
     for (int k = 0; k < L; ++k) {
@@ -516,7 +525,7 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
   g.rlat = h->d_tables + o_rlat; g.coslat = h->d_tables + o_cos; g.tanlat = h->d_tables + o_tan;
   g.cya = h->d_tables + o_cya; g.cyc = h->d_tables + o_cyc; g.fya = h->d_tables + o_fya; g.fyc = h->d_tables + o_fyc;
   g.fxj = h->d_tables + o_fxj;
-  g.plev = h->d_tables + o_p; g.pa = h->d_tables + o_pa; g.pc = h->d_tables + o_pc;
+  g.plev = h->d_tables + o_p; g.pa = h->d_tables + o_pa; g.pc = h->d_tables + o_pc; g.p_2h = p_2h;
   g.sm = h->d_tables + o_sm; g.sp = h->d_tables + o_sp; g.ss = h->d_tables + o_ss;
   g.lon_uniform = uni; g.stencil_uniform = uni_st;
   g.wl_u = m_wl; g.cxa_u = m_a; g.cxc_u = m_c;

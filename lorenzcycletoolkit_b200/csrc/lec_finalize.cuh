@@ -212,7 +212,10 @@ lec_fin_sums_kernel(const FinParams p) {
       rec_means<2>(rkm, ix, sc, km2);
       rec_means<2>(rkp, ix, sc, kp2);
       const double dp_TAE = pa * ((km2[0] - T_AAm) - T_AE) + pc * ((kp2[0] - T_AAp) - T_AE);
-      const double dp_u = pa * (km2[1] - q.um) + pc * (kp2[1] - q.um);
+      // d[u]/dp as np.gradient takes it: on an exactly uniform level axis the centred difference never reads
+      // [u] of level k, so Ck_5 (whose co-factor [w'v'] does not hold u) stays finite when u is missing at k
+      const double dp_u = (p.g.p_2h != 0.0 && k > 0 && k < L - 1) ? (kp2[1] - km2[1]) / p.g.p_2h
+                                                                 : pa * (km2[1] - q.um) + pc * (kp2[1] - q.um);
 
       const double uu_raw = q.uu + q.um * q.um, vv_raw = q.vv + q.vm * q.vm;   // ZA(u^2), ZA(v^2)
       const double uv_raw = q.uv + q.um * q.vm;

@@ -382,14 +382,19 @@ def CalcAreaAverage(f, rlats, coslats, rlons=None, xlength=None):
 # --------------------------------------------------------------------------- #
 def StaticStability(T, p, rlats, coslats, rlons, xlength, ylength):
     """thermodynamics.py:26-73.  ``p`` broadcastable along the level axis."""
+    sigma_AA = static_stability_prefloor(T, p, rlats, coslats, rlons, xlength, ylength)
+    return np.where(sigma_AA > 0.03, sigma_AA, 0.03)
+
+
+def static_stability_prefloor(T, p, rlats, coslats, rlons, xlength, ylength):
+    """:func:`StaticStability` before its floor: the value the floor tests (NaN where a level is missing)."""
     pk = p.reshape((-1, 1, 1))
     FirstTerm = g * T / Cp_d
     SecondTerm = pk * g / Rd
     ThirdTerm = differentiate(T, p, -3)
     function = FirstTerm - (SecondTerm * ThirdTerm)
     sigma_ZA = trapz(function, rlons, -1) / xlength
-    sigma_AA = trapz(sigma_ZA * coslats, rlats, -1) / ylength
-    return np.where(sigma_AA > 0.03, sigma_AA, 0.03)
+    return trapz(sigma_ZA * coslats, rlats, -1) / ylength
 
 
 def AdiabaticHeating(T, p, omega, u, v, lat_deg, lon_deg, coslats, dTdt):
@@ -461,8 +466,10 @@ class BoxState:
         self.Q = AdiabaticHeating(self.tair, self.p, self.omega, self.u, self.v,
                                   self.lat, self.lon, self.coslats, dTdt_box)
         self._means("Q")
-        self.sigma_AA = StaticStability(self.tair, self.p, self.rlats, self.coslats,
-                                        self.rlons, self.xlength, self.ylength)
+        # sigma_prefloor: what the 0.03 floor tests, so a caller can predict when the floor applies
+        self.sigma_prefloor = static_stability_prefloor(self.tair, self.p, self.rlats, self.coslats,
+                                                        self.rlons, self.xlength, self.ylength)
+        self.sigma_AA = np.where(self.sigma_prefloor > 0.03, self.sigma_prefloor, 0.03)
 
     def _means(self, n):
         f = getattr(self, n)
@@ -492,63 +499,78 @@ def _integrate_levels(function, levels):
     return function, trapz(function, levels, -1)
 
 
-def energy_contents(b, lv):
-    """energy_contents.py:99-165."""
+class _Families:
+    """Records the per-level families of one term function: ``lv`` receives them as the reference saves them (after
+    ``_handle_nans`` for the integrated ones), ``raw`` (optional) as they were computed, before ``_handle_nans``."""
+
+    def __init__(self, lv, raw):
+        self.lv, self.raw = lv, raw
+
+    def keep(self, name, f):                # a family that is saved but not integrated
+        self.lv[name] = f
+        if self.raw is not None:
+            self.raw[name] = f
+        return f
+
+    def integrate(self, name, f, levels):   # returns the trapezoid over the kept levels
+        if self.raw is not None:
+            self.raw[name] = f
+        self.lv[name], I = _integrate_levels(f, levels)
+        return I
+
+
+def energy_contents(b, lv, raw=None):
+    """energy_contents.py:99-165.  ``raw``: optional dict of the per-level families before ``_handle_nans``."""
     s = b.sigma_AA
+    F = _Families(lv, raw)
     out = {}
-    f, out["Az"] = _integrate_levels(b.AAz(b.tair_AE ** 2) / (2 * s), b.p); lv["Az"] = f
-    f, out["Ae"] = _integrate_levels(b.AA(b.tair_ZE ** 2) / (2 * s), b.p); lv["Ae"] = f
-    f, I = _integrate_levels(b.AAz(b.u_ZA ** 2 + b.v_ZA ** 2), b.p); lv["Kz"] = f
-    out["Kz"] = I / (2 * g)
-    f, I = _integrate_levels(b.AA(b.u_ZE ** 2 + b.v_ZE ** 2), b.p); lv["Ke"] = f
-    out["Ke"] = I / (2 * g)
+    out["Az"] = F.integrate("Az", b.AAz(b.tair_AE ** 2) / (2 * s), b.p)
+    out["Ae"] = F.integrate("Ae", b.AA(b.tair_ZE ** 2) / (2 * s), b.p)
+    out["Kz"] = F.integrate("Kz", b.AAz(b.u_ZA ** 2 + b.v_ZA ** 2), b.p) / (2 * g)
+    out["Ke"] = F.integrate("Ke", b.AA(b.u_ZE ** 2 + b.v_ZE ** 2), b.p) / (2 * g)
     return out
 
 
-def conversion_terms(b, lv):
-    """conversion_terms.py:103-245 (order of the calls as in the frameworks)."""
+def conversion_terms(b, lv, raw=None):
+    """conversion_terms.py:103-245 (order of the calls as in the frameworks).  ``raw``: as in
+    :func:`energy_contents`."""
     s = b.sigma_AA
     p = b.p
+    F = _Families(lv, raw)
     out = {}
     # calc_cz :168-192
-    term1 = Rd / (p * g)
-    lv["Cz_1"] = term1
-    term2 = b.AAz(b.omega_AE * b.tair_AE)
-    lv["Cz_2"] = term2
-    lv["Cz"], out["Cz"] = _integrate_levels(-(term1 * term2), p)
+    term1 = F.keep("Cz_1", Rd / (p * g))
+    term2 = F.keep("Cz_2", b.AAz(b.omega_AE * b.tair_AE))
+    out["Cz"] = F.integrate("Cz", -(term1 * term2), p)
     # calc_ca :103-140
     DelPhi_tairAE = differentiate(b.tair_AE * b.coslats, b.rlats, -1)
     t1 = (b.v_ZE * b.tair_ZE * DelPhi_tairAE[..., None]) / (2 * Re * s)[..., None, None]
-    t1 = b.AA(t1)
-    lv["Ca_1"] = t1
+    t1 = F.keep("Ca_1", b.AA(t1))
     DelPres_tairAE = differentiate(b.tair_AE, p, -2)
     t2 = (b.omega_ZE * b.tair_ZE) * DelPres_tairAE[..., None]
-    t2 = b.AA(t2) / s
-    lv["Ca_2"] = t2
-    lv["Ca"], out["Ca"] = _integrate_levels(-(t1 + t2), p)
+    t2 = F.keep("Ca_2", b.AA(t2) / s)
+    out["Ca"] = F.integrate("Ca", -(t1 + t2), p)
     # calc_ck :194-245
     tan_lats = np.tan(b.rlats)
     DelPhi_uZA_cosphi = differentiate(b.u_ZA / b.coslats, b.rlats, -1)
     k1 = (b.coslats[:, None] * b.u_ZE * b.v_ZE / Re) * DelPhi_uZA_cosphi[..., None]
-    k1 = b.AA(k1); lv["Ck_1"] = k1
+    k1 = F.keep("Ck_1", b.AA(k1))
     DelPhi_vZA = differentiate(b.v_ZA, b.rlats, -1)
     k2 = ((b.v_ZE ** 2) / Re) * DelPhi_vZA[..., None]
-    k2 = b.AA(k2); lv["Ck_2"] = k2
+    k2 = F.keep("Ck_2", b.AA(k2))
     k3 = (tan_lats[:, None] * (b.u_ZE ** 2) * b.v_ZA[..., None]) / Re
-    k3 = b.AA(k3); lv["Ck_3"] = k3
+    k3 = F.keep("Ck_3", b.AA(k3))
     DelPres_uZAp = differentiate(b.u_ZA, p, -2)
     k4 = b.omega_ZE * b.u_ZE * DelPres_uZAp[..., None]
-    k4 = b.AA(k4); lv["Ck_4"] = k4
+    k4 = F.keep("Ck_4", b.AA(k4))
     DelPres_vZAp = differentiate(b.u_ZA, p, -2)            # sic: u_ZA (:225-229)
     k5 = b.omega_ZE * b.v_ZE * DelPres_vZAp[..., None]
-    k5 = b.AA(k5); lv["Ck_5"] = k5
-    f, I = _integrate_levels(k1 + k2 + k3 + k4 + k5, p); lv["Ck"] = f
-    out["Ck"] = I / g
+    k5 = F.keep("Ck_5", b.AA(k5))
+    out["Ck"] = F.integrate("Ck", k1 + k2 + k3 + k4 + k5, p) / g
     # calc_ce :142-166
-    lv["Ce_1"] = term1
-    e2 = b.AA(b.omega_ZE * b.tair_ZE)
-    lv["Ce_2"] = e2
-    lv["Ce"], out["Ce"] = _integrate_levels(-(term1 * e2), p)
+    F.keep("Ce_1", term1)
+    e2 = F.keep("Ce_2", b.AA(b.omega_ZE * b.tair_ZE))
+    out["Ce"] = F.integrate("Ce", -(term1 * e2), p)
     return out
 
 
@@ -654,12 +676,13 @@ def boundary_terms(b, legacy_0d=False, pieces=None):
     return out
 
 
-def generation_terms(b, lv):
-    """generation_and_dissipation_terms.py:122-152 (Gz, Ge)."""
+def generation_terms(b, lv, raw=None):
+    """generation_and_dissipation_terms.py:122-152 (Gz, Ge).  ``raw``: as in :func:`energy_contents`."""
     s = b.sigma_AA
+    F = _Families(lv, raw)
     out = {}
-    lv["Gz"], out["Gz"] = _integrate_levels(b.AAz(b.Q_AE * b.tair_AE) / (Cp_d * s), b.p)
-    lv["Ge"], out["Ge"] = _integrate_levels(b.AA(b.Q_ZE * b.tair_ZE) / (Cp_d * s), b.p)
+    out["Gz"] = F.integrate("Gz", b.AAz(b.Q_AE * b.tair_AE) / (Cp_d * s), b.p)
+    out["Ge"] = F.integrate("Ge", b.AA(b.Q_ZE * b.tair_ZE) / (Cp_d * s), b.p)
     return out
 
 

@@ -205,17 +205,20 @@ def oracle_step(P, box, it, dTdt):
     """One step evaluated as ``O.lec_moving`` does (a ``BoxState`` of time ``it`` on the box of grid indices
     ``box = (i0, i1, j0, j1)``, ``dTdt`` the global ``np.gradient`` dT/dt), for a ``P`` already in the arithmetic
     of the comparison (``O.to_mode(P, "fp64")``).  Returns (16 terms by name, per-level families by name,
-    boundary pieces ``[6][3][nlev]``)."""
+    boundary pieces ``[6][3][nlev]``, raw): ``raw`` holds the same 19 families as computed, before the reference's
+    ``_handle_nans`` (they differ only where a family has a missing level), and under ``"sigma"`` the static
+    stability before its 0.03 floor."""
     i0, i1, j0, j1 = box
     b = O.BoxState(P, P.lon[i0], P.lon[i1], P.lat[j0], P.lat[j1], fixed=False, dTdt=dTdt[it], tsel=it)
     assert b.idx == tuple(box), (b.idx, box)
-    lv, terms, pieces = {}, {}, {}
-    terms.update(O.energy_contents(b, lv))
-    terms.update(O.conversion_terms(b, lv))
+    lv, raw, terms, pieces = {}, {}, {}, {}
+    terms.update(O.energy_contents(b, lv, raw))
+    terms.update(O.conversion_terms(b, lv, raw))
     terms.update(O.boundary_terms(b, pieces=pieces))
-    terms.update(O.generation_terms(b, lv))
-    return ({k: float(v) for k, v in terms.items()}, {k: np.asarray(v, dtype=np.float64) for k, v in lv.items()},
-            boundary_pieces(pieces))
+    terms.update(O.generation_terms(b, lv, raw))
+    f64 = lambda d: {k: np.asarray(v, dtype=np.float64) for k, v in d.items()}
+    return ({k: float(v) for k, v in terms.items()}, f64(lv), boundary_pieces(pieces),
+            dict(f64(raw), sigma=np.asarray(b.sigma_prefloor, dtype=np.float64)))
 
 
 # --------------------------------------------------------------------------------------- #

@@ -297,6 +297,22 @@ int build_step(const lec_handle* h, const lec_step& s, int nslots, StepDev& d) {
   return LEC_OK;
 }
 
+// The decode a lec_raw_desc or lec_packed_desc states (members of the same names), checked once for both entry points,
+// as IngestParams' decode members; what a field does not use is folded as PackedDev folds it (fills: kNoFill).
+template <typename Desc>
+int read_decode(lec_handle* h, const Desc& d, bool i16, IngestParams (&dec)[5]) {
+  for (int f = 0; f < 5; ++f) {
+    IngestParams& e = dec[f];
+    if (d.nfill[f] < 0 || d.nfill[f] > 2) { h->err = "at most two fill values per field"; return LEC_ERR_INVALID; }
+    for (int n = 0; n < d.nfill[f]; ++n)
+      if (const double v = d.fill[f][n]; i16 && !(v >= -32768.0 && v <= 32767.0 && v == std::floor(v))) { h->err = "a fill value is not an int16 value"; return LEC_ERR_INVALID; }
+    e.nfill = d.nfill[f]; e.fill0 = e.nfill > 0 ? d.fill[f][0] : kNoFill; e.fill1 = e.nfill > 1 ? d.fill[f][1] : kNoFill;
+    e.use_scale = i16 && d.use_scale[f]; e.use_offset = i16 && d.use_offset[f]; e.round32 = i16 && d.round_f32[f];
+    e.scale = e.use_scale ? d.scale[f] : 1.0; e.offset = e.use_offset ? d.offset[f] : -0.0;
+  }
+  return LEC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -759,6 +775,8 @@ int lec_run_device_packed(lec_handle* h, const lec_packed_desc* pd, const int16_
     h->err = "pitch must be at least nlon and a multiple of 8 elements (16-byte rows)";
     return LEC_ERR_INVALID;
   }
+  IngestParams dec[5];
+  if (const int rc = read_decode(h, *pd, true, dec)) return rc;
   PackedDev pk{};
   const void* ptrs[5];
   for (int f = 0; f < 5; ++f) {
@@ -766,17 +784,8 @@ int lec_run_device_packed(lec_handle* h, const lec_packed_desc* pd, const int16_
       h->err = "int16 fields must be 16-byte aligned device pointers";
       return LEC_ERR_INVALID;
     }
-    if (pd->nfill[f] < 0 || pd->nfill[f] > 2) { h->err = "at most two fill values per field"; return LEC_ERR_INVALID; }
-    int fill[2] = {kNoFill, kNoFill};
-    for (int n = 0; n < pd->nfill[f]; ++n) {
-      const double v = pd->fill[f][n];
-      if (!(v >= -32768.0 && v <= 32767.0 && v == std::floor(v))) { h->err = "a fill value is not an int16 value"; return LEC_ERR_INVALID; }
-      fill[n] = (int)v;
-    }
-    pk.fill0[f] = fill[0]; pk.fill1[f] = fill[1];
-    pk.scale[f] = pd->use_scale[f] ? pd->scale[f] : 1.0;
-    pk.offset[f] = pd->use_offset[f] ? pd->offset[f] : -0.0;
-    pk.round32[f] = pd->round_f32[f] != 0;
+    pk.scale[f] = dec[f].scale; pk.offset[f] = dec[f].offset; pk.round32[f] = dec[f].round32;
+    pk.fill0[f] = (int)dec[f].fill0; pk.fill1[f] = (int)dec[f].fill1;
     ptrs[f] = fields[f];
   }
   pk.ntab = (h->desc.nlon + 3) & ~3;
@@ -787,6 +796,7 @@ int lec_run_device_packed(lec_handle* h, const lec_packed_desc* pd, const int16_
 struct HostSource {
   const void* const* fields = nullptr;
   const lec_raw_desc* raw = nullptr;
+  IngestParams dec[5] = {};                            // read_decode of raw; none for engine-layout arrays
   const int32_t* slot_record = nullptr;
   int nrecords = 0;
   int jr_lo = 0, jr_hi = 0, kr_lo = 0, kr_hi = 0;     // raw rows / levels the maps touch
@@ -807,13 +817,10 @@ static int stage_field(lec_handle* h, const HostSource& src, int f, int b, int w
   const size_t relem = r.dtype == LEC_RAW_I16 ? 2 : r.dtype == LEC_RAW_F32 ? 4 : 8;
   const int nj = src.jr_hi - src.jr_lo + 1, nk = src.kr_hi - src.kr_lo + 1;
   const size_t row_bytes = (size_t)r.nlon * relem, rec_bytes = row_bytes * r.nlat * r.nlev;
-  IngestParams ip{};
+  IngestParams ip = src.dec[f];
   ip.lon_map = h->d_maps; ip.lat_map = h->d_maps + h->desc.nlon; ip.lev_map = ip.lat_map + h->desc.nlat;
   ip.nlon = h->desc.nlon; ip.nlat = h->desc.nlat; ip.nlev = h->desc.nlev; ip.pitch = h->pitch;
   ip.rlon = r.nlon; ip.nj_raw = nj; ip.jr_lo = src.jr_lo; ip.kr_lo = src.kr_lo;
-  ip.scale = r.scale[f]; ip.offset = r.offset[f]; ip.fill0 = r.fill[f][0]; ip.fill1 = r.fill[f][1];
-  ip.use_scale = r.dtype == LEC_RAW_I16 && r.use_scale[f]; ip.use_offset = r.dtype == LEC_RAW_I16 && r.use_offset[f];
-  ip.round32 = r.dtype == LEC_RAW_I16 && r.round_f32[f]; ip.nfill = r.nfill[f];
   ip.big_endian = r.big_endian != 0;
   const size_t rec_stride = r.record_stride[f] > 0 ? (size_t)r.record_stride[f] : rec_bytes;
   const dim3 grid((h->desc.nlon + 4 * kIngestThreads - 1) / (4 * kIngestThreads), h->desc.nlat, h->desc.nlev);
@@ -1054,13 +1061,14 @@ int lec_run_host_raw(lec_handle* h, const lec_raw_desc* rd, const void* const ra
   if (!h || !rd || !raw || !slot_record || !steps || nsteps < 0 || nslots < 1 || nrecords < 1 || !out_terms ||
       !rd->lon_map || !rd->lat_map || !rd->lev_map || rd->nlon < 1 || rd->nlat < 1 || rd->nlev < 1)
     return LEC_ERR_INVALID;
-  for (int f = 0; f < 5; ++f) if (!raw[f] || rd->nfill[f] < 0 || rd->nfill[f] > 2 || rd->record_stride[f] < 0) return LEC_ERR_INVALID;
+  for (int f = 0; f < 5; ++f) if (!raw[f] || rd->record_stride[f] < 0) return LEC_ERR_INVALID;
   if (rd->dtype != LEC_RAW_F32 && rd->dtype != LEC_RAW_F64 && rd->dtype != LEC_RAW_I16) return LEC_ERR_INVALID;
   if ((rd->dtype == LEC_RAW_F32 && h->desc.dtype != LEC_F32) || (rd->dtype == LEC_RAW_F64 && h->desc.dtype != LEC_F64)) {
     h->err = "raw float records need a handle of the same float type";
     return LEC_ERR_INVALID;
   }
   HostSource src;
+  if (const int rc = read_decode(h, *rd, rd->dtype == LEC_RAW_I16, src.dec)) return rc;
   src.fields = raw; src.raw = rd; src.slot_record = slot_record; src.nrecords = nrecords;
   auto range = [](const int32_t* m, int n, int limit, int& lo, int& hi) {
     lo = 1 << 30; hi = -1;

@@ -304,10 +304,10 @@ def pin_arrays(arrays, limit_bytes=None):
     return True
 
 
-def _set_decode(d, decode, strict=False):
+def _set_decode(d, decode):
     """Fill the decode fields (scale, offset, use_*, round_f32, nfill, fill) that ``lec_raw_desc`` and
-    ``lec_packed_desc`` share from per-field dicts ``scale``, ``offset``, ``fills``, ``float32``.  ``strict``: more than
-    two fill values, or one that is not an int16 value, is an error (otherwise the first two are used)."""
+    ``lec_packed_desc`` share from per-field dicts ``scale``, ``offset``, ``fills``, ``float32``.  ``nfill`` is the
+    number of fill values given, so the library rejects more than two."""
     for f, dec in enumerate(decode or [{}] * 5):
         d.scale[f] = float(dec.get("scale", 1.0) if dec.get("scale") is not None else 1.0)
         d.offset[f] = float(dec.get("offset", 0.0) if dec.get("offset") is not None else 0.0)
@@ -315,13 +315,8 @@ def _set_decode(d, decode, strict=False):
         d.use_offset[f] = int(dec.get("offset") is not None)
         d.round_f32[f] = int(bool(dec.get("float32", False)))
         fills = list(dec.get("fills", ()))
-        if strict and (len(fills) > 2 or any(not (float(v) == int(v) and -32768 <= int(v) <= 32767)
-                                             for v in fills if np.isfinite(float(v)))
-                       or not all(np.isfinite(float(v)) for v in fills)):
-            raise ValueError(f"field {f}: int16 decoding takes at most two fill values, each an int16 value (got {fills})")
-        fills = fills[:2]
         d.nfill[f] = len(fills)
-        for n, fv in enumerate(fills):
+        for n, fv in enumerate(fills[:2]):
             d.fill[f][n] = float(fv)
 
 
@@ -558,7 +553,7 @@ class LecEngine:
         ``decode`` = per field a dict as in :meth:`run_host_raw`; asynchronous on ``stream``."""
         d = _PackedDesc()
         d.pitch = int(pitch)
-        _set_decode(d, decode, strict=True)
+        _set_decode(d, decode)
         steps, sp = self._steps_arg(steps)
         ptrs = (C.c_void_p * 5)(*[int(p) for p in field_ptrs])
         rc = self._lib.lec_run_device_packed(self._h, C.byref(d), ptrs, int(nslots), sp, steps.size,
@@ -601,7 +596,7 @@ class LecEngine:
             flags = torch.zeros(n, dtype=torch.int32, device=dev)
         if load_torch_extension():
             d = _PackedDesc()
-            _set_decode(d, decode, strict=True)
+            _set_decode(d, decode)
             st, _ = self._steps_arg(steps)
             raw = np.frombuffer(bytes(d), dtype=np.uint8).copy()
             rc = torch.ops.lec_b200.run_device_packed(int(self._h.value), list(fields), torch.from_numpy(raw),

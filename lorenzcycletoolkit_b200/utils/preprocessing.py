@@ -47,25 +47,86 @@ class RawStore:
         return RawStore(self.fields, self.decode, **maps)
 
     def dtype_of(self, var):
-        raw = self.fields[var]
-        if raw.dtype.kind == "i":
-            return np.dtype(np.float32 if self.decode[var].get("float32") else np.float64)
-        return raw.dtype.newbyteorder("=")
+        return decoded_dtype(self.fields[var].dtype, self.decode[var])
 
     def materialise(self, var, level=None):
         """The array the eager pipeline would hold for ``var`` (one dataset level if ``level`` is given)."""
-        raw, dec = self.fields[var], self.decode[var]
         lev = self.lev if level is None else self.lev[level:level + 1]
-        sub = raw[np.ix_(self.rec, lev, self.lat, self.lon)]
-        out = sub.astype(self.dtype_of(var))
-        for fv in dec.get("fills", ()):
-            out[sub == fv] = np.nan
-        if raw.dtype.kind == "i":
-            if dec.get("scale") is not None:
-                out *= dec["scale"]
-            if dec.get("offset") is not None:
-                out += dec["offset"]
+        out = apply_decode(self.fields[var][np.ix_(self.rec, lev, self.lat, self.lon)], self.decode[var])
         return out if level is None else out[:, 0]
+
+
+def decode_rule(stored_dtype, attrs):
+    """The CF decode of a variable stored as ``stored_dtype`` with attributes ``attrs`` (what ``xr.open_dataset``
+    applies, preprocessing.py:35-147): ``dict(scale=, offset=, fills=[...], float32=)`` as :class:`RawStore` and
+    ``LecEngine.run_host_raw`` take it, or None for a variable that is not decoded (a plain integer or a
+    non-numeric one).  Integers with a ``scale_factor`` and/or ``add_offset`` are unpacked, to float32 when the
+    stored type has at most 2 bytes and there is no offset, else to float64; stored floats are only masked.
+    ``_FillValue`` / ``missing_value`` entries are kept as values of the stored type, and only those the type holds
+    exactly: no stored value equals one it cannot hold (the device compares in the stored type too)."""
+    dt = np.dtype(stored_dtype).newbyteorder("=")
+    scale, offset = attrs.get("scale_factor"), attrs.get("add_offset")
+    if dt.kind not in "iuf" or (dt.kind != "f" and scale is None and offset is None):
+        return None
+    if dt.kind == "f":
+        scale = offset = None
+    fills = []
+    with np.errstate(invalid="ignore", over="ignore"):
+        for fv in (x for k in ("_FillValue", "missing_value") if k in attrs for x in np.atleast_1d(attrs[k]).ravel()):
+            held = fv.astype(dt)
+            if held == fv:
+                fills.append(held)
+    return dict(scale=None if scale is None else np.float64(scale), offset=None if offset is None else np.float64(offset),
+                fills=fills, float32=dt.kind != "f" and dt.itemsize <= 2 and offset is None)
+
+
+def decoded_dtype(stored_dtype, rule):
+    """The dtype :func:`apply_decode` gives a variable stored as ``stored_dtype`` under ``rule``."""
+    if rule is None or stored_dtype.kind == "f":
+        return stored_dtype.newbyteorder("=")
+    return np.dtype(np.float32 if rule["float32"] else np.float64)
+
+
+def apply_decode(raw, rule):
+    """``raw`` decoded by ``rule`` (:func:`decode_rule`) on the host, a new native-endian array: fill values to NaN,
+    then an in-place multiply by the scale and an in-place add of the offset in the decoded dtype -- xarray's
+    operations, which ``lec_ingest_kernel`` reproduces bit for bit."""
+    out = raw.astype(decoded_dtype(raw.dtype, rule))
+    if rule is not None:
+        for fv in rule["fills"]:
+            out[raw == fv] = np.nan
+        if rule["scale"] is not None:
+            out *= rule["scale"]
+        if rule["offset"] is not None:
+            out += rule["offset"]
+    return out
+
+
+def raw_store(fields, order):
+    """A :class:`RawStore` over ``fields`` = ``{var: (array as stored, dims, decode_rule)}``, or None when the
+    device cannot decode them and the host path has to: every field stored in ``order`` (the engine's dimension
+    order), one shape and one dtype for all, that dtype int16 / float32 / float64 in either byte order, at most two
+    fill values, integers packed (a scale or an offset) and floats not."""
+    arrays = [a for a, _, _ in fields.values()]
+    first = arrays[0]
+    if not all(dims == order and rule is not None and len(rule["fills"]) <= 2 and a.dtype == first.dtype and
+               a.shape == first.shape and (a.dtype.kind == "i") == (rule["scale"] is not None or rule["offset"] is not None)
+               for a, dims, rule in fields.values()):
+        return None
+    if first.dtype.newbyteorder("=") not in (np.dtype(np.int16), np.dtype(np.float32), np.dtype(np.float64)):
+        return None
+    nrec, nlev, nlat, nlon = first.shape
+    return RawStore({v: a for v, (a, _, _) in fields.items()}, {v: rule for v, (_, _, rule) in fields.items()},
+                    np.arange(nrec), np.arange(nlev), np.arange(nlat), np.arange(nlon))
+
+
+def _engine_order(var, data, dims, order, surface=False):
+    """``data`` with dimensions ``dims`` transposed to ``order``; with ``surface``, a field without a level dimension
+    goes to (time, lat, lon)."""
+    want = (order[0], order[2], order[3]) if surface and len(dims) == 3 else order
+    if sorted(dims) != sorted(want):
+        raise ValueError(f"{var} has dimensions {dims}, expected a permutation of {want}")
+    return np.transpose(data, [dims.index(d) for d in want])
 
 
 def packed_device_fields(store: RawStore, names, device="cuda"):
@@ -262,61 +323,32 @@ def open_netcdf3(path, variable_list_df, lazy=None):
             raise KeyError(f"variables {missing} named by the namelist are not in {path} "
                            f"(file has {sorted(f.variables)})")
 
-        def decode(name):
+        def read(name):          # (data as stored, big-endian, dims, attributes, decode rule)
             v = f.variables[name]
-            data = np.array(v.data)
-            if data.dtype.byteorder == ">":
-                data = data.astype(data.dtype.newbyteorder("="))
-            at = {a: getattr(v, a) for a in v._attributes}
-            at = {k: (x.decode() if isinstance(x, bytes) else x) for k, x in at.items()}
-            fills = [at[k] for k in ("_FillValue", "missing_value") if k in at]
-            scale, offset = at.get("scale_factor"), at.get("add_offset")
-            if data.dtype.kind in "iu" and (scale is not None or offset is not None):
-                raw = data
-                data = raw.astype(np.float32 if (raw.dtype.itemsize <= 2 and offset is None) else np.float64)
-                for fv in fills:
-                    data[raw == fv] = np.nan
-                if scale is not None:
-                    data *= scale
-                if offset is not None:
-                    data += offset
-            elif data.dtype.kind == "f":
-                for fv in fills:
-                    data[data == fv] = np.nan
-            return data, at, tuple(v.dimensions)
+            at = {a: (x.decode() if isinstance(x, bytes) else x) for a, x in ((a, getattr(v, a)) for a in v._attributes)}
+            return v.data, tuple(v.dimensions), at, decode_rule(v.data.dtype, at)
 
-        t, t_at, _ = decode(names["Time"])
+        def decode(name):
+            data, _, at, rule = read(name)
+            return apply_decode(data, rule), at
+
+        t, t_at = decode(names["Time"])
         units = t_at.get("units", "")
         ds.time = _decode_cf_time(t, units, t_at.get("calendar")) if " since " in str(units) else t
-        ds.level, lev_at, _ = decode(names["Vertical Level"])
-        ds.lat, _, _ = decode(names["Latitude"])
-        ds.lon, _, _ = decode(names["Longitude"])
-        ds.attrs[names["Vertical Level"]] = lev_at
+        ds.level, ds.attrs[names["Vertical Level"]] = decode(names["Vertical Level"])
+        ds.lat, ds.lon = decode(names["Latitude"])[0], decode(names["Longitude"])[0]
         order = (names["Time"], names["Vertical Level"], names["Latitude"], names["Longitude"])
-        if lazy:
-            store = _raw_store(f, wanted, order)
-            if store is not None:
-                ds.raw, ds.variables = store, _LazyVariables(store)
-                for var in wanted:
-                    v = f.variables[var]
-                    ds.attrs[var] = {a: (x.decode() if isinstance(x, bytes) else x)
-                                     for a, x in ((a, getattr(v, a)) for a in v._attributes)}
-                return ds
-        for var in wanted:
-            data, at, dims = decode(var)
-            if sorted(dims) != sorted(order):
-                raise ValueError(f"{var} has dimensions {dims}, expected a permutation of {order}")
-            ds.variables[var] = np.transpose(data, [dims.index(d) for d in order])
-            ds.attrs[var] = at
-        for var in extra:                    # (time, level, lat, lon) or a surface field (time, lat, lon)
+        fields = {var: read(var) for var in wanted}
+        store = raw_store({var: (a, dims, rule) for var, (a, dims, _, rule) in fields.items()}, order) if lazy else None
+        if store is not None:
+            ds.raw, ds.variables = store, _LazyVariables(store)
+            ds.attrs.update({var: at for var, (_, _, at, _) in fields.items()})
+            return ds
+        for var in wanted + extra:           # extra rows: (time, level, lat, lon) or a surface field (time, lat, lon)
             if var not in f.variables:
                 raise KeyError(f"variable {var} named by the namelist is not in {path}")
-            data, at, dims = decode(var)
-            want = order if len(dims) == 4 else (order[0], order[2], order[3])
-            if sorted(dims) != sorted(want):
-                raise ValueError(f"{var} has dimensions {dims}, expected a permutation of {want}")
-            ds.variables[var] = np.transpose(data, [dims.index(d) for d in want])
-            ds.attrs[var] = at
+            data, dims, ds.attrs[var], rule = fields[var] if var in fields else read(var)
+            ds.variables[var] = _engine_order(var, apply_decode(data, rule), dims, order, surface=var in extra)
     return ds
 
 
@@ -331,7 +363,8 @@ def open_netcdf4(path, variable_list_df, lazy=None):
     """NetCDF-4 (HDF5) input -- what current CDS ERA5 downloads are, ``xr.open_dataset`` in the reference
     (preprocessing.py:74) -- through ``netCDF4`` or ``h5py`` when one of them is importable (neither ships with
     this image; both are optional).  Variables are read AS STORED (no mask-and-scale), so int16-packed fields
-    stay raw-backed and are decoded on the GPU like NetCDF-3 records (:func:`from_xarray` does the rest)."""
+    stay raw-backed and are decoded on the GPU like NetCDF-3 records (:func:`from_xarray` does the rest, packed
+    coordinates included)."""
     import os
     if lazy is None:
         lazy = os.environ.get("LEC_DEVICE_INGEST", "1") != "0"
@@ -378,11 +411,7 @@ def open_netcdf4(path, variable_list_df, lazy=None):
     units = str(tv.attrs.get("units", ""))
     if " since " in units:
         tv.values = _decode_cf_time(tv.values, units, tv.attrs.get("calendar"))
-    for v in names[1:]:                       # coordinates: apply a packing if someone packed them
-        cv = ds[v]
-        if cv.values.dtype.kind in "iu" and ("scale_factor" in cv.attrs or "add_offset" in cv.attrs):
-            cv.values = cv.values * cv.attrs.get("scale_factor", 1.0) + cv.attrs.get("add_offset", 0.0)
-    return from_xarray(ds, variable_list_df, lazy=lazy and not any(r in variable_list_df.index for r in EXTRA_ROWS))
+    return from_xarray(ds, variable_list_df, lazy=lazy)
 
 
 def open_dataset(path, variable_list_df, lazy=None):
@@ -397,113 +426,42 @@ def open_dataset(path, variable_list_df, lazy=None):
     raise ValueError(f"{path}: neither a NetCDF-3 (CDF) nor a NetCDF-4 / HDF5 file")
 
 
-def _raw_store(f, wanted, order):
-    """A :class:`RawStore` over the variables of an open scipy ``netcdf_file`` (``mmap=False``: the arrays
-    own their memory), or None when the file layout needs the host path."""
-    fields, decode = {}, {}
-    for var in wanted:
-        v = f.variables[var]
-        data = v.data
-        if tuple(v.dimensions) != order or data.dtype.newbyteorder("=") not in (np.dtype(np.int16), np.dtype(np.float32),
-                                                                            np.dtype(np.float64)):
-            return None
-        at = {a: getattr(v, a) for a in v._attributes}
-        scale, offset = at.get("scale_factor"), at.get("add_offset")
-        fills = [at[k] for k in ("_FillValue", "missing_value") if k in at]
-        if len(fills) > 2 or (data.dtype.kind == "f" and (scale is not None or offset is not None)):
-            return None
-        if data.dtype.kind == "i" and scale is None and offset is None:
-            return None                                   # plain integers stay integers in xarray: not a field
-        fields[var] = data
-        decode[var] = dict(scale=None if scale is None else np.float64(scale),
-                           offset=None if offset is None else np.float64(offset),
-                           fills=[x.item() if hasattr(x, "item") else x for x in np.atleast_1d(fills).ravel()] if fills else [],
-                           float32=bool(data.dtype.kind == "i" and data.dtype.itemsize <= 2 and offset is None))
-    first = next(iter(fields.values()))
-    if any(a.dtype != first.dtype or a.shape != first.shape for a in fields.values()):
-        return None
-    nrec, nlev, nlat, nlon = first.shape
-    return RawStore(fields, decode, np.arange(nrec), np.arange(nlev), np.arange(nlat), np.arange(nlon))
-
-
 def from_xarray(ds, variable_list_df, lazy=True):
     """Adaptor for the reference's own loader: an ``xr.Dataset`` (``xr.open_dataset(infile)`` as in
     ``get_data``, preprocessing.py:35-147, or opened with ``mask_and_scale=False`` to keep packed int16
     records) -> :class:`LecDataset`, ready for :func:`process_data` / :func:`slice_domain`.  Duck-typed: only
     ``ds[name].values / .dims / .attrs`` are used, so xarray itself is not imported here.  Fields stored as
     ``(time, level, lat, lon)`` in one of int16 / float32 / float64 stay raw-backed (``lazy``); anything
-    else is transposed on the host."""
+    else is decoded and transposed on the host."""
     names = {row: variable_list_df.loc[row]["Variable"] for row in ("Time", "Vertical Level", "Latitude", "Longitude")}
     wanted = [variable_list_df.loc[r]["Variable"] for r in FIELD_ROWS if r in variable_list_df.index]
+    extra = [variable_list_df.loc[r]["Variable"] for r in EXTRA_ROWS if r in variable_list_df.index]
     out = LecDataset(names=names)
+
+    def read(name):                       # (values as stored, dims, attributes, decode rule)
+        a, at = np.asarray(ds[name].values), dict(ds[name].attrs)
+        return a, tuple(ds[name].dims), at, decode_rule(a.dtype, at)
     t = np.asarray(ds[names["Time"]].values)
     out.time = t.astype("datetime64[ns]") if np.issubdtype(t.dtype, np.datetime64) else t
-    out.level = np.asarray(ds[names["Vertical Level"]].values)
-    out.lat = np.asarray(ds[names["Latitude"]].values)
-    out.lon = np.asarray(ds[names["Longitude"]].values)
+    for row, attr in (("Vertical Level", "level"), ("Latitude", "lat"), ("Longitude", "lon")):
+        a, _, at, rule = read(names[row])
+        setattr(out, attr, apply_decode(a, rule))
     out.attrs[names["Vertical Level"]] = dict(ds[names["Vertical Level"]].attrs)
     order = (names["Time"], names["Vertical Level"], names["Latitude"], names["Longitude"])
-    arrays, dims, decode = {}, {}, {}
-    for var in wanted:
-        da = ds[var]
-        arrays[var], dims[var] = np.asarray(da.values), tuple(da.dims)
-        if sorted(dims[var]) != sorted(order):
-            raise ValueError(f"{var} has dimensions {dims[var]}, expected a permutation of {order}")
-        at = dict(da.attrs)
+    fields = {var: read(var) for var in wanted}
+    for var, (_, _, at, _) in fields.items():
         out.attrs[var] = at
-        packed = arrays[var].dtype.kind == "i"
-        scale, offset = (at.get("scale_factor"), at.get("add_offset")) if packed else (None, None)
-        fills = [at[k] for k in ("_FillValue", "missing_value") if k in at] if (packed or arrays[var].dtype.kind == "f") else []
-        decode[var] = dict(scale=None if scale is None else np.float64(scale),
-                           offset=None if offset is None else np.float64(offset),
-                           fills=[x.item() if hasattr(x, "item") else x for x in np.atleast_1d(fills).ravel()] if fills else [],
-                           float32=bool(packed and arrays[var].dtype.itemsize <= 2 and offset is None))
-    first = arrays[wanted[0]]
-    lazy = lazy and not any(r in variable_list_df.index for r in EXTRA_ROWS)
-    can_raw = lazy and all(dims[v] == order and a.dtype == first.dtype and a.shape == first.shape and
-                           a.dtype.newbyteorder("=") in (np.dtype(np.int16), np.dtype(np.float32), np.dtype(np.float64)) and
-                           (a.dtype.kind == "f" or decode[v]["scale"] is not None or decode[v]["offset"] is not None) and
-                           len(decode[v]["fills"]) <= 2
-                           for v, a in arrays.items())
-    if can_raw:
+    store = raw_store({var: (a, dims, rule) for var, (a, dims, _, rule) in fields.items()}, order) \
+        if lazy and not extra else None
+    if store is not None:
         def contiguous_records(a):        # the ABI wants every record C-contiguous
             return a if a.strides[1:] == np.empty(a.shape[1:], a.dtype).strides and a.strides[0] > 0 else np.ascontiguousarray(a)
-        nrec, nlev, nlat, nlon = first.shape
-        store = RawStore({v: contiguous_records(a) for v, a in arrays.items()}, decode,
-                         np.arange(nrec), np.arange(nlev), np.arange(nlat), np.arange(nlon))
+        store.fields = {v: contiguous_records(a) for v, a in store.fields.items()}
         out.raw, out.variables = store, _LazyVariables(store)
         return out
-    for var, a in arrays.items():         # eager: decode like xarray would have, then (time, level, lat, lon)
-        dec = decode[var]
-        if a.dtype.kind == "i" and (dec["scale"] is not None or dec["offset"] is not None):
-            raw = a
-            a = raw.astype(np.float32 if dec["float32"] else np.float64)
-            for fv in dec["fills"]:
-                a[raw == fv] = np.nan
-            if dec["scale"] is not None:
-                a *= dec["scale"]
-            if dec["offset"] is not None:
-                a += dec["offset"]
-        out.variables[var] = np.transpose(a, [dims[var].index(d) for d in order])
-    for row in EXTRA_ROWS:                # surface / extra fields of the host-side terms: (time[, level], lat, lon)
-        if row not in variable_list_df.index:
-            continue
-        var = variable_list_df.loc[row]["Variable"]
-        da = ds[var]
-        a, d = np.asarray(da.values), tuple(da.dims)
-        want = order if a.ndim == 4 else (order[0], order[2], order[3])
-        if sorted(d) != sorted(want):
-            raise ValueError(f"{var} has dimensions {d}, expected a permutation of {want}")
-        at = dict(da.attrs)
-        if a.dtype.kind in "iu" and ("scale_factor" in at or "add_offset" in at):
-            raw = a
-            a = raw.astype(np.float64)
-            for k in ("_FillValue", "missing_value"):
-                if k in at:
-                    a[raw == at[k]] = np.nan
-            a = a * at.get("scale_factor", 1.0) + at.get("add_offset", 0.0)
-        out.variables[var] = np.transpose(a, [d.index(x) for x in want])
-        out.attrs[var] = at
+    for var in wanted + extra:            # extra rows: (time, level, lat, lon) or a surface field (time, lat, lon)
+        a, dims, out.attrs[var], rule = fields[var] if var in fields else read(var)
+        out.variables[var] = _engine_order(var, apply_decode(a, rule), dims, order, surface=var in extra)
     return out
 
 

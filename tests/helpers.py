@@ -165,9 +165,23 @@ def write_era5_like(path, packed, nlon):
                 var[:] = arr
 
 
-def write_netcdf3_copy(src, dst, edit=None, extra=None):
+def write_era5_unheld_fill(path, nlon):
+    """:func:`write_era5_like`'s int16 file with a ``_FillValue`` no int16 can hold (40000) and stored 32767 values
+    (the value that fill saturates to in int16) spread over T and Z: no record is missing."""
+    src = path + ".src.nc"
+    write_era5_like(src, True, nlon)
+
+    def plant(name, data):
+        if name in ("T", "Z"):
+            data.reshape(-1)[::97] = 32767
+        return data
+    write_netcdf3_copy(src, path, plant, attrs={v: {"_FillValue": np.int32(40000)} for v in "TUVWZ"})
+
+
+def write_netcdf3_copy(src, dst, edit=None, extra=None, attrs=None):
     """Copy a NetCDF-3 classic file variable by variable, letting ``edit(name, array)`` change the data
-    (e.g. plant ``_FillValue`` entries); dimensions, dtypes and attributes are kept.  ``extra``: new variables,
+    (e.g. plant ``_FillValue`` entries; the variable takes the dtype of the array it returns); dimensions, dtypes and
+    attributes are kept, ``attrs``: ``name -> {attribute: value}`` set on top.  ``extra``: new variables,
     ``name -> (dims, array, attrs)``."""
     from scipy.io import netcdf_file
     with netcdf_file(src, mmap=False) as f, netcdf_file(dst, "w") as g:
@@ -177,13 +191,13 @@ def write_netcdf3_copy(src, dst, edit=None, extra=None):
             g.createDimension(name, size)
         for name, v in f.variables.items():
             data = np.array(v.data)
-            native = data.dtype.newbyteorder("=")
-            var = g.createVariable(name, native if native.kind != "S" else "c", v.dimensions)
-            for a in v._attributes:
-                setattr(var, a, getattr(v, a))
-            data = data.astype(native)
+            data = data.astype(data.dtype.newbyteorder("="))
             out = edit(name, data) if edit else None
-            var[:] = data if out is None else out
+            data = data if out is None else out
+            var = g.createVariable(name, data.dtype if data.dtype.kind != "S" else "c", v.dimensions)
+            for a, x in dict({a: getattr(v, a) for a in v._attributes}, **(attrs or {}).get(name, {})).items():
+                setattr(var, a, x)
+            var[:] = data
         for name, (dims, arr, attrs) in (extra or {}).items():
             var = g.createVariable(name, np.asarray(arr).dtype, dims)
             for k, v in attrs.items():

@@ -57,11 +57,11 @@ def test_catarina_lon_wrap_and_level_sort():
     assert np.all(np.diff(d.level) > 0) and d.level[0] == 1000.0 and d.level[-1] == 100000.0
 
 
-@pytest.mark.parametrize("case", ["ncep_fixed", "ncep_track", "catarina", "era5_f32", "era5_packed"])
+@pytest.mark.parametrize("case", ["ncep_fixed", "ncep_track", "catarina", "era5_f32", "era5_packed", "era5_unheld_fill"])
 def test_raw_backed_dataset_equals_host_prepared(case, tmp_path, monkeypatch):
     """Default loading keeps the fields in file layout (RawStore: only index maps move through
     process_data / slice_domain); what it materialises on access has the bits of the eager host pipeline
-    (LEC_DEVICE_INGEST=0)."""
+    (LEC_DEVICE_INGEST=0), also when the fill value is one the int16 records cannot hold."""
     nml = os.path.join(INP, "namelist_NCEP-R2")
     if case == "ncep_fixed":
         a = _args(fixed=True, box_limits=os.path.join(INP, "box_limits_Reg1"))
@@ -71,7 +71,10 @@ def test_raw_backed_dataset_equals_host_prepared(case, tmp_path, monkeypatch):
         a = _args(infile=os.path.join(SAM, "Catarina_NCEP-R2.nc"), fixed=True, box_limits=os.path.join(INP, "box_limits_Reg1"))
     else:
         nc = str(tmp_path / "testdata_ERA5.nc")
-        H.write_era5_like(nc, case == "era5_packed", 160)
+        if case == "era5_unheld_fill":
+            H.write_era5_unheld_fill(nc, 160)
+        else:
+            H.write_era5_like(nc, case == "era5_packed", 160)
         a = _args(infile=nc, track=True, trackfile=os.path.join(INP, "track_testdata_ERA5"))
         nml = os.path.join(INP, "namelist_ERA5")
     kw = dict(box_limits_file=a.box_limits) if a.box_limits else {}
@@ -97,15 +100,55 @@ class _FakeDataArray:
         self.values, self.dims, self.attrs = values, dims, dict(attrs or {})
 
 
-@pytest.mark.parametrize("packed", [False, True])
-def test_from_xarray_adaptor_equals_file_loader(tmp_path, packed):
+def _plant_float_fills(name, data):
+    if name in ("T", "U"):
+        data.reshape(-1)[::53] = -999.0 if name == "T" else 1e20
+    return data
+
+
+def _pack_coordinates(name, data):
+    if name == "latitude":                   # -5 - 0.25 k: decoded with the offset, to float64
+        return np.round((data + 5.0) / 0.25).astype(np.int16)
+    if name == "longitude":                  # -65 + 0.25 i: scale only, to float32
+        return np.round(data / np.float32(0.25)).astype(np.int16)
+    return None
+
+
+_PACKED_COORDS = {"latitude": {"scale_factor": 0.25, "add_offset": -5.0}, "longitude": {"scale_factor": np.float32(0.25)}}
+
+
+def _era5_case(tmp_path, case):
+    """The ERA5-like file and namelist of a :func:`test_from_xarray_adaptor_equals_file_loader` case."""
+    nc, nlf = str(tmp_path / "testdata_ERA5.nc"), os.path.join(INP, "namelist_ERA5")
+    H.write_era5_like(nc + ".src", case not in (False, "float_fills"), 160)
+    edit, attrs, extra = None, None, None
+    if case == "float_fills":
+        edit, attrs = _plant_float_fills, {v: {"_FillValue": np.float32(-999.0), "missing_value": np.float32(1e20)}
+                                           for v in "TUVWZ"}
+    elif case == "unsigned":                 # values NetCDF-3 can store as int16 and from_xarray gets as uint16
+        edit = lambda name, data: np.abs(data) if name in list("TUVWZ") else None
+    elif case == "extra_rows":
+        ust = np.round(np.random.default_rng(3).uniform(0, 3, size=(5, 141, 160)) / 1e-4).astype(np.int16)
+        ust.reshape(-1)[::53] = -32767
+        extra = {"UST": (("time", "latitude", "longitude"), ust, {"scale_factor": 1e-4, "_FillValue": np.int16(-32767)})}
+        nlf = str(tmp_path / "namelist")
+        with open(nlf, "w") as f:
+            f.write(open(os.path.join(INP, "namelist_ERA5")).read().rstrip("\n") + "\nFriction Velocity;;UST;m/s\n")
+    elif case == "packed_coords":
+        edit, attrs = _pack_coordinates, _PACKED_COORDS
+    H.write_netcdf3_copy(nc + ".src", nc, edit, extra, attrs)
+    return nc, PP.read_namelist(nlf)
+
+
+@pytest.mark.parametrize("case", [False, True, "float_fills", "unsigned", "extra_rows", "packed_coords"])
+def test_from_xarray_adaptor_equals_file_loader(tmp_path, case):
     """from_xarray on a duck-typed Dataset (``ds[name].values/.dims/.attrs``: what xr.open_dataset(...,
     mask_and_scale=False, decode_times=True) exposes) gives the dataset open_netcdf3 gives, raw-backed or not,
-    and one whose field is stored (time, lat, level, lon) is transposed on the host."""
+    and one whose field is stored (time, lat, level, lon) is transposed on the host.  Cases: float32 (False) or
+    int16-packed (True) fields; float32 fields with _FillValue and missing_value entries; packed fields held as
+    uint16; a packed Friction Velocity row with fill values; int16-packed latitude and longitude."""
     from scipy.io import netcdf_file
-    nc = str(tmp_path / "testdata_ERA5.nc")
-    H.write_era5_like(nc, packed, 160)
-    nl = PP.read_namelist(os.path.join(INP, "namelist_ERA5"))
+    nc, nl = _era5_case(tmp_path, case)
     ref = PP.open_netcdf3(nc, nl)
     with netcdf_file(nc, mmap=False) as f:
         ds = {}
@@ -113,14 +156,22 @@ def test_from_xarray_adaptor_equals_file_loader(tmp_path, packed):
             at = {a: (getattr(v, a).decode() if isinstance(getattr(v, a), bytes) else getattr(v, a)) for a in v._attributes}
             ds[name] = _FakeDataArray(np.array(v.data).astype(v.data.dtype.newbyteorder("=")), tuple(v.dimensions), at)
     ds["time"] = _FakeDataArray(ref.time, ("time",))                       # decode_times=True
+    if case == "unsigned":
+        for name in "TUVWZ":
+            ds[name].values = ds[name].values.astype(np.uint16)
     a = _args(infile=nc, track=True, trackfile=os.path.join(INP, "track_testdata_ERA5"))
     want = PP.slice_domain(PP.process_data(ref, a, nl), a, nl)
+    if case == "float_fills":
+        assert np.isnan(want["T"]).any() and np.isnan(want["U"]).any()
+    if case == "extra_rows":
+        assert want["UST"].dtype == np.float32 and np.isnan(want["UST"]).any()
     for lazy in (True, False):
         d = PP.from_xarray(ds, nl, lazy=lazy)
-        assert (d.raw is not None) == lazy
+        assert (d.raw is not None) == (lazy and case not in ("unsigned", "extra_rows"))
         got = PP.slice_domain(PP.process_data(d, a, nl), a, nl)
-        for c in ("time", "level", "lat", "lon"):
-            assert np.array_equal(getattr(got, c), getattr(want, c))
+        for c in ("time", "level", "lat", "lon", "rlats", "coslats", "rlons"):
+            assert getattr(got, c).dtype == getattr(want, c).dtype and np.array_equal(getattr(got, c), getattr(want, c)), c
+        assert set(got.variables.keys()) == set(want.variables.keys())
         for var in want.variables.keys():
             assert got[var].dtype == want[var].dtype and np.array_equal(got[var], want[var], equal_nan=True), var
     ds["T"] = _FakeDataArray(np.ascontiguousarray(np.swapaxes(ds["T"].values, 1, 2)),
@@ -168,8 +219,8 @@ def test_budget_and_residual_columns():
 
 def test_netcdf4_input_through_an_optional_reader(tmp_path, monkeypatch):
     """A NetCDF-4 (HDF5) file is routed by its signature to netCDF4 / h5py (neither ships with this image: a stand-in
-    module with netCDF4's API serves the bundled NetCDF-3 contents) and yields the dataset the NetCDF-3 path yields;
-    without a reader the error says what to install."""
+    module with netCDF4's API serves the bundled NetCDF-3 contents) and yields the dataset the NetCDF-3 path yields,
+    also from a copy whose latitude and longitude are int16-packed; without a reader the error says what to install."""
     import argparse
     import sys
     import types
@@ -202,10 +253,12 @@ def test_netcdf4_input_through_an_optional_reader(tmp_path, monkeypatch):
         def getncattr(self, a):
             return getattr(self._v, a)
 
+    served = [src]
+
     class Dataset:
         def __init__(self, path, mode="r"):
             assert path == str(fake)
-            self._f = netcdf_file(src, mmap=False)
+            self._f = netcdf_file(served[0], mmap=False)
             self.variables = {k: Var(v) for k, v in self._f.variables.items()}
             self.auto = True
 
@@ -222,11 +275,18 @@ def test_netcdf4_input_through_an_optional_reader(tmp_path, monkeypatch):
     mod = types.ModuleType("netCDF4")
     mod.Dataset = Dataset
     monkeypatch.setitem(sys.modules, "netCDF4", mod)
-    got = PP.prepare_data(args, nlf, box_limits_file=box)
-    args.infile = src
-    want = PP.prepare_data(args, nlf, box_limits_file=box)
-    assert got.raw is not None and want.raw is not None          # both stay raw-backed (decoded on the GPU)
-    for k in ("time", "level", "lat", "lon", "rlats", "coslats", "rlons"):
-        assert np.array_equal(getattr(got, k), getattr(want, k)), k
-    for var in ("TMP_2_ISBL", "V_VEL_2_ISBL"):
-        assert np.array_equal(np.asarray(got[var]), np.asarray(want[var]))
+    packed = str(tmp_path / "packed_coords.nc")      # latitude: scale only (float32), longitude: with an offset (float64)
+    H.write_netcdf3_copy(src, packed, lambda name, data: np.round(data / 2.5).astype(np.int16) if name == "lat_2" else
+                         np.round((data + 100.0) / 2.5).astype(np.int16) if name == "lon_2" else None,
+                         attrs={"lat_2": {"scale_factor": np.float32(2.5)}, "lon_2": {"scale_factor": 2.5, "add_offset": -100.0}})
+    for served[0], dtypes in ((src, (np.float32, np.float32)), (packed, (np.float32, np.float64))):
+        args.infile = str(fake)
+        got = PP.prepare_data(args, nlf, box_limits_file=box)
+        args.infile = served[0]
+        want = PP.prepare_data(args, nlf, box_limits_file=box)
+        assert got.raw is not None and want.raw is not None          # both stay raw-backed (decoded on the GPU)
+        assert (want.lat.dtype, want.lon.dtype) == dtypes
+        for k in ("time", "level", "lat", "lon", "rlats", "coslats", "rlons"):
+            assert getattr(got, k).dtype == getattr(want, k).dtype and np.array_equal(getattr(got, k), getattr(want, k)), k
+        for var in ("TMP_2_ISBL", "V_VEL_2_ISBL"):
+            assert np.array_equal(np.asarray(got[var]), np.asarray(want[var]))

@@ -1,11 +1,14 @@
 """lec_run_host_raw: fields still in FILE layout (latitude north-to-south, longitudes 0..360, levels in any
 order with extra ones above 10 hPa, int16-packed or float, a time selection) against lec_run_host on the
 arrays the host pipeline would have prepared -- bit-identical results, fewer PCIe bytes."""
+import os
+
 import numpy as np
 import pytest
 
 import helpers as H
 from lorenzcycletoolkit_b200 import engine as E
+from lorenzcycletoolkit_b200.utils import preprocessing as PP
 from test_engine_synthetic_gpu import _dataset
 
 pytestmark = pytest.mark.gpu
@@ -139,6 +142,29 @@ def test_big_endian_interleaved_records(dtype):
         assert np.array_equal(x, y)
 
 
+def test_fill_value_the_records_cannot_hold(tmp_path):
+    """int16 records with _FillValue = 40000, which no int16 equals, and stored 32767 values (what 40000 saturates to in
+    int16): lec_run_host_raw on the raw-backed dataset has the bits of lec_run_host on what it materialises, where the
+    32767 values are values, not missing."""
+    nc = str(tmp_path / "era5.nc")
+    H.write_era5_unheld_fill(nc, 160)
+    ds = PP.open_netcdf3(nc, PP.read_namelist(os.path.join(H.GOLDEN, "inputs", "namelist_ERA5")))
+    store = ds.raw.select("lat", slice(None, None, -1)).select("lev", slice(None, None, -1))
+    names = list("TUVWZ")
+    assert (store.fields["T"] == 32767).any() and not np.isnan(store.materialise("T")).any()
+    lat, lon = ds.lat[::-1], ds.lon
+    lev = np.asarray(ds.level[::-1], dtype=np.float64) * 100.0
+    rl, rp = np.deg2rad(lon), np.deg2rad(lat)
+    nt = len(store.rec)
+    steps = E.time_stencil(np.arange(nt) * 3600.0, E.make_steps(nt))
+    steps["i0"], steps["i1"], steps["j0"], steps["j1"] = 0, 159, 0, 140
+    with E.LecEngine(lon, lat, rl, rp, np.cos(rp), lev, np.float64, [1.0] * 5, max_steps=nt) as eng:
+        a = eng.run_host([np.ascontiguousarray(store.materialise(v)) for v in names], steps)
+        b = eng.run_host_raw([store.fields[v] for v in names], store.lon, store.lat, store.lev, store.rec, steps,
+                             decode=[store.decode[v] for v in names])
+    H.same_bits(a, b)
+
+
 def test_raw_records_in_staged_chunks():
     """Several staged chunks (small windows): the two raw staging buffers and the ingest stream are reused
     across chunks and calls; T halo slots come device-to-device from the previous chunk.  Every result has the bits of
@@ -233,3 +259,9 @@ def test_raw_errors():
             eng.run_host_raw(fields, ident[0][:-1], ident[1], ident[2], np.arange(3), steps)
         t, _, _ = eng.run_host_raw(fields, *ident, np.arange(3), steps)
         assert np.array_equal(t, eng.run_host(fields, steps)[0])
+        with pytest.raises(ValueError, match=r"invalid argument \(at most two fill values per field\)"):
+            eng.run_host_raw(fields, *ident, np.arange(3), steps, decode=[dict(fills=[1.0, 2.0, 3.0])] + [{}] * 4)
+        packed = [np.zeros(f.shape, dtype=np.int16) for f in fields]
+        scaled = [dict(scale=np.float64(0.01), float32=True)] * 5
+        with pytest.raises(ValueError, match=r"invalid argument \(a fill value is not an int16 value\)"):
+            eng.run_host_raw(packed, *ident, np.arange(3), steps, decode=[dict(scaled[0], fills=[40000.0])] + scaled[1:])

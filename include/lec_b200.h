@@ -238,6 +238,29 @@ int lec_run_device_packed(lec_handle *h, const lec_packed_desc *pd, const int16_
 #define LEC_NBOUNDARY_PIECES 18
 int lec_set_boundary_levels(lec_handle *h, double *out);
 
+/* 1: the following lec_run_host / lec_run_host_raw calls on this handle stage only each slot's window;
+ * 0 (default): whole slots.  Results keep their bits; only the bytes staged (lec_last_transfer) change.
+ * For a track run, whose prepared domain spans the whole track, the bytes follow the box instead of the domain.
+ * The windows of one call, computed once from all its steps:
+ *   - window of a slot: the union of the boxes (i0..i1 x j0..j1) of the steps that read it -- for T as centre slot or
+ *     time neighbour (slot, slot_m, slot_p), for u, v, omega and Phi as centre slot only.  The row kernels need no
+ *     value outside a box (the j-1 / j+1 rows and lon neighbours they use lie inside it), so there is no margin.
+ *   - column origin x0: rounded down to a multiple of 4 (LEC_F32) or 2 (LEC_F64) columns, so that the row kernels'
+ *     128-bit chunks and summation order are those of the grid.
+ *   - a slot is stored as its T window; all slots of the call share one buffer shape (the largest T window, rows
+ *     padded to whole 128-bit chunks), so a larger staging window (host_stage_bytes) fits in the same bytes.
+ * lec_last_transfer then counts, per (slot, field) that a greedy chunk stages (as without windows: T over the
+ * chunk's slot range minus the slots the previous chunk holds, the other four over its centre slot range; slots
+ * no step reads are skipped):
+ *   lec_run_host      nlev * (y1 - y0 + 1) * (x1 - x0 + 1) elements of the handle's dtype;
+ *   lec_run_host_raw  (max - min + 1 of lev_map: the raw level range, untouched levels inside it included)
+ *                     * (max - min + 1 of lat_map[y0..y1]) * w raw elements, where w = x1 - x0 + 1 when
+ *                     lon_map[x0..x1] is one increasing run of raw columns, else the raw row length: whole raw
+ *                     rows, e.g. when a longitude wrap's seam falls inside the window (the whole globe's row for
+ *                     a global file, where the two runs either side of the seam would do).
+ * LEC_ERR_INVALID unless on is 0 or 1. */
+int lec_set_host_windows(lec_handle *h, int32_t on);
+
 /* Page-lock (cudaHostRegister) / release a host range the caller keeps alive, so that the lec_run_host* copies
  * out of it run at the pinned PCIe rate instead of through the driver's pageable staging.  For the record arrays a
  * NetCDF reader returns (the reference's loader, src/utils/preprocessing.py:35-147, hands over pageable numpy
@@ -279,7 +302,8 @@ int lec_last_dispatch(const lec_handle *h, lec_dispatch *out);
 
 /* Bytes the last lec_run_host moved over PCIe: out[0] host->device (fields: T for every slot a step
  * or its time neighbours touch, u/v/omega/Phi for the centre slots only; slots shared by two staged
- * chunks are copied device-to-device and not counted), out[1] device->host (results). */
+ * chunks are copied device-to-device and not counted; with lec_set_host_windows, the windows' bytes),
+ * out[1] device->host (results). */
 int lec_last_transfer(lec_handle *h, int64_t out_bytes[2]);
 
 /* ---- 850-hPa track diagnostics (SURVEY.md 8(f) rank 1) --------------------------------------------
@@ -322,6 +346,15 @@ int lec_diag850_device(const lec_diag_grid *grid, const void *u, const void *v, 
                        void *cuda_stream);          /* u, v, z, out_* in device memory; steps on the host */
 int lec_diag850_host(const lec_diag_grid *grid, const void *u, const void *v, const void *z, int32_t nslots,
                      const lec_diag_step *steps, int32_t nsteps, double *out_val, int32_t *out_idx);
+/* lec_diag850_host on WINDOWS of the planes: u, v, z are [nslots][win_rows][win_cols] host arrays, plane s holding the
+ * domain points of columns origin[2 s] .. + win_cols - 1 and rows origin[2 s + 1] .. + win_rows - 1.  Box and centre
+ * indices of the steps stay domain indices; the results are those of lec_diag850_host on the whole planes, bit for
+ * bit.  The window a step needs: its box (and its centre point, when ic, jc >= 0) grown by one point a side and
+ * clamped to the domain, and where that meets a domain edge, at least three points along that axis (MetPy's
+ * one-sided first_derivative reads points 0..2 and n-3..n-1).  LEC_ERR_BOUNDS if a step reads outside its window. */
+int lec_diag850_host_windows(const lec_diag_grid *grid, const void *u, const void *v, const void *z, int32_t nslots,
+                             int32_t win_rows, int32_t win_cols, const int32_t *origin, const lec_diag_step *steps,
+                             int32_t nsteps, double *out_val, int32_t *out_idx);
 
 const char *lec_strerror(int code);
 const char *lec_last_error(lec_handle *h);   /* CUDA error text after LEC_ERR_CUDA (NULL: handle-free calls of this thread) */

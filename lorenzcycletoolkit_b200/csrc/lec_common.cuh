@@ -50,6 +50,13 @@ struct StepDev {
   // fp32 copies for the fp32-arithmetic row kernels (no double -> float conversions in the row set-up);
   // f_wWn / f_wEn are the edge weights relative to the uniform interior weight (LONW == 0)
   float f_ct_m, f_ct_p, f_ct_s, f_cxW, f_cxE, f_wW, f_wE, f_wWn, f_wEn, f_cyS, f_cyN, f_pad;
+  // Fields are addressed in the coordinates of each slot's window (lec_set_host_windows; origin 0 and window = grid
+  // otherwise): global column i, row j of slot s sit at window column i - ox(s), row j - oy(s).  Box indices and the
+  // grid tables stay global.  ox, oy: window origin of the centre slot; oxm, oym / oxp, oyp: of slot_m / slot_p (the
+  // tiled kernel's TMA coordinates); d_m, d_p: element offset of T(slot_m) / T(slot_p) from T(slot) at the same
+  // global point (the direct and sub-warp kernels; the host checks that they fit 31 bits).
+  int ox, oy, oxm, oym, oxp, oyp;
+  int d_m, d_p;
 };
 
 // Grid tables resident on the device (all fp64; built once in lec_create).

@@ -25,10 +25,11 @@ struct DiagAxis {          // first_derivative along one axis: out[i] = A[i] f[s
   int n;
 };
 
-struct DiagStepDev { int slot, i0, i1, j0, j1, ic, jc; };
+struct DiagStepDev { int slot, i0, i1, j0, j1, ic, jc, ox, oy; };   // ox, oy: window origin of the slot's planes
 
 struct DiagParams {
-  const void* u; const void* v; const void* z;      // [slot][lat][lon] planes of the 850-hPa level
+  const void* u; const void* v; const void* z;      // [slot][rows][ld] planes of the 850-hPa level: the domain, or a
+                                                     // window of it (lec_diag850_host_windows; origin per step)
   DiagAxis ax, ay;
   const double* ps;        // [nlat] parallel scale k
   const double* ms;        // [nlat] meridional scale h
@@ -38,7 +39,9 @@ struct DiagParams {
   const DiagStepDev* steps;
   double* out_val;                                     // [nsteps][5]: zeta min, zeta max, hgt min, wind max (NaNs skipped), zeta at the centre
   int* out_idx;                                        // [nsteps][4]: numpy argmin/argmax of the box, row-major flat index
-  int nlon, nlat;
+  int nlon, nlat;           // the domain (the stencil clamps, the metric tables)
+  int ld;                   // row length of the planes
+  long long plane;          // elements per plane
 };
 
 __device__ __forceinline__ double diag_d3(const DiagAxis& A, int i, double f0, double f1, double f2) {
@@ -49,14 +52,14 @@ __device__ __forceinline__ double diag_d3(const DiagAxis& A, int i, double f0, d
 template <typename FT>
 __device__ __forceinline__ double diag_zeta(const DiagParams& p, const FT* __restrict__ U, const FT* __restrict__ V,
                                             int j, int i, double& u0, double& v0) {
-  const long long o = (long long)j * p.nlon + i;
+  const long long o = (long long)j * p.ld + i;
   u0 = __dmul_rn(double(U[o]), p.su); v0 = __dmul_rn(double(V[o]), p.sv);
   const int si = min(max(i - 1, 0), p.nlon - 3), sj = min(max(j - 1, 0), p.nlat - 3);
-  const long long orow = (long long)j * p.nlon + si, ocol = (long long)sj * p.nlon + i;
+  const long long orow = (long long)j * p.ld + si, ocol = (long long)sj * p.ld + i;
   const double va = __dmul_rn(double(V[orow]), p.sv), vb = __dmul_rn(double(V[orow + 1]), p.sv),
                vc = __dmul_rn(double(V[orow + 2]), p.sv);
-  const double ua = __dmul_rn(double(U[ocol]), p.su), ub = __dmul_rn(double(U[ocol + p.nlon]), p.su),
-               uc = __dmul_rn(double(U[ocol + 2LL * p.nlon]), p.su);
+  const double ua = __dmul_rn(double(U[ocol]), p.su), ub = __dmul_rn(double(U[ocol + p.ld]), p.su),
+               uc = __dmul_rn(double(U[ocol + 2LL * p.ld]), p.su);
   const double dvdx_n = diag_d3(p.ax, i, va, vb, vc);
   const double dudy_n = diag_d3(p.ay, j, ua, ub, uc);
   const double mj = p.ms[j], pj = p.ps[j];
@@ -103,10 +106,11 @@ template <typename FT>
 __global__ void __launch_bounds__(kDiagThreads) lec_diag850_kernel(const DiagParams p) {
   const DiagStepDev st = p.steps[blockIdx.x];
   const int nx = st.i1 - st.i0 + 1, ny = st.j1 - st.j0 + 1;
-  const long long plane = (long long)p.nlat * p.nlon;
-  const FT* __restrict__ U = static_cast<const FT*>(p.u) + st.slot * plane;
-  const FT* __restrict__ V = static_cast<const FT*>(p.v) + st.slot * plane;
-  const FT* __restrict__ Z = static_cast<const FT*>(p.z) + st.slot * plane;
+  // shifted by the window origin: domain indices (j, i) address the planes
+  const long long base = st.slot * p.plane - ((long long)st.oy * p.ld + st.ox);
+  const FT* __restrict__ U = static_cast<const FT*>(p.u) + base;
+  const FT* __restrict__ V = static_cast<const FT*>(p.v) + base;
+  const FT* __restrict__ Z = static_cast<const FT*>(p.z) + base;
 
   DiagExt zmin, zmax, hmin, wmax;
   zmin.init(); zmax.init(); hmin.init(); wmax.init();
@@ -116,7 +120,7 @@ __global__ void __launch_bounds__(kDiagThreads) lec_diag850_kernel(const DiagPar
     double u0, v0;
     const double zeta = diag_zeta<FT>(p, U, V, j, i, u0, v0);
     const double wspd = __dsqrt_rn(__dadd_rn(__dmul_rn(u0, u0), __dmul_rn(v0, v0)));
-    const double hgt = __ddiv_rn(__dmul_rn(double(Z[(long long)j * p.nlon + i]), p.sz), p.zdiv);
+    const double hgt = __ddiv_rn(__dmul_rn(double(Z[(long long)j * p.ld + i]), p.sz), p.zdiv);
     zmin.take<true>(zeta, q); zmax.take<false>(zeta, q); hmin.take<true>(hgt, q); wmax.take<false>(wspd, q);
   }
   if (threadIdx.x == kDiagThreads - 1) {       // zeta at the track centre (domain indices; -1 = not requested)

@@ -44,7 +44,8 @@ struct lec_handle {
   std::vector<double> lon_deg, lat_deg, rlon, rlat, coslat, plev;
   // host-staging path
   void* stage[2][5] = {{nullptr}};
-  long long stage_slots = 0;
+  size_t stage_cap = 0;                       // bytes of each stage[b][f]: stage_cap / (bytes of one staged slot) slots
+  int host_windows = 0;                       // lec_set_host_windows
   void* raw_stage[2] = {nullptr, nullptr};   // raw sub-volumes (lec_run_host_raw): copy of n+1 overlaps ingest of n
   size_t raw_stage_bytes = 0;
   cudaStream_t s_ingest = nullptr;
@@ -141,7 +142,7 @@ EncodeTiledFn encode_tiled_fn() {
   return fn;
 }
 
-// 4-D tensor map over a [slot][level][lat][lon] field of `esize`-byte elements (fp64 / fp32 / int16) with a
+// 4-D tensor map over a [slot][level][lat][lon] field (or [slot][level][window row][window column]) of `esize`-byte elements (fp64 / fp32 / int16) with a
 // (bx x by) box in (lon, lat).
 bool make_map(CUtensorMap* m, const void* base, int esize, int nlon, int nlat, int nlev, int nslots, int bx, int by) {
   EncodeTiledFn enc = encode_tiled_fn();
@@ -257,14 +258,19 @@ cudaEvent_t next_event(lec_handle* h) {
   return h->ev_pool[h->ev_used++];
 }
 
-// Validate one step and build its device form.
-int build_step(const lec_handle* h, const lec_step& s, int nslots, StepDev& d) {
-  const int nlon = h->desc.nlon, nlat = h->desc.nlat;
+// The slot and box checks of one step (build_step; lec_run_host* before they compute windows from the steps).
+int check_step(const lec_handle* h, const lec_step& s, int nslots) {
   if (s.slot < 0 || s.slot >= nslots || s.slot_m < 0 || s.slot_m >= nslots || s.slot_p < 0 ||
       s.slot_p >= nslots)
     return LEC_ERR_BOUNDS;
-  if (s.i0 < 0 || s.i1 >= nlon || s.j0 < 0 || s.j1 >= nlat) return LEC_ERR_BOUNDS;
+  if (s.i0 < 0 || s.i1 >= h->desc.nlon || s.j0 < 0 || s.j1 >= h->desc.nlat) return LEC_ERR_BOUNDS;
   if (s.i1 - s.i0 < 1 || s.j1 - s.j0 < 1) return LEC_ERR_DEGENERATE;
+  return LEC_OK;
+}
+
+// Validate one step and build its device form.
+int build_step(const lec_handle* h, const lec_step& s, int nslots, StepDev& d) {
+  if (const int rc = check_step(h, s, nslots)) return rc;
   if (s.j1 - s.j0 + 1 > h->max_ny) return LEC_ERR_BOUNDS;
   const double* x = h->lon_deg.data();
   const double* y = h->lat_deg.data();
@@ -272,6 +278,8 @@ int build_step(const lec_handle* h, const lec_step& s, int nslots, StepDev& d) {
   const double* rp = h->rlat.data();
   d.slot = s.slot; d.slot_m = s.slot_m; d.slot_p = s.slot_p;
   d.i0 = s.i0; d.i1 = s.i1; d.j0 = s.j0; d.j1 = s.j1; d.rec_base = 0;
+  d.ox = d.oy = d.oxm = d.oym = d.oxp = d.oyp = 0;       // window origins and T offsets: run_batch
+  d.d_m = d.d_p = 0;
   // every constant factor of Q = cp (dT/dt + u dT/dx + v dT/dy - S omega) is folded on the host
   const double q0 = kCp * h->g.scale[0], qv = q0 * h->g.scale[2];
   d.ct_m = q0 * s.ct_m; d.ct_p = q0 * s.ct_p; d.ct_s = q0 * (s.ct_m + s.ct_0 + s.ct_p);
@@ -583,17 +591,22 @@ int lec_create(lec_handle** out, const lec_grid_desc* desc) {
   return LEC_OK;
 }
 
+// Window of every staged slot of a kernel batch (lec_set_host_windows): the shared shape and each slot's origin,
+// indexed by the batch's slot numbers.
+struct WinView { int rows, pitch; const int* ox; const int* oy; };
+
 // One kernel batch (<= max_steps steps) on `st`.  pitch: row length of the fields in elements (0: the grid's);
-// pk: the fields are int16, decoded by the row kernel (lec_run_device_packed).
+// pk: the fields are int16, decoded by the row kernel (lec_run_device_packed); win: the fields are staged windows.
 static int run_batch(lec_handle* h, const void* const fields[5], int nslots, const lec_step* steps, int n,
                      double* out_terms, double* out_levels, int* out_flags, double* out_bnd, cudaStream_t st,
-                     int pitch = 0, const PackedDev* pk = nullptr) {
+                     int pitch = 0, const PackedDev* pk = nullptr, const WinView* win = nullptr) {
   // nlon below is the ROW LENGTH of the field buffers: the grid's for caller-owned fp device fields, the padded
   // pitch of the engine's own staging or of caller-owned int16 fields (box indices are checked against the grid
-  // in build_step)
-  const int L = h->desc.nlev, nlon = pitch > 0 ? pitch : h->desc.nlon;
+  // in build_step); with windows, the rows of a slot are win->rows rows of win->pitch elements
+  const int L = h->desc.nlev, nlon = win ? win->pitch : pitch > 0 ? pitch : h->desc.nlon;
+  const int nrows = win ? win->rows : h->desc.nlat;
   GridDev gd = h->g;
-  gd.nlon = nlon;
+  gd.nlon = pitch > 0 ? pitch : h->desc.nlon;       // (the tiled kernel's shared weight table: global columns)
   int max_rows = 0, max_cols = 0;
   bool same_box = true, same_rows = true;
   const int par = h->batch_parity;
@@ -604,16 +617,18 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   for (int s = 0; s < n; ++s) {
     const int rc = build_step(h, steps[s], nslots, hs[s]);
     if (rc != LEC_OK) return rc;
+    if (win) {
+      StepDev& d = hs[s];
+      d.ox = win->ox[d.slot]; d.oy = win->oy[d.slot];
+      d.oxm = win->ox[d.slot_m]; d.oym = win->oy[d.slot_m];
+      d.oxp = win->ox[d.slot_p]; d.oyp = win->oy[d.slot_p];
+    }
     max_rows = std::max(max_rows, steps[s].j1 - steps[s].j0 + 1);
     max_cols = std::max(max_cols, steps[s].i1 - steps[s].i0 + 1);
     same_box = same_box && steps[s].i0 == steps[0].i0 && steps[s].i1 == steps[0].i1 &&
                steps[s].j0 == steps[0].j0 && steps[s].j1 == steps[0].j1;
     same_rows = same_rows && steps[s].j1 - steps[s].j0 == steps[0].j1 - steps[0].j0;
   }
-  CK(cudaMemcpyAsync(ds, hs, sizeof(StepDev) * n, cudaMemcpyHostToDevice, st));
-  CK(cudaEventRecord(h->ev_steps[par], st));
-  h->steps_pending[par] = true;
-
   // latitude banding (fixed box, several steps): sweep time inside a band of box rows so T(t+-1) stays in L2
   int band_rows = h->desc.band_rows;
   if (band_rows <= 0) {
@@ -661,15 +676,17 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
     // The direct and sub-warp kernels address T(slot_m) and T(slot_p) as 32-bit element offsets from T(slot) (64-bit
     // bases instead spill in the sub-warp kernel's fp64-arithmetic instances); the tiled kernel takes slots as TMA
     // coordinates and has no such limit.
-    const long long stride = (long long)L * h->desc.nlat * nlon;
+    const long long stride = (long long)L * nrows * nlon;
     for (int s = 0; s < n; ++s) {
-      const long long dm = (long long)(steps[s].slot_m - steps[s].slot) * stride;
-      const long long dp = (long long)(steps[s].slot_p - steps[s].slot) * stride;
+      StepDev& q = hs[s];
+      const long long dm = (long long)(q.slot_m - q.slot) * stride + (long long)(q.oy - q.oym) * nlon + (q.ox - q.oxm);
+      const long long dp = (long long)(q.slot_p - q.slot) * stride + (long long)(q.oy - q.oyp) * nlon + (q.ox - q.oxp);
       if (dm <= -(1LL << 31) || dm >= (1LL << 31) || dp <= -(1LL << 31) || dp >= (1LL << 31)) {
         h->err = "slot_m / slot_p lie 2^31 or more elements from slot, which the direct and sub-warp row kernels "
                  "cannot address (the tiled kernel can)";
         return LEC_ERR_INVALID;
       }
+      q.d_m = (int)dm; q.d_p = (int)dp;
     }
   }
   const int tile_rows = d.tile_rows;
@@ -688,7 +705,9 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   rp.dv_lev = FastDiv::make((unsigned)L);
   rp.dv_steps = FastDiv::make((unsigned)n);
   rp.nbands = (max_rows + band_rows - 1) / band_rows;
-  rp.slot_stride = (long long)L * h->desc.nlat * nlon;
+  rp.slot_stride = (long long)L * nrows * nlon;
+  rp.lev_stride = (long long)nrows * nlon;
+  rp.row_stride = nlon;
   if (rp.slot_stride >= (1LL << 31)) { h->err = "one time slot holds 2^31 or more elements"; return LEC_ERR_INVALID; }
   const long long grid = (long long)rp.nbands * n * L * rp.tiles_per_band;
   if (grid > 0x7fffffffLL) return LEC_ERR_INVALID;
@@ -697,6 +716,9 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
   d.tiles_per_band = rp.tiles_per_band; d.nbands = rp.nbands;
   h->dispatch = d;
   h->dispatched = true;
+  CK(cudaMemcpyAsync(ds, hs, sizeof(StepDev) * n, cudaMemcpyHostToDevice, st));
+  CK(cudaEventRecord(h->ev_steps[par], st));
+  h->steps_pending[par] = true;
 
   cudaEvent_t e0 = next_event(h), e1 = next_event(h), e2 = next_event(h);
   if (!e0 || !e1 || !e2) { h->err = "cudaEventCreate"; return LEC_ERR_CUDA; }
@@ -707,13 +729,12 @@ static int run_batch(lec_handle* h, const void* const fields[5], int nslots, con
     const int C = f64 ? 64 : 128, V = f64 ? 2 : 4, R = d.tile_rows;
     // box widths of TileGeom: int16 boxes have 8 more columns and a 16-byte halo on each side (aligned box starts)
     const int esz = pk ? 2 : f64 ? 8 : 4, PW = pk ? C + 8 : C, HV = pk ? 8 : V;
-    const int nlat = h->desc.nlat;
-    bool ok = make_map(&maps.t_halo, fields[0], esz, nlon, nlat, L, nslots, PW + 2 * HV, R + 2) &&
-              make_map(&maps.t_plain, fields[0], esz, nlon, nlat, L, nslots, PW, R) &&
-              make_map(&maps.u, fields[1], esz, nlon, nlat, L, nslots, PW, R) &&
-              make_map(&maps.v, fields[2], esz, nlon, nlat, L, nslots, PW, R) &&
-              make_map(&maps.w, fields[3], esz, nlon, nlat, L, nslots, PW, R) &&
-              make_map(&maps.f, fields[4], esz, nlon, nlat, L, nslots, PW, R);
+    bool ok = make_map(&maps.t_halo, fields[0], esz, nlon, nrows, L, nslots, PW + 2 * HV, R + 2) &&
+              make_map(&maps.t_plain, fields[0], esz, nlon, nrows, L, nslots, PW, R) &&
+              make_map(&maps.u, fields[1], esz, nlon, nrows, L, nslots, PW, R) &&
+              make_map(&maps.v, fields[2], esz, nlon, nrows, L, nslots, PW, R) &&
+              make_map(&maps.w, fields[3], esz, nlon, nrows, L, nslots, PW, R) &&
+              make_map(&maps.f, fields[4], esz, nlon, nrows, L, nslots, PW, R);
     if (!ok) { h->err = "cuTensorMapEncodeTiled failed"; return LEC_ERR_CUDA; }
   }
   const cudaError_t le = launch_rows(h, d, rp, maps, grid, st);
@@ -802,6 +823,135 @@ struct HostSource {
   int jr_lo = 0, jr_hi = 0, kr_lo = 0, kr_hi = 0;     // raw rows / levels the maps touch
 };
 
+// lec_set_host_windows: the window of every slot of one lec_run_host* call.  A rectangle of global columns x0..x1 and
+// rows y0..y1 (x1 < x0: the slot is not read), and for raw records the part of a record it is decoded from: raw rows
+// jr0 .. jr0 + nj - 1 of every touched level, raw columns rc0 .. rc0 + rw - 1.
+struct Rect { int x0 = 0, x1 = -1, y0 = 0, y1 = -1; int jr0 = 0, nj = 0, rc0 = 0, rw = 0; };
+struct HostWindows {
+  int rows = 0, pitch = 0;                 // the shape all slots share
+  std::vector<Rect> t, c;                  // per slot: T (= the slot's window: its origin), u / v / omega / Phi
+  std::vector<int> ox, oy;                 // per slot: origin of the window
+};
+
+// The windows of a call (header: lec_set_host_windows).  The row kernels read, around a box, the T rows j - 1 / j + 1
+// of its interior rows and the lon neighbours of its interior columns -- all inside the box -- and load (tiled kernel:
+// the halo rows and the 16-byte lon-halo vector of every tile; every kernel: the pad columns of a box's edge chunks)
+// values outside it that never reach a result.  So a window is the union of the boxes, its column origin rounded down
+// to a 128-bit chunk so that window chunks are grid chunks (the lane <-> column map, and with it every sum, keeps its
+// order).
+static void host_windows(const lec_handle* h, const HostSource& src, int nslots, const lec_step* steps, int nsteps,
+                         HostWindows& w) {
+  const int vecw = h->desc.dtype == LEC_F64 ? 2 : 4;
+  w.t.assign(nslots, Rect{}); w.c.assign(nslots, Rect{});
+  auto grow = [](Rect& r, const lec_step& s) {
+    if (r.x1 < r.x0) { r.x0 = s.i0; r.x1 = s.i1; r.y0 = s.j0; r.y1 = s.j1; return; }
+    r.x0 = std::min(r.x0, s.i0); r.x1 = std::max(r.x1, s.i1); r.y0 = std::min(r.y0, s.j0); r.y1 = std::max(r.y1, s.j1);
+  };
+  for (int n = 0; n < nsteps; ++n) {
+    const lec_step& s = steps[n];
+    grow(w.c[s.slot], s); grow(w.t[s.slot], s); grow(w.t[s.slot_m], s); grow(w.t[s.slot_p], s);
+  }
+  w.rows = w.pitch = 0;
+  w.ox.assign(nslots, 0); w.oy.assign(nslots, 0);
+  for (int sl = 0; sl < nslots; ++sl) {
+    for (Rect* r : {&w.t[sl], &w.c[sl]}) {
+      if (r->x1 < r->x0) continue;
+      r->x0 -= r->x0 % vecw;
+      if (src.raw) {                      // raw rows of the window rows; raw columns if they are one increasing run
+        const int* lat = src.raw->lat_map + r->y0;
+        const int* lon = src.raw->lon_map + r->x0;
+        int lo = lat[0], hi = lat[0];
+        for (int j = 1; j <= r->y1 - r->y0; ++j) { lo = std::min(lo, lat[j]); hi = std::max(hi, lat[j]); }
+        r->jr0 = lo; r->nj = hi - lo + 1;
+        bool run = true;
+        for (int i = 1; i <= r->x1 - r->x0 && run; ++i) run = lon[i] == lon[0] + i;
+        r->rc0 = run ? lon[0] : 0; r->rw = run ? r->x1 - r->x0 + 1 : src.raw->nlon;
+      }
+    }
+    const Rect& t = w.t[sl];
+    if (t.x1 < t.x0) continue;
+    w.ox[sl] = t.x0; w.oy[sl] = t.y0;
+    w.rows = std::max(w.rows, t.y1 - t.y0 + 1);
+    w.pitch = std::max(w.pitch, (t.x1 - t.x0 + vecw) / vecw * vecw);
+  }
+}
+
+// The ingest kernel over ip (raw element type of r, the handle's field type) on s_ingest.
+static void launch_ingest(const lec_handle* h, const lec_raw_desc& r, const IngestParams& ip, dim3 grid) {
+  const bool f64 = h->desc.dtype == LEC_F64;
+  if (r.dtype == LEC_RAW_I16) {
+    if (f64) lec_ingest_kernel<short, double><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
+    else lec_ingest_kernel<short, float><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
+  } else if (r.dtype == LEC_RAW_F32) {
+    lec_ingest_kernel<float, float><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
+  } else {
+    lec_ingest_kernel<double, double><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
+  }
+}
+
+// stage_field with windows: the rectangle of field f of every slot in [s_lo, s_hi] that has one, into that slot's
+// window (slot s at position s - win_lo of stage[b][f]), on s_copy.  Engine-layout arrays: one 3-D copy per slot.  Raw
+// records: one 3-D copy of the rectangle's raw rows (and raw columns, when they are one run) of every touched level,
+// then the ingest kernel over the rectangle.
+static int stage_field_windows(lec_handle* h, const HostSource& src, const HostWindows& w, int f, int b, int win_lo,
+                               int s_lo, int s_hi, size_t slot_bytes) {
+  const int L = h->desc.nlev;
+  const size_t elem = h->elem;
+  const std::vector<Rect>& rects = f == 0 ? w.t : w.c;
+  for (int s = s_lo; s <= s_hi; ++s) {
+    const Rect& q = rects[s];
+    if (q.x1 < q.x0) continue;
+    const int nx = q.x1 - q.x0 + 1, ny = q.y1 - q.y0 + 1;
+    char* slot_dst = static_cast<char*>(h->stage[b][f]) + (size_t)(s - win_lo) * slot_bytes;
+    if (!src.raw) {
+      cudaMemcpy3DParms cp{};
+      cp.srcPtr = make_cudaPitchedPtr(const_cast<void*>(src.fields[f]), h->desc.nlon * elem, h->desc.nlon * elem, h->desc.nlat);
+      cp.srcPos = make_cudaPos(q.x0 * elem, q.y0, (size_t)s * L);
+      cp.dstPtr = make_cudaPitchedPtr(slot_dst, w.pitch * elem, w.pitch * elem, w.rows);
+      cp.dstPos = make_cudaPos((q.x0 - w.ox[s]) * elem, q.y0 - w.oy[s], 0);
+      cp.extent = make_cudaExtent(nx * elem, ny, L);
+      cp.kind = cudaMemcpyHostToDevice;
+      CK(cudaMemcpy3DAsync(&cp, h->s_copy));
+      h->h2d_bytes += (long long)L * ny * nx * (long long)elem;
+      continue;
+    }
+    const lec_raw_desc& r = *src.raw;
+    const size_t relem = r.dtype == LEC_RAW_I16 ? 2 : r.dtype == LEC_RAW_F32 ? 4 : 8;
+    const int nk = src.kr_hi - src.kr_lo + 1;
+    const size_t row_bytes = (size_t)r.nlon * relem, rec_bytes = row_bytes * r.nlat * r.nlev;
+    const size_t rec_stride = r.record_stride[f] > 0 ? (size_t)r.record_stride[f] : rec_bytes;
+    const char* rec = static_cast<const char*>(src.fields[f]) + (size_t)src.slot_record[s] * rec_stride;
+    const int rb = int(h->raw_seq & 1);
+    if (h->raw_seq >= 2) CK(cudaStreamWaitEvent(h->s_copy, h->ev_raw_free[rb], 0));   // its last ingest has read it
+    ++h->raw_seq;
+    cudaMemcpy3DParms cp{};
+    cp.srcPtr = make_cudaPitchedPtr(const_cast<char*>(rec), row_bytes, row_bytes, r.nlat);
+    cp.srcPos = make_cudaPos(q.rc0 * relem, q.jr0, src.kr_lo);
+    cp.dstPtr = make_cudaPitchedPtr(h->raw_stage[rb], q.rw * relem, q.rw * relem, q.nj);
+    cp.dstPos = make_cudaPos(0, 0, 0);
+    cp.extent = make_cudaExtent(q.rw * relem, q.nj, nk);
+    cp.kind = cudaMemcpyHostToDevice;
+    CK(cudaMemcpy3DAsync(&cp, h->s_copy));
+    h->h2d_bytes += (long long)nk * q.nj * q.rw * (long long)relem;
+    CK(cudaEventRecord(h->ev_raw_ready[rb], h->s_copy));
+    CK(cudaStreamWaitEvent(h->s_ingest, h->ev_raw_ready[rb], 0));
+    IngestParams ip = src.dec[f];
+    // the maps from the rectangle's origin on; the source pointer is shifted so that raw column rc0 is its element 0
+    ip.lon_map = h->d_maps + q.x0; ip.lat_map = h->d_maps + h->desc.nlon + q.y0;
+    ip.lev_map = h->d_maps + h->desc.nlon + h->desc.nlat;
+    ip.nlon = nx; ip.nlat = w.rows; ip.nlev = L; ip.pitch = w.pitch;      // (nlat: rows per level of the window)
+    ip.rlon = q.rw; ip.nj_raw = q.nj; ip.jr_lo = q.jr0; ip.kr_lo = src.kr_lo;
+    ip.big_endian = r.big_endian != 0;
+    ip.src = static_cast<const char*>(h->raw_stage[rb]) - (ptrdiff_t)q.rc0 * (ptrdiff_t)relem;
+    ip.dst = slot_dst + ((size_t)(q.y0 - w.oy[s]) * w.pitch + (q.x0 - w.ox[s])) * elem;
+    launch_ingest(h, r, ip, dim3((nx + 4 * kIngestThreads - 1) / (4 * kIngestThreads), ny, L));
+    CK(cudaEventRecord(h->ev_raw_free[rb], h->s_ingest));
+    CK(cudaGetLastError());
+    ++h->launches;
+  }
+  return LEC_OK;
+}
+
 // Bring engine slots [s_lo, s_hi] of field f into stage[b][f] (slot s at position s - win_lo), on s_copy.
 static int stage_field(lec_handle* h, const HostSource& src, int f, int b, int win_lo, int s_lo, int s_hi,
                        size_t slot_bytes) {
@@ -847,15 +997,7 @@ static int stage_field(lec_handle* h, const HostSource& src, int f, int b, int w
     CK(cudaStreamWaitEvent(h->s_ingest, h->ev_raw_ready[rb], 0));
     ip.src = h->raw_stage[rb];
     ip.dst = dst + (size_t)(s - s_lo) * slot_bytes;
-    const bool f64 = h->desc.dtype == LEC_F64;
-    if (r.dtype == LEC_RAW_I16) {
-      if (f64) lec_ingest_kernel<short, double><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
-      else lec_ingest_kernel<short, float><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
-    } else if (r.dtype == LEC_RAW_F32) {
-      lec_ingest_kernel<float, float><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
-    } else {
-      lec_ingest_kernel<double, double><<<grid, kIngestThreads, 0, h->s_ingest>>>(ip);
-    }
+    launch_ingest(h, r, ip, grid);
     CK(cudaEventRecord(h->ev_raw_free[rb], h->s_ingest));
     CK(cudaGetLastError());
     ++h->launches;
@@ -870,10 +1012,19 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
   // The engine's own slots have rows padded to whole 128-bit chunks, so the vector / sub-warp kernels run
   // for every grid width.  Engine-layout host arrays whose rows are not such a multiple take the ingest
   // route too (identity maps): a contiguous H2D copy per slot, then a device pass that re-pitches it.
-  const size_t slot_bytes = (size_t)L * h->desc.nlat * h->pitch * h->elem;
+  // With windows (lec_set_host_windows) a staged slot is one window of every level instead, for both sources.
+  HostWindows win;
+  const bool windows = h->host_windows != 0;
+  if (windows) {                       // the windows come from every step: check them first (as build_step does)
+    for (int s = 0; s < nsteps; ++s)
+      if (const int rc = check_step(h, steps[s], nslots)) { h->err = "step " + std::to_string(s) + ": bad slot or box"; return rc; }
+    host_windows(h, src, nslots, steps, nsteps, win);
+  }
+  const size_t slot_bytes = windows ? (size_t)L * win.rows * win.pitch * h->elem
+                                    : (size_t)L * h->desc.nlat * h->pitch * h->elem;
   lec_raw_desc ident;
   std::vector<int32_t> iota;
-  if (!src.raw && h->pitch != h->desc.nlon) {
+  if (!src.raw && h->pitch != h->desc.nlon && !windows) {
     const int m = std::max(std::max(h->desc.nlon, h->desc.nlat), std::max(L, (int)nslots));
     iota.resize(m);
     for (int i = 0; i < m; ++i) iota[i] = i;
@@ -895,7 +1046,13 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
   if (src.raw) {
     const lec_raw_desc& r = *src.raw;
     const size_t relem = r.dtype == LEC_RAW_I16 ? 2 : r.dtype == LEC_RAW_F32 ? 4 : 8;
-    const size_t need = (size_t)(src.kr_hi - src.kr_lo + 1) * (src.jr_hi - src.jr_lo + 1) * r.nlon * relem;
+    size_t need = (size_t)(src.kr_hi - src.kr_lo + 1) * (src.jr_hi - src.jr_lo + 1) * r.nlon * relem;
+    if (windows) {                     // the largest window part of a record
+      need = 0;
+      for (const std::vector<Rect>* rs : {&win.t, &win.c})
+        for (const Rect& q : *rs)
+          if (q.x0 <= q.x1) need = std::max(need, (size_t)(src.kr_hi - src.kr_lo + 1) * q.nj * q.rw * relem);
+    }
     if (!h->s_ingest) {
       CK(cudaStreamCreateWithFlags(&h->s_ingest, cudaStreamNonBlocking));
       for (int b = 0; b < 2; ++b) {
@@ -924,19 +1081,22 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
   // Staging window: as many slots as this call can use (nslots, max_steps + 2 halo slots) within the byte
   // budget.  A reused handle whose earlier call was shorter gets a larger window here -- the window of the
   // first call must not cap the later ones (a 1- or 2-slot window cannot hold slot_m, slot, slot_p).
-  if (h->stage_slots < std::min<long long>((long long)h->max_steps + 2, nslots)) {
+  // (Windows make a staged slot smaller, so the same buffers hold more of them: the window counts in slots of this
+  // call's size.)
+  long long stage_slots = (long long)(h->stage_cap / slot_bytes);
+  if (stage_slots < std::min<long long>((long long)h->max_steps + 2, nslots)) {
     long long budget = h->desc.host_stage_bytes;
     if (budget <= 0) {
       size_t fr = 0, tot = 0;
       CK(cudaMemGetInfo(&fr, &tot));
-      fr += (size_t)h->stage_slots * slot_bytes * 10;          // what the old window gives back
+      fr += h->stage_cap * 10;                                  // what the old window gives back
       budget = (long long)std::min<size_t>(fr / 4, (size_t)32 << 30);
     }
     long long slots = budget / (long long)(2 * 5 * slot_bytes);
     slots = std::min<long long>(slots, (long long)h->max_steps + 2);
     slots = std::min<long long>(slots, nslots);
     if (slots < 1) { h->err = "host_stage_bytes too small for one slot"; return LEC_ERR_NOMEM; }
-    if (slots > h->stage_slots) {
+    if (slots > stage_slots) {
       if (h->stage[0][0]) {            // nothing of an earlier call may still read or write the old window
         CK(cudaStreamSynchronize(h->s_copy));
         CK(cudaStreamSynchronize(h->s_comp));
@@ -944,13 +1104,14 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
       }
       for (int b = 0; b < 2; ++b)
         for (int f = 0; f < 5; ++f) { cudaFree(h->stage[b][f]); h->stage[b][f] = nullptr; }
-      h->stage_slots = 0;
+      h->stage_cap = 0;
       for (int b = 0; b < 2; ++b)
         for (int f = 0; f < 5; ++f)
           if (cudaMalloc(&h->stage[b][f], (size_t)slots * slot_bytes) != cudaSuccess) {
             cudaGetLastError(); h->err = "staging buffers"; return LEC_ERR_NOMEM;
           }
-      h->stage_slots = slots;
+      h->stage_cap = (size_t)slots * slot_bytes;
+      stage_slots = slots;
     }
   }
   if (h->out_cap < nsteps) {
@@ -982,7 +1143,7 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
         return LEC_ERR_BOUNDS;
       const int nlo = std::min(std::min(lo, s.slot), std::min(s.slot_m, s.slot_p));
       const int nhi = std::max(std::max(hi, s.slot), std::max(s.slot_m, s.slot_p));
-      if (nhi - nlo + 1 > h->stage_slots) break;
+      if (nhi - nlo + 1 > stage_slots) break;
       lo = nlo; hi = nhi; ++s1;
     }
     if (s1 == s0) { h->err = "one step needs more slots than the staging window holds"; return LEC_ERR_NOMEM; }
@@ -1001,12 +1162,16 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
                          (size_t)(ov_hi - lo + 1) * slot_bytes, cudaMemcpyDeviceToDevice, h->s_copy));
       t_lo = ov_hi + 1;
     }
-    { const int rc = stage_field(h, src, 0, b, lo, t_lo, hi, slot_bytes); if (rc != LEC_OK) return rc; }
+    auto stage = [&](int f, int s_lo, int s_hi) {
+      return windows ? stage_field_windows(h, src, win, f, b, lo, s_lo, s_hi, slot_bytes)
+                     : stage_field(h, src, f, b, lo, s_lo, s_hi, slot_bytes);
+    };
+    { const int rc = stage(0, t_lo, hi); if (rc != LEC_OK) return rc; }
     // u, v, omega, Phi are read at the centre slots only
     int c_lo = 1 << 30, c_hi = -1;
     for (int s = s0; s < s1; ++s) { c_lo = std::min(c_lo, steps[s].slot); c_hi = std::max(c_hi, steps[s].slot); }
     for (int f = 1; f < 5; ++f) {
-      const int rc = stage_field(h, src, f, b, lo, c_lo, c_hi, slot_bytes);
+      const int rc = stage(f, c_lo, c_hi);
       if (rc != LEC_OK) return rc;
     }
     prev_lo = lo; prev_hi = hi;
@@ -1018,10 +1183,12 @@ static int run_host_impl(lec_handle* h, HostSource& src, int32_t nslots, const l
     CK(cudaStreamWaitEvent(h->s_comp, h->ev_copied[b], 0));
     local.assign(steps + s0, steps + s1);
     for (lec_step& s : local) { s.slot -= lo; s.slot_m -= lo; s.slot_p -= lo; }
+    const WinView wv{win.rows, win.pitch, windows ? win.ox.data() + lo : nullptr, windows ? win.oy.data() + lo : nullptr};
     const int rc = run_batch(h, h->stage[b], hi - lo + 1, local.data(), s1 - s0,
                              h->d_out_terms + (size_t)s0 * LEC_NTERMS,
                              h->d_out_levels + (size_t)s0 * LEC_NLEVEL_TERMS * L, h->d_out_flags + s0,
-                             h->bnd_user ? h->d_out_bnd + (size_t)s0 * kNB * L : nullptr, h->s_comp, h->pitch);
+                             h->bnd_user ? h->d_out_bnd + (size_t)s0 * kNB * L : nullptr, h->s_comp, h->pitch,
+                             nullptr, windows ? &wv : nullptr);
     if (rc != LEC_OK) return rc;
     CK(cudaEventRecord(h->ev_done[b], h->s_comp));
     s0 = s1; ++chunk;
@@ -1105,6 +1272,12 @@ int lec_unpin_host(void* ptr) {
   return LEC_OK;
 }
 
+int lec_set_host_windows(lec_handle* h, int32_t on) {
+  if (!h || (on != 0 && on != 1)) return LEC_ERR_INVALID;
+  h->host_windows = on;
+  return LEC_OK;
+}
+
 int lec_set_boundary_levels(lec_handle* h, double* out) {
   if (!h) return LEC_ERR_INVALID;
   h->bnd_user = out;
@@ -1169,9 +1342,11 @@ struct DiagAxisHost {
   }
 };
 
+// win_rows / win_cols / origin: the planes are windows of the domain, origin[2 s] = (column, row) of slot s's
+// window (lec_diag850_host_windows); origin NULL: whole-domain planes.
 int diag850_run(const lec_diag_grid* g, const void* u, const void* v, const void* z, int32_t nslots,
                 const lec_diag_step* steps, int32_t nsteps, double* out_val, int32_t* out_idx, cudaStream_t st,
-                bool host_io) {
+                bool host_io, int win_rows = 0, int win_cols = 0, const int32_t* origin = nullptr) {
   if (!g || !u || !v || !z || !steps || !out_val || !out_idx || nsteps < 0 || nslots < 1 || !g->dx || !g->dy ||
       !g->parallel_scale || !g->meridional_scale || (g->dtype != LEC_F32 && g->dtype != LEC_F64))
     return LEC_ERR_INVALID;
@@ -1183,10 +1358,32 @@ int diag850_run(const lec_diag_grid* g, const void* u, const void* v, const void
         q.j0 > q.j1 || q.ic >= g->nlon || q.jc >= g->nlat)
       return LEC_ERR_BOUNDS;
   }
+  if (origin) {        // every value the kernel reads must lie inside the step's window (header: the window rule)
+    if (win_rows < 1 || win_cols < 1) return LEC_ERR_INVALID;
+    for (int s = 0; s < nsteps; ++s) {
+      const lec_diag_step& q = steps[s];
+      const int ox = origin[2 * q.slot], oy = origin[2 * q.slot + 1];
+      // columns / rows the 3-point stencils of the box points (and of the centre point) read
+      auto span = [](int a, int b, int n, int& lo, int& hi) {
+        lo = std::min(std::max(a - 1, 0), n - 3); hi = std::max(std::min(b + 1, n - 1), 2);
+      };
+      int xl, xh, yl, yh;
+      span(q.ic >= 0 && q.jc >= 0 ? std::min(q.i0, q.ic) : q.i0, q.ic >= 0 && q.jc >= 0 ? std::max(q.i1, q.ic) : q.i1,
+           g->nlon, xl, xh);
+      span(q.ic >= 0 && q.jc >= 0 ? std::min(q.j0, q.jc) : q.j0, q.ic >= 0 && q.jc >= 0 ? std::max(q.j1, q.jc) : q.j1,
+           g->nlat, yl, yh);
+      if (xl < ox || xh >= ox + win_cols || yl < oy || yh >= oy + win_rows) {
+        g_free_err = "a step reads outside its window";
+        return LEC_ERR_BOUNDS;
+      }
+    }
+  }
   int rc = LEC_OK;
   const int nx = g->nlon, ny = g->nlat;
   const size_t elem = g->dtype == LEC_F64 ? 8 : 4;
-  const size_t plane_bytes = (size_t)nslots * ny * nx * elem;
+  const int ld = origin ? win_cols : nx;
+  const long long plane = origin ? (long long)win_rows * win_cols : (long long)ny * nx;
+  const size_t plane_bytes = (size_t)nslots * plane * elem;
   DiagAxisHost ax(g->dx, nx), ay(g->dy, ny);
   // one table upload: [ax.A ax.B ax.C | ay.A ay.B ay.C | k | h | (h/k) dk/dy | k/h] then the steps
   std::vector<double> tab;
@@ -1208,7 +1405,8 @@ int diag850_run(const lec_diag_grid* g, const void* u, const void* v, const void
   const void* src[3] = {u, v, z};
   std::vector<DiagStepDev> hs(nsteps);
   for (int s = 0; s < nsteps; ++s)
-    hs[s] = DiagStepDev{steps[s].slot, steps[s].i0, steps[s].i1, steps[s].j0, steps[s].j1, steps[s].ic, steps[s].jc};
+    hs[s] = DiagStepDev{steps[s].slot, steps[s].i0, steps[s].i1, steps[s].j0, steps[s].j1, steps[s].ic, steps[s].jc,
+                        origin ? origin[2 * steps[s].slot] : 0, origin ? origin[2 * steps[s].slot + 1] : 0};
   DiagParams p{};
   CKF(cudaSetDevice(g->device));
   CKF(cudaMalloc(&d_tab, tab.size() * sizeof(double)));
@@ -1229,7 +1427,7 @@ int diag850_run(const lec_diag_grid* g, const void* u, const void* v, const void
   p.ps = d_tab + 3 * nx + 3 * ny; p.ms = p.ps + ny; p.dxcorr = p.ms + ny; p.pm = p.dxcorr + ny;
   p.su = g->scale[0]; p.sv = g->scale[1]; p.sz = g->scale[2]; p.zdiv = g->z_div;
   p.steps = d_steps; p.out_val = host_io ? d_val : out_val; p.out_idx = host_io ? d_idx : out_idx;
-  p.nlon = nx; p.nlat = ny;
+  p.nlon = nx; p.nlat = ny; p.ld = ld; p.plane = plane;
   if (g->dtype == LEC_F64) lec_diag850_kernel<double><<<nsteps, kDiagThreads, 0, st>>>(p);
   else lec_diag850_kernel<float><<<nsteps, kDiagThreads, 0, st>>>(p);
   CKF(cudaGetLastError());
@@ -1254,6 +1452,13 @@ int lec_diag850_device(const lec_diag_grid* grid, const void* u, const void* v, 
 int lec_diag850_host(const lec_diag_grid* grid, const void* u, const void* v, const void* z, int32_t nslots,
                      const lec_diag_step* steps, int32_t nsteps, double* out_val, int32_t* out_idx) {
   return diag850_run(grid, u, v, z, nslots, steps, nsteps, out_val, out_idx, nullptr, true);
+}
+
+int lec_diag850_host_windows(const lec_diag_grid* grid, const void* u, const void* v, const void* z, int32_t nslots,
+                             int32_t win_rows, int32_t win_cols, const int32_t* origin, const lec_diag_step* steps,
+                             int32_t nsteps, double* out_val, int32_t* out_idx) {
+  if (!origin) return LEC_ERR_INVALID;
+  return diag850_run(grid, u, v, z, nslots, steps, nsteps, out_val, out_idx, nullptr, true, win_rows, win_cols, origin);
 }
 
 }  // extern "C"

@@ -70,7 +70,9 @@ struct RowParams {
   int nbands;            // (read by the host only)
   int tiles_per_band;    // CTA row-tiles per latitude band
   FastDiv dv_tiles, dv_lev, dv_steps;   // block / tile index -> (band, step, level, row tile)
-  long long slot_stride; // elements per slot = nlev*nlat*nlon
+  long long slot_stride; // elements per slot = nlev * lev_stride
+  long long lev_stride;  // elements per level of a slot: rows * row_stride (the window's rows, or nlat)
+  int row_stride;        // elements per row (the window's pitch, or the fields' row length)
   long long grid;        // number of CTAs
   PackedDev pk;          // int16 instances only
 };
@@ -302,19 +304,19 @@ lec_row_moments_kernel(const RowParams p) {
   const int jrel = (band * p.tiles_per_band + jt) * kRowsPerCta + warp;
   if (jrel > j1 - j0) return;                 // warp-uniform; no block barriers below
   const int j = j0 + jrel;
-  const int nlon = p.g.nlon, nlat = p.g.nlat, nlev = p.g.nlev;
+  const int nlon = p.row_stride, nlev = p.g.nlev;
 
-  // One 64-bit base per field (the centre row); the six T neighbours are 32-bit element offsets
-  // from the T base, so a load address is one IMAD.WIDE (the host checks the offsets fit 31 bits).
-  const long long plane = (long long)nlat * nlon;
-  const long long row_c = ((long long)st->slot * nlev + k) * plane + (long long)j * nlon;
+  // One 64-bit base per field (the centre row, shifted by the window origin so that global columns index it); the six
+  // T neighbours are 32-bit element offsets from the T base, so a load address is one IMAD.WIDE (the host checks the
+  // offsets fit 31 bits).
+  const long long plane = p.lev_stride;
+  const long long row_c = ((long long)st->slot * nlev + k) * plane + (long long)(j - st->oy) * nlon - st->ox;
   const FT* __restrict__ Tc_row = static_cast<const FT*>(p.field[0]) + row_c;
   const FT* __restrict__ U_row = static_cast<const FT*>(p.field[1]) + row_c;
   const FT* __restrict__ V_row = static_cast<const FT*>(p.field[2]) + row_c;
   const FT* __restrict__ W_row = static_cast<const FT*>(p.field[3]) + row_c;
   const FT* __restrict__ F_row = static_cast<const FT*>(p.field[4]) + row_c;
-  const int d_m = int((long long)(st->slot_m - st->slot) * p.slot_stride);
-  const int d_p = int((long long)(st->slot_p - st->slot) * p.slot_stride);
+  const int d_m = st->d_m, d_p = st->d_p;
   const int d_km = (k > 0) ? -int(plane) : 0, d_kp = (k < nlev - 1) ? int(plane) : 0;
   const int d_jm = (j > j0) ? -nlon : 0, d_jp = (j < j1) ? nlon : 0;
 

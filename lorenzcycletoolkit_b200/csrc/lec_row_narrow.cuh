@@ -71,17 +71,17 @@ lec_row_moments_narrow_kernel(const RowParams p) {
   const bool row_on = jrel_first + wr <= j1 - j0; // groups past the last row compute on a clamped row, write nothing
   const int jrel = min(jrel_first + wr, j1 - j0);
   const int j = j0 + jrel;
-  const int nlon = p.g.nlon, nlat = p.g.nlat, nlev = p.g.nlev;
+  const int nlon = p.row_stride, nlev = p.g.nlev;
 
-  const long long plane = (long long)nlat * nlon;
-  const long long row_c = ((long long)st->slot * nlev + k) * plane + (long long)j * nlon;
+  // (window coordinates: see lec_row_moments_kernel)
+  const long long plane = p.lev_stride;
+  const long long row_c = ((long long)st->slot * nlev + k) * plane + (long long)(j - st->oy) * nlon - st->ox;
   const ST* __restrict__ Tc_row = static_cast<const ST*>(p.field[0]) + row_c;
   const ST* __restrict__ U_row = static_cast<const ST*>(p.field[1]) + row_c;
   const ST* __restrict__ V_row = static_cast<const ST*>(p.field[2]) + row_c;
   const ST* __restrict__ W_row = static_cast<const ST*>(p.field[3]) + row_c;
   const ST* __restrict__ F_row = static_cast<const ST*>(p.field[4]) + row_c;
-  const int d_m = int((long long)(st->slot_m - st->slot) * p.slot_stride);
-  const int d_p = int((long long)(st->slot_p - st->slot) * p.slot_stride);
+  const int d_m = st->d_m, d_p = st->d_p;
   const int d_km = (k > 0) ? -int(plane) : 0, d_kp = (k < nlev - 1) ? int(plane) : 0;
   const int d_jm = (j > j0) ? -nlon : 0, d_jp = (j < j1) ? nlon : 0;
 

@@ -209,33 +209,38 @@ lec_row_moments_tile_kernel(const __grid_constant__ TmaMaps maps, const RowParam
         const int jt0 = st->j0 + jr;
         const int k = t.k, km = k > 0 ? k - 1 : k, kp = k < nlev - 1 ? k + 1 : k;
         const int slot = st->slot, slot_m = st->slot_m, slot_p = st->slot_p;
+        // TMA coordinates are window-local (StepDev): the centre slot's, and slot_m's / slot_p's for T(t-1) / T(t+1);
+        // a coordinate outside the window is zero-filled like one outside the grid
+        const int jc = jt0 - st->oy, jm = jt0 - st->oym, jp = jt0 - st->oyp;
+        const int dxm = st->ox - st->oxm, dxp = st->ox - st->oxp;
         int col = c0 * VEC;
         if constexpr (G::I16) col &= ~7;             // 16-byte aligned box start
+        col -= st->ox;
         for (int ch = 0; ch < nch; ++ch, col += C) {
           mbar_wait(empty0 + 8 * stg, phase ^ 1);
           const unsigned fb = full0 + 8 * stg;
           mbar_expect_tx(fb, (unsigned)G::tx_bytes);
           const unsigned base = smem_u32(smem) + (unsigned)stg * G::stage_bytes;
-          tma_load_4d(base, &maps.t_halo, fb, col - HV, jt0 - 1, k, slot);
+          tma_load_4d(base, &maps.t_halo, fb, col - HV, jc - 1, k, slot);
           unsigned d = base + G::halo_bytes_pad;
           // u, v, omega, Phi with the L2 evict-first hint over fp64 fields (decoded type for int16 fields): 46.7 -> 39.0
           // GB of DRAM reads per 24-step launch, +3.4 %.  With fp32 fields the working set of a band fits in L2 without
           // it and the hint costs 2 %.
           if constexpr (sizeof(FT) == 8) {
-            tma_load_4d_hint(d, &maps.u, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
-            tma_load_4d_hint(d, &maps.v, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
-            tma_load_4d_hint(d, &maps.w, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
-            tma_load_4d_hint(d, &maps.f, fb, col, jt0, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.u, fb, col, jc, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.v, fb, col, jc, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.w, fb, col, jc, k, slot, pol_stream); d += G::tile_bytes;
+            tma_load_4d_hint(d, &maps.f, fb, col, jc, k, slot, pol_stream); d += G::tile_bytes;
           } else {
-            tma_load_4d(d, &maps.u, fb, col, jt0, k, slot); d += G::tile_bytes;
-            tma_load_4d(d, &maps.v, fb, col, jt0, k, slot); d += G::tile_bytes;
-            tma_load_4d(d, &maps.w, fb, col, jt0, k, slot); d += G::tile_bytes;
-            tma_load_4d(d, &maps.f, fb, col, jt0, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.u, fb, col, jc, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.v, fb, col, jc, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.w, fb, col, jc, k, slot); d += G::tile_bytes;
+            tma_load_4d(d, &maps.f, fb, col, jc, k, slot); d += G::tile_bytes;
           }
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, k, slot_p); d += G::tile_bytes;
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, k, slot_m); d += G::tile_bytes;
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, km, slot); d += G::tile_bytes;
-          tma_load_4d(d, &maps.t_plain, fb, col, jt0, kp, slot);
+          tma_load_4d(d, &maps.t_plain, fb, col + dxp, jp, k, slot_p); d += G::tile_bytes;
+          tma_load_4d(d, &maps.t_plain, fb, col + dxm, jm, k, slot_m); d += G::tile_bytes;
+          tma_load_4d(d, &maps.t_plain, fb, col, jc, km, slot); d += G::tile_bytes;
+          tma_load_4d(d, &maps.t_plain, fb, col, jc, kp, slot);
           if (++stg == NSTG) { stg = 0; phase ^= 1; }
         }
       }

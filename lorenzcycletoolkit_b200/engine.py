@@ -172,6 +172,8 @@ def load_library():
     lib.lec_last_transfer.restype = C.c_int
     lib.lec_set_boundary_levels.argtypes = [vp, vp]
     lib.lec_set_boundary_levels.restype = C.c_int
+    lib.lec_set_host_windows.argtypes = [vp, C.c_int32]
+    lib.lec_set_host_windows.restype = C.c_int
     lib.lec_pin_host.argtypes = [vp, C.c_int64]
     lib.lec_pin_host.restype = C.c_int
     lib.lec_unpin_host.argtypes = [vp]
@@ -181,6 +183,9 @@ def load_library():
     lib.lec_last_dispatch.argtypes = [vp, C.POINTER(_Dispatch)]
     lib.lec_last_dispatch.restype = C.c_int
     lib.lec_diag850_host.argtypes = [C.POINTER(_DiagGrid), vp, vp, vp, C.c_int32, vp, C.c_int32, vp, vp]
+    lib.lec_diag850_host_windows.argtypes = [C.POINTER(_DiagGrid), vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, vp, vp,
+                                             C.c_int32, vp, vp]
+    lib.lec_diag850_host_windows.restype = C.c_int
     lib.lec_diag850_host.restype = C.c_int
     lib.lec_diag850_device.argtypes = [C.POINTER(_DiagGrid), vp, vp, vp, C.c_int32, vp, C.c_int32, vp, vp, vp]
     lib.lec_diag850_device.restype = C.c_int
@@ -218,21 +223,17 @@ def gradient_coefs(x):
     return a, b, c
 
 
-def diag850_host(u, v, z, lon_deg, lat_deg, steps, scale=(1.0, 1.0, 1.0), z_div=1.0, device=0):
-    """850-hPa track diagnostics on the GPU (``lec_diag850_host``): ``u, v, z`` are ``[slot][lat][lon]``
-    planes of the 850-hPa level (one float dtype), ``steps`` a :data:`DIAG_STEP_DTYPE` array of
-    label-sliced boxes (:func:`diag_steps`).  Vorticity is MetPy's on the lat / lon grid
-    (``utils.geodesy.latlon_grid_metrics``).  Returns ``(values[n, 5], flat_index[n, 4])``: the extrema in
-    :data:`DIAG_NAMES` order with NaNs skipped and zeta at the step's centre point (NaN if none), and numpy
-    ``argmin`` / ``argmax`` of the box (row-major)."""
+def _diag850(u, v, z, lon_deg, lat_deg, steps, scale, z_div, device, origins=None):
+    """lec_diag850_host (``origins`` None: whole planes) or lec_diag850_host_windows (``origins[nslots][2]``)."""
     from .utils.geodesy import latlon_grid_metrics
     lib = load_library()
     dt = np.float32 if all(np.asarray(a).dtype == np.float32 for a in (u, v, z)) else np.float64
     planes = [np.ascontiguousarray(a, dtype=dt) for a in (u, v, z)]
     if planes[0].ndim != 3 or any(a.shape != planes[0].shape for a in planes):
         raise ValueError("u, v, z must be [slot][lat][lon] planes of one shape")
-    nslots, nlat, nlon = planes[0].shape
-    if np.size(lon_deg) != nlon or np.size(lat_deg) != nlat:
+    nslots, rows, cols = planes[0].shape
+    nlon, nlat = np.size(lon_deg), np.size(lat_deg)
+    if origins is None and (nlon, nlat) != (cols, rows):
         raise ValueError("coordinate sizes do not match the planes")
     if nlon < 3 or nlat < 3:
         raise ValueError("the 850-hPa diagnostics need at least three grid points along each axis "
@@ -247,13 +248,61 @@ def diag850_host(u, v, z, lon_deg, lat_deg, steps, scale=(1.0, 1.0, 1.0), z_div=
     st = np.ascontiguousarray(steps, dtype=DIAG_STEP_DTYPE)
     vals = np.empty((st.size, NDIAG_VALUES), dtype=np.float64)
     idx = np.empty((st.size, len(DIAG_NAMES)), dtype=np.int32)
-    rc = lib.lec_diag850_host(C.byref(g), planes[0].ctypes.data, planes[1].ctypes.data, planes[2].ctypes.data,
-                              nslots, st.ctypes.data, st.size, vals.ctypes.data, idx.ctypes.data)
+    ptrs = (planes[0].ctypes.data, planes[1].ctypes.data, planes[2].ctypes.data)
+    if origins is None:
+        what = "lec_diag850_host"
+        rc = lib.lec_diag850_host(C.byref(g), *ptrs, nslots, st.ctypes.data, st.size, vals.ctypes.data, idx.ctypes.data)
+    else:
+        what = "lec_diag850_host_windows"
+        org = np.ascontiguousarray(origins, dtype=np.int32)
+        if org.shape != (nslots, 2):
+            raise ValueError("origins must be [nslots][2] (column, row)")
+        rc = lib.lec_diag850_host_windows(C.byref(g), *ptrs, nslots, rows, cols, org.ctypes.data, st.ctypes.data,
+                                          st.size, vals.ctypes.data, idx.ctypes.data)
     if rc != 0:
-        msg = f"lec_diag850_host: {lib.lec_strerror(rc).decode()}"
+        msg = f"{what}: {lib.lec_strerror(rc).decode()}"
         extra = lib.lec_last_error(None).decode()
-        raise _ERRORS.get(rc, RuntimeError)(msg + (f" ({extra})" if extra and rc == -2 else ""))
+        raise _ERRORS.get(rc, RuntimeError)(msg + (f" ({extra})" if extra and rc in (-2, -4) else ""))
     return vals, idx
+
+
+def diag850_host(u, v, z, lon_deg, lat_deg, steps, scale=(1.0, 1.0, 1.0), z_div=1.0, device=0):
+    """850-hPa track diagnostics on the GPU (``lec_diag850_host``): ``u, v, z`` are ``[slot][lat][lon]``
+    planes of the 850-hPa level (one float dtype), ``steps`` a :data:`DIAG_STEP_DTYPE` array of
+    label-sliced boxes (:func:`diag_steps`).  Vorticity is MetPy's on the lat / lon grid
+    (``utils.geodesy.latlon_grid_metrics``).  Returns ``(values[n, 5], flat_index[n, 4])``: the extrema in
+    :data:`DIAG_NAMES` order with NaNs skipped and zeta at the step's centre point (NaN if none), and numpy
+    ``argmin`` / ``argmax`` of the box (row-major)."""
+    return _diag850(u, v, z, lon_deg, lat_deg, steps, scale, z_div, device)
+
+
+def diag_windows(steps, nlon, nlat):
+    """The plane windows ``lec_diag850_host_windows`` needs, one per step (plane ``s`` = step ``s``): the box and the
+    centre point grown by one point a side, clamped to the domain, at least three points along an axis where it meets
+    a domain edge (MetPy's one-sided 3-point derivatives), then one shape for all (the largest), origins moved so that
+    every window lies inside the domain.  Returns ``(origins[n][2] (column, row), rows, cols)``."""
+    st = np.asarray(steps)
+    n = st.size
+    spans = np.zeros((n, 4), dtype=np.int64)
+    for s in range(n):
+        q = st[s]
+        centre = q["ic"] >= 0 and q["jc"] >= 0
+        for ax, (a, b, c, m) in enumerate(((q["i0"], q["i1"], q["ic"], nlon), (q["j0"], q["j1"], q["jc"], nlat))):
+            lo, hi = (min(a, c), max(b, c)) if centre else (a, b)
+            spans[s, 2 * ax] = min(max(lo - 1, 0), m - 3)
+            spans[s, 2 * ax + 1] = max(min(hi + 1, m - 1), 2)
+    cols = int((spans[:, 1] - spans[:, 0] + 1).max()) if n else 3
+    rows = int((spans[:, 3] - spans[:, 2] + 1).max()) if n else 3
+    origins = np.stack([np.minimum(spans[:, 0], nlon - cols), np.minimum(spans[:, 2], nlat - rows)], axis=1)
+    return origins.astype(np.int32), rows, cols
+
+
+def diag850_host_windows(u, v, z, origins, lon_deg, lat_deg, steps, scale=(1.0, 1.0, 1.0), z_div=1.0, device=0):
+    """:func:`diag850_host` on windows of the planes (``lec_diag850_host_windows``): ``u, v, z`` are
+    ``[slot][rows][cols]``, plane ``s`` holding the domain points from column ``origins[s][0]``, row
+    ``origins[s][1]`` on (:func:`diag_windows` gives the windows a step list needs).  Box and centre indices of
+    ``steps`` stay domain indices; same results as :func:`diag850_host` on the whole planes, bit for bit."""
+    return _diag850(u, v, z, lon_deg, lat_deg, steps, scale, z_div, device, origins=origins)
 
 
 _PINNED = {}          # start address -> (bytes, weakref to the owner of the memory)
@@ -318,6 +367,73 @@ def _set_decode(d, decode):
         d.nfill[f] = len(fills)
         for n, fv in enumerate(fills[:2]):
             d.fill[f][n] = float(fv)
+
+
+def track_windows(steps, grid, dtype, nslots=None, max_steps=64, stage_slots=None, raw=None):
+    """The staging windows of one ``lec_run_host*`` call with ``lec_set_host_windows(1)`` (include/lec_b200.h), in
+    numpy: what the engine stages and the host->device bytes ``last_transfer()[0]`` reports.
+
+    ``grid`` = ``(nlev, nlat, nlon)``; ``dtype`` the engine dtype; ``stage_slots`` the staging window in slots (default:
+    ``min(max_steps + 2, nslots)``, a fresh handle whose budget holds that many); ``raw`` = ``(lon_map, lat_map,
+    lev_map, raw_nlon, raw_itemsize)`` for ``lec_run_host_raw``.  Returns a dict: ``t`` and ``c`` ``[nslots][4]``
+    rectangles ``(x0, x1, y0, y1)`` of T and of u / v / omega / Phi (``x1 < x0``: not read), ``rows`` and ``pitch``
+    of the shared window shape, ``h2d_bytes``."""
+    steps = np.asarray(steps)
+    nlev, nlat, nlon = (int(n) for n in grid)
+    vecw = 2 if np.dtype(dtype) == np.float64 else 4
+    elem = np.dtype(dtype).itemsize
+    if nslots is None:
+        nslots = int(max(steps["slot"].max(), steps["slot_m"].max(), steps["slot_p"].max())) + 1
+    t = np.tile(np.array([0, -1, 0, -1], dtype=np.int64), (nslots, 1))
+    c = t.copy()
+
+    def grow(r, s):
+        box = (int(s["i0"]), int(s["i1"]), int(s["j0"]), int(s["j1"]))
+        r[:] = box if r[1] < r[0] else (min(r[0], box[0]), max(r[1], box[1]), min(r[2], box[2]), max(r[3], box[3]))
+    for s in steps:
+        grow(c[s["slot"]], s)
+        for k in ("slot", "slot_m", "slot_p"):
+            grow(t[s[k]], s)
+    for r in (t, c):
+        live = r[:, 1] >= r[:, 0]
+        r[live, 0] -= r[live, 0] % vecw
+    live = t[:, 1] >= t[:, 0]
+    rows = int((t[live, 3] - t[live, 2] + 1).max())
+    pitch = int(((t[live, 1] - t[live, 0] + vecw) // vecw * vecw).max())
+
+    def nbytes(r):
+        if r[1] < r[0]:
+            return 0
+        nx, ny = int(r[1] - r[0] + 1), int(r[3] - r[2] + 1)
+        if raw is None:
+            return nlev * ny * nx * elem
+        lon_map, lat_map, lev_map, raw_nlon, itemsize = raw
+        lat = np.asarray(lat_map)[r[2]:r[3] + 1]
+        lon = np.asarray(lon_map)[r[0]:r[1] + 1]
+        nk = int(np.max(lev_map) - np.min(lev_map) + 1)
+        run = np.array_equal(lon, lon[0] + np.arange(nx))
+        return nk * int(lat.max() - lat.min() + 1) * (nx if run else int(raw_nlon)) * int(itemsize)
+    tb, cb = [nbytes(r) for r in t], [nbytes(r) for r in c]
+
+    window = min(max_steps + 2, nslots) if stage_slots is None else int(stage_slots)
+    n, s0, chunk, prev_lo, prev_hi, total = len(steps), 0, 0, 0, -1, 0
+    while s0 < n:                       # the greedy chunks of run_host_impl
+        lo, hi, s1 = 1 << 30, -1, s0
+        while s1 < n and s1 - s0 < max_steps:
+            sl = [int(steps[k][s1]) for k in ("slot", "slot_m", "slot_p")]
+            if max(hi, *sl) - min(lo, *sl) + 1 > window:
+                break
+            lo, hi, s1 = min(lo, *sl), max(hi, *sl), s1 + 1
+        if s1 == s0:
+            raise MemoryError("one step needs more slots than the staging window holds")
+        t_lo = lo
+        if chunk >= 1 and prev_lo <= lo <= prev_hi:
+            t_lo = min(prev_hi, hi) + 1
+        total += sum(tb[t_lo:hi + 1])
+        centre = steps["slot"][s0:s1]
+        total += 4 * sum(cb[int(centre.min()):int(centre.max()) + 1])
+        prev_lo, prev_hi, s0, chunk = lo, hi, s1, chunk + 1
+    return {"t": t, "c": c, "rows": rows, "pitch": pitch, "h2d_bytes": total}
 
 
 def make_steps(nsteps: int) -> np.ndarray:
@@ -414,6 +530,11 @@ class LecEngine:
         self.last_boundary = np.empty((n, 6, 3, self.nlev), dtype=np.float64) if want else None
         self._check(self._lib.lec_set_boundary_levels(
             self._h, self.last_boundary.ctypes.data if want else None), "lec_set_boundary_levels")
+
+    def set_host_windows(self, on: bool):
+        """``lec_set_host_windows``: stage only each slot's window in the following :meth:`run_host` /
+        :meth:`run_host_raw` calls (the rule and the bytes: :func:`track_windows`); same results."""
+        self._check(self._lib.lec_set_host_windows(self._h, int(bool(on))), "lec_set_host_windows")
 
     def run_host(self, fields, steps, want_levels=True, want_boundary=False):
         """``lec_run_host``: ``fields`` = five C-contiguous host arrays

@@ -65,28 +65,34 @@ def get_limits(args, t, data850, track=None):
             "min_lat": central_lat - length / 2, "max_lat": central_lat + length / 2}
 
 
-def diagnostics_850(data, variable_list_df, limits_list, device=None):
+def diagnostics_850(data, variable_list_df, limits_list, device=None, windows=True):
     """850-hPa wind speed, relative vorticity (MetPy's ``vorticity`` on the lat / lon grid) and geopotential
     height (lec_moving_framework.py:650-663), their extrema inside every step's label-sliced box
     (get_position, :269-417) and the vorticity at the grid point nearest to the track centre (the ``-z``
     branch, :317-324), for ALL time steps in one ``lec_diag850_host`` call on the GPU (the reference recomputes
     the domain-wide fields per step inside its time loop).
     Returns per step ``(values[5], flat_index[4], lat_of_box, lon_of_box)``: ``engine.DIAG_NAMES`` order, then
-    zeta at the centre."""
+    zeta at the centre.  ``windows``: gather and copy only each step's window of the three planes
+    (``lec_diag850_host_windows``, same bits), else the whole planes (``lec_diag850_host``)."""
     from .. import engine as E
     k = int(np.argmin(np.abs(np.asarray(data.level, dtype=np.float64) - 85000.0)))
     if float(data.level[k]) != 85000.0:
         raise KeyError("85000 Pa level not found (the moving framework needs 850 hPa)")
 
-    def plane(row):
-        return data.level_plane(variable_list_df.loc[row]["Variable"], k), \
-            unit_factor(variable_list_df.loc[row]["Units"], row)
-    (u, su), (v, sv) = plane("Eastward Wind Component"), plane("Northward Wind Component")
-    if "Geopotential" in variable_list_df.index:
-        (z, sz), z_div = plane("Geopotential"), G
-    else:
-        (z, sz), z_div = plane("Geopotential Height"), 1.0
     lat, lon = np.asarray(data.lat), np.asarray(data.lon)
+    rows_z = ["Geopotential", G] if "Geopotential" in variable_list_df.index else ["Geopotential Height", 1.0]
+    z_div = rows_z[1]
+    names = ["Eastward Wind Component", "Northward Wind Component", rows_z[0]]
+    su, sv, sz = (unit_factor(variable_list_df.loc[row]["Units"], row) for row in names)
+
+    def planes(a, b, origins=None, shape=None):
+        """u, v, z of times a..b-1: whole planes, or the windows of ``origins`` (one per time)."""
+        out = []
+        for row in names:
+            var = variable_list_df.loc[row]["Variable"]
+            out.append(data.level_plane(var, k)[a:b] if origins is None else
+                       data.level_plane_windows(var, k, origins, *shape, times=np.arange(a, b)))
+        return out
     steps = np.zeros(len(limits_list), dtype=E.DIAG_STEP_DTYPE)
     boxes = []
     for it, lim in enumerate(limits_list):
@@ -108,8 +114,15 @@ def diagnostics_850(data, variable_list_df, limits_list, device=None):
         import torch
         device = int(os.environ.get("LOCAL_RANK", rank)) % max(torch.cuda.device_count(), 1) if world > 1 else \
             int(os.environ.get("LOCAL_RANK", 0))
+    def run(st, a, b):                 # steps of times a..b-1, slot = time - a
+        if not windows:
+            return E.diag850_host(*planes(a, b), lon, lat, st, scale=(su, sv, sz), z_div=z_div, device=device)
+        origins, wy, wx = E.diag_windows(st, len(lon), len(lat))
+        return E.diag850_host_windows(*planes(a, b, origins, (wy, wx)), origins, lon, lat, st, scale=(su, sv, sz),
+                                      z_div=z_div, device=device)
+
     if world == 1:
-        vals, idx = E.diag850_host(u, v, z, lon, lat, steps, scale=(su, sv, sz), z_div=z_div, device=device)
+        vals, idx = run(steps, 0, len(steps))
     else:
         # time-sharded like the LEC terms: this rank's steps (no halo: the diagnostics are per-time), then one
         # all-gather of the 4 values + 4 indices per step
@@ -121,8 +134,7 @@ def diagnostics_850(data, variable_list_df, limits_list, device=None):
         if b > a:
             st = steps[a:b].copy()
             st["slot"] -= a
-            lv, li = E.diag850_host(u[a:b], v[a:b], z[a:b], lon, lat, st, scale=(su, sv, sz), z_div=z_div,
-                                    device=device)
+            lv, li = run(st, a, b)
             local[:, :5], local[:, 5:] = lv, li
         t = torch.from_numpy(local)
         if dist.get_backend() == "nccl":
@@ -256,7 +268,10 @@ def lec_moving(data, variable_list_df, dTdt, results_subdirectory, figures_direc
     track = handle_track_file(data, times, LonIndexer, LatIndexer, TimeName, args, app_logger)
 
     limits_list = [get_limits(args, t, None, track) for t in times]
-    d850 = diagnostics_850(data, variable_list_df, limits_list)
+    # staging windows (lec_set_host_windows, lec_diag850_host_windows): the run's host->device bytes follow the box,
+    # not the domain; engine_options={"host_windows": False} stages whole slots / planes (the same bits)
+    windows = bool((engine_options or {}).get("host_windows", True))
+    d850 = diagnostics_850(data, variable_list_df, limits_list, windows=windows)
     rows = []
     for it, t in enumerate(times):
         limits = limits_list[it]

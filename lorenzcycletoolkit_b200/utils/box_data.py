@@ -108,8 +108,10 @@ def run_time_sharded(data, dtype, scale, fields, steps, max_box_rows, opts):
     except ImportError:
         dist = None
     opts = dict(opts)
+    windows = bool(opts.pop("host_windows", False))      # lec_set_host_windows: each rank windows its own shard
 
     def run(eng, f, st):
+        eng.set_host_windows(windows)
         if isinstance(f, RawInput):
             out = f.run(eng, st, want_boundary=True)
         else:
@@ -289,8 +291,11 @@ class BoxBatch(BoxData):
             steps["i0"][it], steps["i1"][it], steps["j0"][it], steps["j1"][it] = i0, i1, j0, j1
             self.boxes.append((i0, i1, j0, j1))
         rows = int(max(b[3] - b[2] + 1 for b in self.boxes))
+        # moving boxes stage only each slot's window (engine_options={"host_windows": False}: whole slots)
+        opts = dict(engine_options or {})
+        opts.setdefault("host_windows", True)
         self.terms, self.levels, self.flags, self.timing_ms, self.boundary_levels = run_time_sharded(
-            data, dtype, scale, fields, steps, rows, dict(engine_options or {}))
+            data, dtype, scale, fields, steps, rows, opts)
         self.dtype = dtype
         self.idx = None
         self.c12 = np.array([boundary_constants(data, *b) for b in self.boxes])

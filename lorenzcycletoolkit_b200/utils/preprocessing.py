@@ -55,6 +55,15 @@ class RawStore:
         out = apply_decode(self.fields[var][np.ix_(self.rec, lev, self.lat, self.lon)], self.decode[var])
         return out if level is None else out[:, 0]
 
+    def plane_windows(self, var, level, times, origins, rows, cols):
+        """``materialise(var, level)[t, y0:y0 + rows, x0:x0 + cols]`` for each ``t`` of ``times`` with its origin
+        ``(x0, y0)`` of ``origins``, decoding only those points: ``[len(times)][rows][cols]``."""
+        raw = self.fields[var]
+        out = [apply_decode(raw[np.ix_(self.rec[[t]], self.lev[[level]], self.lat[y0:y0 + rows],
+                                       self.lon[x0:x0 + cols])], self.decode[var])[0, 0]
+               for t, (x0, y0) in zip(times, origins)]
+        return np.stack(out) if out else np.zeros((0, rows, cols))
+
 
 def decode_rule(stored_dtype, attrs):
     """The CF decode of a variable stored as ``stored_dtype`` with attributes ``attrs`` (what ``xr.open_dataset``
@@ -261,6 +270,16 @@ class LecDataset:
                 return v[tuple(idx)]
             out.variables = {k: pick(v) for k, v in out.variables.items()}
         return out
+
+    def level_plane_windows(self, var, k, origins, rows, cols, times=None):
+        """``level_plane(var, k)[t, y0:y0 + rows, x0:x0 + cols]`` for every time ``t`` (or those of ``times``) with its
+        window origin ``(x0, y0)``: ``[n][rows][cols]``.  A raw-backed dataset decodes only those points."""
+        times = np.arange(len(origins)) if times is None else np.asarray(times)
+        if self.raw is not None and var not in dict.keys(self.variables):
+            return self.raw.plane_windows(var, k, times, origins, rows, cols)
+        a = self[var]
+        return np.stack([np.asarray(a[t, k, y0:y0 + rows, x0:x0 + cols]) for t, (x0, y0) in zip(times, origins)]) \
+            if len(times) else np.zeros((0, rows, cols))
 
     def level_plane(self, var, k):
         """``self[var][:, k]`` without materialising the other levels of a raw-backed dataset."""
